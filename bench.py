@@ -69,7 +69,32 @@ def parse():
     ap.add_argument("--no-from-images", action="store_true", help="skip the images -> disparity leg (then e2e = e2e_pyramids)")
     ap.add_argument("--no-extras", action="store_true", help="skip tf32 / gpu_reference / bands / density sweep")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="host time of the bounded CPU sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="our arm: write what the last timed step returned (rank 0's final disparity) as DIR/disparity.npy, "
+                         "float32; inputs and weights are seeded, so two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to our arm only")
+    return args
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, outputs):
+    """Each tensor of `outputs` as out_dir/<name>.npy in float32, all of them together at most DUMP_BYTES.  A tensor larger
+    than its share is replaced by a fixed sample of it: the elements at sorted positions drawn without replacement by a
+    numpy generator seeded with 0, as a flat array (the same positions in every run with the same arguments)."""
+    import numpy as np
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    share = DUMP_BYTES // len(outputs) - 1024                    # room for the .npy header
+    for name, t in outputs.items():
+        a = t.detach().float().cpu().numpy()
+        if a.nbytes > share:
+            pos = np.sort(np.random.default_rng(0).choice(a.size, share // 4, replace=False))
+            a = a.reshape(-1)[pos]
+        np.save(out_dir / f"{name}.npy", a)
 
 
 def peaks():
@@ -262,7 +287,7 @@ def run_reference(args):
     # K steps, each a bounded sample (pairs for ~1.5 s of host time, at most the arm's batch)
     v1, cores, el1, n1 = cpu_port_pairs_per_s(args.workload, args.rho, min_seconds=1.5, max_pairs=args.batch,
                                               warmup=max(1, min(args.warmup, 2)))
-    steps = max(1, min(args.steps, 40))
+    steps = max(1, args.steps)
     tot_pairs, tot_s = n1, el1
     for _ in range(steps - 1):
         v, _, el, n = cpu_port_pairs_per_s(args.workload, args.rho, min_seconds=1.5, max_pairs=args.batch, warmup=0)
@@ -319,15 +344,18 @@ class Env:
         return ms
 
     def timed(self, fn, steps):
-        """`steps` calls of fn between barrier + synchronize on both sides, CUDA events on the launching stream, MAX over ranks."""
+        """`steps` calls of fn between barrier + synchronize on both sides, CUDA events on the launching stream, MAX over ranks.
+        What the last call returned is kept in self.last."""
         torch = self.torch
         self.barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        out = None
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         self.barrier()
+        self.last = out
         return self.max_over_ranks(e0.elapsed_time(e1))
 
 
@@ -743,6 +771,8 @@ def run_ours(args):
     if prof_range:
         torch.cuda.profiler.stop()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"disparity": env.last})     # before any later leg replays the graph again
     n_units = B if bands_mode else world * B          # bands: all ranks work on the SAME B pairs
     value = n_units * args.steps / (ms * 1e-3)
 

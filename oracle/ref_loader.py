@@ -1,18 +1,42 @@
-"""oracle/ref_loader.py -- TEST INFRASTRUCTURE.  Imports the UNMODIFIED reference package from /root/reference (build
-container) or from baseline/_ref (the git-ignored copy __graft_entry__.build() stages so that it travels to the GPU box):
-stubs the missing matplotlib / visdom modules (utils/utils.py:8, eval.py:10) and registers
+"""oracle/ref_loader.py -- TEST INFRASTRUCTURE.  Imports the UNMODIFIED reference package from the original DecNet
+project's source tree (source(): $DECNET_REFERENCE, else BASELINE.json's reference_path) or from baseline/_ref (the
+git-ignored copy __graft_entry__.build() stages from that tree so that it travels with the repository tree to a GPU
+machine): stubs the missing matplotlib / visdom modules (utils/utils.py:8, eval.py:10) and registers
 `modules.Sparse{Matching,Var}.build.lib` with an extension object of the caller's choice
 (the CPU oracle by default) so `from ..build.lib import SpaMat` resolves
 (modules/SparseMatching/functions/SpaMat.py:4).
 """
 from __future__ import annotations
 
+import json
+import os
 import sys
 import types
 from pathlib import Path
 
 _ROOT = Path(__file__).resolve().parents[1]
-REF = Path("/root/reference") if (Path("/root/reference") / "modules" / "submodule.py").exists() else _ROOT / "baseline" / "_ref"
+STAGED = _ROOT / "baseline" / "_ref"
+
+
+def _is_tree(p: Path) -> bool:
+    try:
+        return (p / "modules" / "submodule.py").exists()
+    except OSError:                         # a location this user may not read (another user's home) counts as absent
+        return False
+
+
+def source() -> Path | None:
+    """The original project's source tree, when this machine has one: $DECNET_REFERENCE, else BASELINE.json's
+    reference_path."""
+    cands = [Path(os.environ["DECNET_REFERENCE"])] if os.environ.get("DECNET_REFERENCE") else []
+    try:
+        cands.append(Path(json.loads((_ROOT / "BASELINE.json").read_text())["reference_path"]))
+    except (OSError, KeyError, ValueError):
+        pass
+    return next((p for p in cands if _is_tree(p)), None)
+
+
+REF = source() or STAGED
 
 
 class _OracleSpaMatExt:
@@ -50,14 +74,14 @@ class _OracleSpaVarExt:
 
 
 def available() -> bool:
-    return (REF / "modules" / "submodule.py").exists()
+    return _is_tree(REF)
 
 
 def install(spamat_ext=None, spavar_ext=None):
     """Make `import modules` (the reference package) work; returns the imported package."""
     if not available():
-        raise RuntimeError("the reference tree is present neither at /root/reference nor at baseline/_ref "
-                           "(run __graft_entry__.build() in the build container)")
+        raise RuntimeError("the original DecNet source tree was found neither at $DECNET_REFERENCE / BASELINE.json's "
+                           "reference_path nor staged at baseline/_ref (run __graft_entry__.build() where it is present)")
     for m in ("matplotlib", "matplotlib.pyplot", "visdom"):
         if m not in sys.modules:
             sys.modules[m] = types.ModuleType(m)

@@ -34,7 +34,8 @@ if __name__ == "__main__":
     for m in ("matplotlib", "matplotlib.pyplot", "visdom"):
         sys.modules.setdefault(m, types.ModuleType(m))
     sys.modules["matplotlib"].pyplot = sys.modules["matplotlib.pyplot"]
-    sys.path.insert(0, "/root/reference")
+    from oracle import ref_loader
+    sys.path.insert(0, str(ref_loader.REF))         # the original project's tree (oracle/ref_loader.py)
     from utils.utils import detailDetection          # the reference function itself (utils/utils.py:483-534)
     out = {"meta": np.array([SEED, H, W], dtype=np.int64)}
     for b, seed in enumerate((SEED, SEED + 1)):

@@ -2,6 +2,7 @@
 hot path behind the reference's module API.  See DESIGN.md / INTEGRATION.md."""
 from . import _lib  # noqa: F401  (does not load the .so until first use)
 from .modules import SpaMat, SpaMatFunction, SpaVar, SpaVarFunction
+from .predictor import StereoMatcher
 
-__all__ = ["SpaMat", "SpaMatFunction", "SpaVar", "SpaVarFunction"]
+__all__ = ["SpaMat", "SpaMatFunction", "SpaVar", "SpaVarFunction", "StereoMatcher"]
 __version__ = "0.1.0"

@@ -69,6 +69,7 @@ SIGNATURES = {
     "decnet_dynup_pack_nhwc": (_i, [_f32p] * 3 + [_i] * 7 + [C.c_void_p]),
     "decnet_dynup_set_disp_nhwc": (_i, [_f32p] * 2 + [_i] * 6 + [C.c_void_p]),
     "decnet_dynup_glue_nhwc": (_i, [_f32p] * 3 + [_i] * 5 + [C.c_void_p]),
+    "decnet_bicubic_up3": (_i, [_f32p] * 2 + [_i] * 5 + [C.c_void_p]),
     "decnet_sqdiff_pair": (_i, [_f32p] * 6 + [C.c_longlong, C.c_void_p]),
     "decnet_detail_head": (_i, [_f32p] * 3 + [C.c_float, C.c_float] + [_f32p] * 2 + [_i] * 3 + [C.c_void_p]),
     "decnet_detail_level_scratch_floats": (C.c_longlong, [_i] * 3),

@@ -27,7 +27,6 @@ on the path, so the whole banded step is captured in ONE CUDA graph per rank and
 from __future__ import annotations
 
 import torch
-import torch.nn.functional as F
 
 from . import conv3d as c3
 from . import ops, shard
@@ -303,8 +302,7 @@ def forward_bands(model, left_feats, right_feats, transport, left_mask_list=None
             out = {}
             for r in tr.ranks_here:
                 b = shard.level_band(H0, tr.world, r, s - 1, 2)
-                up = F.interpolate(full[r][:, b.e0:b.e1].unsqueeze(1) * 3, [3 * (b.e1 - b.e0), Lf.shape[3]],
-                                   mode="bicubic").squeeze(1)
+                up = ops.bicubic_skip(full[r][:, b.e0:b.e1].contiguous(), 3 * (b.e1 - b.e0), Lf.shape[3])
                 out[r] = up[:, 3 * (b.r0 - b.e0): 3 * (b.r1 - b.e0)].contiguous()
             full = gather(out, s)
             continue

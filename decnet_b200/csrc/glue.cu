@@ -783,6 +783,81 @@ haar_mask_kernel(const float *__restrict__ v, const unsigned int *__restrict__ m
     }
 }
 
+// ---------------------------------------------------------------------------------------------
+// a15: skip-stage up-sampling F.interpolate(pred*3, (H, W), mode="bicubic") (SparseDenseNetRefinementMask.py:143-144),
+// align_corners=False, A = -0.75, border taps clamped.  Bit-identical to ATen's upsample_bicubic2d_out_frame on CUDA:
+// the source index, the coefficients and the 4-tap sums below are ATen's expressions (UpSample.cuh) in the same fp32
+// types, so nvcc contracts them into the same FMAs; the scales are (float)in / out, computed on the host as ATen does.
+// One thread per output column and a strip of kBicRows output rows: the horizontal pass of an input row depends on the
+// column only, so the four rows under the vertical window slide down the strip and each input row is interpolated once
+// per column instead of four times; the stores of a warp are one coalesced 128-byte row segment per output row.
+// ---------------------------------------------------------------------------------------------
+constexpr int kBicRows = 8;
+
+__device__ __forceinline__ float bic_source_index(float scale, int dst_index) {
+    return scale * (dst_index + static_cast<float>(0.5)) - static_cast<float>(0.5);
+}
+
+__device__ __forceinline__ float bic_conv1(float x, float A) { return ((A + 2) * x - (A + 3)) * x * x + 1; }
+__device__ __forceinline__ float bic_conv2(float x, float A) { return ((A * x - 5 * A) * x + 8 * A) * x - 4 * A; }
+
+__device__ __forceinline__ float bic_interp1d(float x0, float x1, float x2, float x3, float t) {
+    float coeffs[4];
+    const float A = -0.75;
+    const float xa = t;
+    coeffs[0] = bic_conv2(xa + 1.0, A);
+    coeffs[1] = bic_conv1(xa, A);
+    const float xb = 1.0 - t;
+    coeffs[2] = bic_conv1(xb, A);
+    coeffs[3] = bic_conv2(xb + 1.0, A);
+    return x0 * coeffs[0] + x1 * coeffs[1] + x2 * coeffs[2] + x3 * coeffs[3];
+}
+
+// horizontal pass of input row y (clamped) at the four clamped columns around in_x; v = fl(pred * 3) first
+__device__ __forceinline__ float bic_row(const float *__restrict__ in, int y, int h, int w, int in_x, float t_x) {
+    const float *row = in + (size_t)max(min(y, h - 1), 0) * w;
+    const float v0 = __ldg(row + max(min(in_x - 1, w - 1), 0)) * 3.0f;
+    const float v1 = __ldg(row + max(min(in_x + 0, w - 1), 0)) * 3.0f;
+    const float v2 = __ldg(row + max(min(in_x + 1, w - 1), 0)) * 3.0f;
+    const float v3 = __ldg(row + max(min(in_x + 2, w - 1), 0)) * 3.0f;
+    return bic_interp1d(v0, v1, v2, v3, t_x);
+}
+
+__global__ void __launch_bounds__(128)
+bicubic_up3_kernel(const float *__restrict__ in, float *__restrict__ out, int h, int w, int H, int W,
+                   float scale_h, float scale_w)
+{
+    const int x = blockIdx.x * blockDim.x + threadIdx.x;
+    const int y0 = blockIdx.y * kBicRows;
+    if (x >= W) return;
+    const float *src = in + (size_t)blockIdx.z * h * w;
+    float *dst = out + (size_t)blockIdx.z * H * W;
+    const int y1 = min(y0 + kBicRows, H);
+    if (h == H && w == W) {                          // ATen's same-size branch: a copy of pred*3
+        for (int y = y0; y < y1; ++y) dst[(size_t)y * W + x] = __ldg(src + (size_t)y * w + x) * 3.0f;
+        return;
+    }
+    const float real_x = bic_source_index(scale_w, x);
+    const int in_x = floorf(real_x);
+    const float t_x = real_x - in_x;
+    // r0..r3: horizontal results of input rows cur-1 .. cur+2 (in_y is non-decreasing along the strip)
+    int cur = (int)floorf(bic_source_index(scale_h, y0));
+    float r0 = bic_row(src, cur - 1, h, w, in_x, t_x), r1 = bic_row(src, cur, h, w, in_x, t_x);
+    float r2 = bic_row(src, cur + 1, h, w, in_x, t_x), r3 = bic_row(src, cur + 2, h, w, in_x, t_x);
+    for (int y = y0; y < y1; ++y) {
+        const float real_y = bic_source_index(scale_h, y);
+        const int in_y = floorf(real_y);
+        const float t_y = real_y - in_y;
+        if (in_y - cur > 4) cur = in_y - 4;          // down-sampling: skip rows no window covers
+        while (cur < in_y) {
+            ++cur;
+            r0 = r1; r1 = r2; r2 = r3;
+            r3 = bic_row(src, cur + 2, h, w, in_x, t_x);
+        }
+        dst[(size_t)y * W + x] = bic_interp1d(r0, r1, r2, r3, t_y);
+    }
+}
+
 static inline int grid_for(long long n, int cap = 148 * 16) {
     long long g = (n + kBlock - 1) / kBlock;
     return (int)(g < cap ? (g > 0 ? g : 1) : cap);
@@ -1021,6 +1096,18 @@ int decnet_dynup_set_disp_nhwc(const float *disp, float *packed, int B, int h, i
     dynup_set_disp_nhwc_kernel<<<(unsigned)((n + kBlock - 1) / kBlock), kBlock, 0, (cudaStream_t)stream>>>(
         disp, packed, h, w, CP, round_tf32, pad, n);
     return after_launch("dynup_set_disp_nhwc_kernel");
+}
+
+int decnet_bicubic_up3(const float *pred, float *out, int B, int h, int w, int H, int W, void *stream) {
+    DECNET_REQUIRE(pred && out, "null pointer");
+    DECNET_REQUIRE(B > 0 && B <= 65535 && h > 0 && w > 0 && H > 0 && W > 0, "bad size B=%d %dx%d -> %dx%d", B, h, w, H, W);
+    const long long strips = ((long long)H + kBicRows - 1) / kBicRows;
+    DECNET_REQUIRE(strips <= 65535, "H=%d: too many rows for the launch grid", H);
+    // ATen's area_pixel_compute_scale without an explicit scale factor: (float)input_size / output_size
+    const float scale_h = (float)h / (float)H, scale_w = (float)w / (float)W;
+    bicubic_up3_kernel<<<dim3((W + 127) / 128, (unsigned)strips, B), 128, 0, (cudaStream_t)stream>>>(pred, out, h, w, H, W,
+                                                                                                   scale_h, scale_w);
+    return after_launch("bicubic_up3_kernel");
 }
 
 int decnet_dynup_glue_nhwc(const float *logits, const float *disp, float *out, int B, int h, int w, int NP, int pad, void *stream) {

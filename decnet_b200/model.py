@@ -679,8 +679,8 @@ class DecompMatching(nn.Module):
                         taps["cost"] = cost
                 pre_l, pre_r = Lf, Rf
             elif s >= self.skip_stage_id:
-                # SparseDenseNetRefinementMask.py:143-144 (Middlebury's finest level); single ATen kernel
-                pred = F.interpolate(pred.unsqueeze(1) * self.down_scale, list(Lf.shape[-2:]), mode="bicubic").squeeze(1)
+                # SparseDenseNetRefinementMask.py:143-144 (Middlebury's finest level): bicubic x3 of pred*3
+                pred = ops.bicubic_skip(pred, Lf.shape[-2], Lf.shape[-1])
             else:
                 l = s - 1
                 if branch is not None:

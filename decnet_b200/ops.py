@@ -332,6 +332,18 @@ def detail_detection(img, iters=3, thold=0.3):
     return masks
 
 
+def bicubic_skip(pred, out_h, out_w):
+    """Skip-stage up-sampling (SparseDenseNetRefinementMask.py:143-144): pred [B,h,w] -> [B,out_h,out_w] equal, bit for bit,
+    to F.interpolate((pred*3).unsqueeze(1), (out_h, out_w), mode="bicubic").squeeze(1) on CUDA."""
+    _chk("pred", pred)
+    if pred.dim() != 3:
+        raise ValueError(f"pred must be [B,h,w], got {tuple(pred.shape)}")
+    B, h, w = pred.shape
+    out = torch.empty((B, int(out_h), int(out_w)), dtype=torch.float32, device=pred.device)
+    _call("decnet_bicubic_up3", pred, pred.data_ptr(), out.data_ptr(), B, h, w, int(out_h), int(out_w))
+    return out
+
+
 def dynup_pack(disp, left_fea):
     _chk("disp", disp)
     B, h, w = disp.shape

@@ -381,6 +381,12 @@ int decnet_dynup_glue_nhwc(const float *logits, const float *disp, float *out,
 int decnet_dynup_set_disp_nhwc(const float *disp, float *packed,
                                int B, int h, int w, int CP, int round_tf32, int pad, void *stream);
 
+/* Skip-stage up-sampling (row a15; modules/SparseDenseNetRefinementMask.py:143-144): pred fp32 [B,h,w] (contiguous) ->
+ * out fp32 [B,H,W] = F.interpolate(pred*3, (H, W), mode="bicubic", align_corners=False), bit for bit what ATen's CUDA
+ * kernel returns: v = pred*3 rounded first, source index (h/H)*(y+0.5)-0.5, A = -0.75, clamped border taps, the four
+ * rows interpolated along x, then along y.  Any output size (a row band of the map is not an exact x3). */
+int decnet_bicubic_up3(const float *pred, float *out, int B, int h, int w, int H, int W, void *stream);
+
 /* Tail of GenerateSparseMask (modules/submodule.py:363-369) for BOTH views in one launch each:
  *   decnet_sqdiff_pair : out_i = (a_i - b_i)^2, i = 0 (left), 1 (right); n elements each
  *   decnet_detail_head : logit = bias + sum_c w3[c] * x[b,c,h,w] (the 3->1 1x1 conv with BN folded; w3 is a HOST

@@ -5,8 +5,12 @@
 //   disp_to_u16      : the KITTI-style 16-bit disparity image demo.py:191-197 writes: clamp(pred * 256, 0, 65535)
 //                      truncated to uint16, cropped to the last ori_h rows / ori_w columns (the PNG deflate stays on the host).
 //   epe_3px          : modules/loss.py:427-437 `test_loss_func`: EPE and 3-px / 5 % error over 0 < gt < max_disp.
+//   mirror_swap_u8   : the input of the reverse direction of StereoMatcher's left-right check: (mirror(right), mirror(left)).
+//   lr_check         : the left-right consistency check itself, on the forward and mirrored reverse predictions.
+//                      Neither of the last two has a counterpart in the reference.
 #include "common.cuh"
 #include <algorithm>
+#include <cstdint>
 
 namespace decnet {
 namespace codec {
@@ -36,6 +40,15 @@ image_prepare_u8_kernel(const unsigned char *__restrict__ img, float *__restrict
     }
 }
 
+// demo.py:191-197 for one value: clamp(d * 256, 0, 65535) truncated; shared by disp_to_u16 and lr_check.
+__device__ __forceinline__ unsigned short disp_u16(float d)
+{
+    float v = __fmul_rn(d, 256.f);
+    v = v < 0.f ? 0.f : v;                                                 // also sends NaN comparisons' false branch through
+    v = v > 65535.f ? 65535.f : v;
+    return (unsigned short)(v == v ? v : 0.f);                             // truncation like numpy's astype('uint16')
+}
+
 __global__ void __launch_bounds__(kBlock)
 disp_to_u16_kernel(const float *__restrict__ pred, unsigned short *__restrict__ out, int H, int W, int oh, int ow, long long n)
 {
@@ -43,10 +56,75 @@ disp_to_u16_kernel(const float *__restrict__ pred, unsigned short *__restrict__ 
     if (i >= n) return;
     const int x = (int)(i % ow), y = (int)((i / ow) % oh);
     const long long b = i / ((long long)ow * oh);
-    float v = __fmul_rn(pred[(b * H + (H - oh + y)) * (long long)W + (W - ow + x)], 256.f);
-    v = v < 0.f ? 0.f : v;                                                 // also sends NaN comparisons' false branch through
-    v = v > 65535.f ? 65535.f : v;
-    out[i] = (unsigned short)(v == v ? v : 0.f);                           // truncation like numpy's astype('uint16')
+    out[i] = disp_u16(pred[(b * H + (H - oh + y)) * (long long)W + (W - ow + x)]);
+}
+
+// Reverse order of 4 RGB pixels held in 3 little-endian words: pixel k is bytes 3k..3k+2 of (a, b, c).
+__device__ __forceinline__ void reverse4(unsigned a, unsigned b, unsigned c, unsigned &o0, unsigned &o1, unsigned &o2)
+{
+    o0 = __byte_perm(c, b, 0x6321);                                        // p3 (c1 c2 c3), p2[0] (b2)
+    o1 = __byte_perm(__byte_perm(b, c, 0x0043), a, 0x3710);                // p2[1..2] (b3 c0), p1[0..1] (a3 b0)
+    o2 = __byte_perm(b, a, 0x6541);                                        // p1[2] (b1), p0 (a0 a1 a2)
+}
+
+// out_left = mirror(right), out_right = mirror(left) on uint8 RGB [B,h,w,3].  Each thread writes P output pixels of one row
+// (view 0: out_left, view 1: out_right): P = 16 as three 16-byte accesses, P = 4 as three words, P = 1 byte by byte.
+template <int P>
+__global__ void __launch_bounds__(kBlock)
+mirror_swap_u8_kernel(const unsigned char *__restrict__ left, const unsigned char *__restrict__ right,
+                      unsigned char *__restrict__ out_left, unsigned char *__restrict__ out_right, int w, long long rows)
+{
+    const int nc = w / P;                                                  // chunks per row (w % P == 0)
+    const long long per_view = rows * nc;
+    const long long i = (long long)blockIdx.x * kBlock + threadIdx.x;
+    if (i >= 2 * per_view) return;
+    const int view = (int)(i / per_view);
+    const long long j = i - view * per_view, row = j / nc;
+    const int c = (int)(j - row * nc);
+    const unsigned char *src = (view ? left : right) + (row * w + (w - (c + 1) * P)) * 3;    // the mirrored chunk, read forward
+    unsigned char *dst = (view ? out_right : out_left) + (row * w + c * P) * 3;
+    if constexpr (P == 16) {
+        const uint4 *s = reinterpret_cast<const uint4 *>(src);
+        const uint4 v0 = __ldg(s), v1 = __ldg(s + 1), v2 = __ldg(s + 2);
+        const unsigned in[12] = {v0.x, v0.y, v0.z, v0.w, v1.x, v1.y, v1.z, v1.w, v2.x, v2.y, v2.z, v2.w};
+        unsigned o[12];
+#pragma unroll
+        for (int g = 0; g < 4; ++g)                                        // output group g = reversed input group 3 - g
+            reverse4(in[9 - 3 * g], in[10 - 3 * g], in[11 - 3 * g], o[3 * g], o[3 * g + 1], o[3 * g + 2]);
+        uint4 *d = reinterpret_cast<uint4 *>(dst);
+        d[0] = make_uint4(o[0], o[1], o[2], o[3]);
+        d[1] = make_uint4(o[4], o[5], o[6], o[7]);
+        d[2] = make_uint4(o[8], o[9], o[10], o[11]);
+    } else if constexpr (P == 4) {
+        const unsigned *s = reinterpret_cast<const unsigned *>(src);
+        unsigned *d = reinterpret_cast<unsigned *>(dst);
+        unsigned o0, o1, o2;
+        reverse4(__ldg(s), __ldg(s + 1), __ldg(s + 2), o0, o1, o2);
+        d[0] = o0; d[1] = o1; d[2] = o2;
+    } else {
+        dst[0] = src[0]; dst[1] = src[1]; dst[2] = src[2];
+    }
+}
+
+// Left-right consistency check over the cropped pixels of the forward half of pred [2B,H,W]; the reverse half holds the
+// mirrored run, whose cropped and mirrored-back value at column u sits at padded column W-1-u (oracle/lr_check.py).
+__global__ void __launch_bounds__(kBlock)
+lr_check_kernel(const float *__restrict__ pred, int B, int H, int W, int oh, int ow, float tol, float *__restrict__ out_f32,
+                unsigned short *__restrict__ out_u16, unsigned char *__restrict__ out_valid, long long n)
+{
+    const long long i = (long long)blockIdx.x * kBlock + threadIdx.x;      // over B*oh*ow cropped pixels
+    if (i >= n) return;
+    const int x = (int)(i % ow), y = (int)((i / ow) % oh);
+    const long long b = i / ((long long)ow * oh);
+    const float *fwd = pred + (b * H + (H - oh + y)) * (long long)W;
+    const float *rev = pred + ((b + B) * H + (H - oh + y)) * (long long)W;
+    const float dl = fwd[W - ow + x];
+    const float u = floorf(__fadd_rn(__fsub_rn((float)x, dl), 0.5f));      // NaN / inf dl fail every test below
+    bool valid = isfinite(dl) && u >= 0.f && u < (float)ow;
+    if (valid) valid = fabsf(__fsub_rn(dl, rev[W - 1 - (int)u])) <= tol;   // NaN dr: false
+    if (out_f32) out_f32[i] = valid ? dl : 0.f;
+    if (out_u16) out_u16[i] = valid ? disp_u16(dl) : (unsigned short)0;
+    if (out_valid) out_valid[i] = valid ? 1 : 0;
 }
 
 __global__ void __launch_bounds__(kBlock)
@@ -93,6 +171,39 @@ int decnet_disp_to_u16(const float *pred, unsigned short *out, int B, int H, int
     const long long n = (long long)B * ori_h * ori_w;
     disp_to_u16_kernel<<<(unsigned)((n + kBlock - 1) / kBlock), kBlock, 0, static_cast<cudaStream_t>(stream)>>>(pred, out, H, W, ori_h, ori_w, n);
     return after_launch("disp_to_u16_kernel");
+}
+
+int decnet_mirror_swap_u8(const unsigned char *left, const unsigned char *right, unsigned char *out_left,
+                          unsigned char *out_right, int B, int h, int w, void *stream)
+{
+    DECNET_REQUIRE(left && right && out_left && out_right, "null pointer");
+    DECNET_REQUIRE(B > 0 && h > 0 && w > 0, "empty image batch %dx%dx%d", B, h, w);
+    const long long rows = (long long)B * h;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    auto aligned = [&](unsigned a) {
+        return ((reinterpret_cast<uintptr_t>(left) | reinterpret_cast<uintptr_t>(right) | reinterpret_cast<uintptr_t>(out_left) |
+                 reinterpret_cast<uintptr_t>(out_right)) & (a - 1)) == 0;
+    };
+    auto grid = [&](int P) { return (unsigned)((2 * rows * (w / P) + kBlock - 1) / kBlock); };
+    if (w % 16 == 0 && aligned(16))                                        // rows and chunks start at multiples of 48 bytes
+        mirror_swap_u8_kernel<16><<<grid(16), kBlock, 0, st>>>(left, right, out_left, out_right, w, rows);
+    else if (w % 4 == 0 && aligned(4))
+        mirror_swap_u8_kernel<4><<<grid(4), kBlock, 0, st>>>(left, right, out_left, out_right, w, rows);
+    else
+        mirror_swap_u8_kernel<1><<<grid(1), kBlock, 0, st>>>(left, right, out_left, out_right, w, rows);
+    return after_launch("mirror_swap_u8_kernel");
+}
+
+int decnet_lr_check(const float *pred, int B, int H, int W, int ori_h, int ori_w, float tol, float *out_f32,
+                    unsigned short *out_u16, unsigned char *out_valid, void *stream)
+{
+    DECNET_REQUIRE(pred && (out_f32 || out_u16 || out_valid), "null prediction or no output requested");
+    DECNET_REQUIRE(B > 0 && ori_h > 0 && ori_w > 0 && ori_h <= H && ori_w <= W, "crop %dx%d outside the %dx%d map", ori_h, ori_w, H, W);
+    DECNET_REQUIRE(tol >= 0.f && tol <= 3.402823466e38f, "tolerance must be finite and >= 0");
+    const long long n = (long long)B * ori_h * ori_w;
+    lr_check_kernel<<<(unsigned)((n + kBlock - 1) / kBlock), kBlock, 0, static_cast<cudaStream_t>(stream)>>>(
+        pred, B, H, W, ori_h, ori_w, tol, out_f32, out_u16, out_valid, n);
+    return after_launch("lr_check_kernel");
 }
 
 int decnet_epe_3px(const float *pred, const float *gt, float max_disp, double *sums3, long long n, void *stream)

@@ -4,8 +4,10 @@ the current CUDA stream.  PyTorch is plumbing here (memory + streams), not the p
 from __future__ import annotations
 
 import math
+import numbers
 import os
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -301,6 +303,50 @@ def disp_to_u16(pred, ori_h, ori_w):
     out = torch.empty((B, int(ori_h), int(ori_w)), dtype=torch.uint16, device=pred.device)
     _call("decnet_disp_to_u16", pred, pred.data_ptr(), out.data_ptr(), B, H, W, int(ori_h), int(ori_w))
     return out
+
+
+def mirror_swap_u8(left, right, out_left, out_right):
+    """out_left = left view of the reverse direction = mirror(right), out_right = mirror(left) (mirror flips columns), all
+    contiguous CUDA uint8 [B,h,w,3]; writes into the given tensors (views of a larger buffer are fine) and returns them."""
+    shape = tuple(left.shape) if isinstance(left, torch.Tensor) else None
+    for name, t in (("left", left), ("right", right), ("out_left", out_left), ("out_right", out_right)):
+        if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.uint8 and t.is_contiguous() and t.dim() == 4
+                and t.shape[3] == 3):
+            raise ValueError(f"{name} must be a contiguous CUDA uint8 tensor [B,h,w,3]")
+        if tuple(t.shape) != shape or t.device != left.device:
+            raise ValueError(f"{name} {tuple(t.shape)} on {t.device} does not match left {shape} on {left.device}")
+    B, h, w, _ = shape
+    _call("decnet_mirror_swap_u8", left, left.data_ptr(), right.data_ptr(), out_left.data_ptr(), out_right.data_ptr(), B, h, w)
+    return out_left, out_right
+
+
+def lr_tolerance(tol):
+    """A left-right check tolerance in pixels as a float: a finite real number >= 0 that is not a bool, else ValueError."""
+    if isinstance(tol, (bool, np.bool_)) or not isinstance(tol, numbers.Real) or not math.isfinite(tol) or tol < 0:
+        raise ValueError(f"the left-right check tolerance must be a finite number of pixels >= 0, got {tol!r}")
+    return float(tol)
+
+
+def lr_check(pred, ori_h, ori_w, tol, float_out=True, u16_out=False, valid_out=False):
+    """Left-right consistency check (oracle/lr_check.py).  pred fp32 [2B,H,W]: the forward padded predictions, then
+    those of the mirrored, swapped pairs.  Returns a tuple of the requested [B,ori_h,ori_w] outputs, in this order:
+    float (the forward disparity where valid, else 0), uint16 (disp_to_u16's value where valid, else 0), bool valid."""
+    _chk("pred", pred)
+    if pred.dim() != 3 or pred.shape[0] % 2 or pred.shape[0] == 0:
+        raise ValueError(f"pred must be [2B,H,W] (forward then reverse), got {tuple(pred.shape)}")
+    B2, H, W = pred.shape
+    if not (0 < int(ori_h) <= H and 0 < int(ori_w) <= W):
+        raise ValueError(f"crop {ori_h}x{ori_w} outside the {H}x{W} map")
+    tol = lr_tolerance(tol)
+    if not (float_out or u16_out or valid_out):
+        raise ValueError("request at least one output")
+    shape, dev = (B2 // 2, int(ori_h), int(ori_w)), pred.device
+    f = torch.empty(shape, dtype=torch.float32, device=dev) if float_out else None
+    u = torch.empty(shape, dtype=torch.uint16, device=dev) if u16_out else None
+    v = torch.empty(shape, dtype=torch.bool, device=dev) if valid_out else None
+    _call("decnet_lr_check", pred, pred.data_ptr(), B2 // 2, H, W, int(ori_h), int(ori_w), float(tol),
+          *(t.data_ptr() if t is not None else None for t in (f, u, v)))
+    return tuple(t for t in (f, u, v) if t is not None)
 
 
 def epe_3px(pred, gt, max_disp):

@@ -4,12 +4,20 @@
     disp = m(left, right)                         # fp32 disparity in pixels, cropped to the input size
     png16 = m(left, right, output="u16")          # demo.py:191-197 (x256, uint16)
     for out in m.stream(pairs, output="u16"): ...
+    disp, valid = StereoMatcher(lr_check=1.0)(left, right, return_valid=True)   # left-right check: 0 where it fails
 
 Every call of one shape (B, h, w, max_disp) replays one CUDA graph of the whole step: uint8 -> pad / normalise ->
 feature extractor (both views, the right one on a forked stream) -> [image-space detail masks] -> decomposed matching.
 The graph is captured on the first call of a shape (after one eager run that builds the packed-weight caches), kept in
 an LRU cache of `max_graphs` shapes, and re-captured when any weight changed since its capture (the caches are only
 checked when Python runs forward, which a replay never does).
+
+With a left-right check (`lr_check` = a tolerance in pixels) the graph also runs the reverse direction: the model on the
+mirrored, swapped pair (mirror(right), mirror(left)), whose mirrored-back result is the right view's disparity.  Each
+buffer set then holds 2B pairs: the upload fills the first B, ops.mirror_swap_u8 writes the second B inside the graph, and
+the unchanged step runs at batch 2B.  ops.lr_check compares the two directions outside the graph, so the tolerance is a
+per-call argument that never re-captures.  It keeps the forward disparity where |dl - dr| <= tol at the matched column of
+the right view and writes 0 (KITTI's "no value") elsewhere: occluded pixels and matches outside the right image.
 
 The capture and the double-buffered loop of `stream()` restate bench.py's `capture` / `pipelined_e2e` on purpose:
 bench.py is the fixed measuring stick of the project and does not import the package's public API.
@@ -39,9 +47,10 @@ def round_max_disp(max_disp):
     return -(-int(max_disp) // MULTIPLE) * MULTIPLE
 
 
-def cache_key(B, h, w, max_disp, masks, precision):
-    """What one captured graph is specific to."""
-    return (int(B), int(h), int(w), int(max_disp), masks, precision)
+def cache_key(B, h, w, max_disp, masks, precision, lr=False):
+    """What one captured graph is specific to (a graph with the left-right check's reverse direction has a trailing "lr")."""
+    key = (int(B), int(h), int(w), int(max_disp), masks, precision)
+    return key + ("lr",) if lr else key
 
 
 def split_state_dict(state_dict, fe_keys, hot_keys):
@@ -98,11 +107,14 @@ def check_pair(left, right):
 
 
 class _Set:
-    """One captured graph with its static input / output buffers and pinned host staging."""
+    """One captured graph with its static input / output buffers and pinned host staging.  l, r are the B uploaded pairs;
+    with the left-right check they are the first halves of the graph's [2B,h,w,3] inputs xl, xr."""
 
-    def __init__(self, B, h, w, dev):
-        self.l = torch.empty((B, h, w, 3), dtype=torch.uint8, device=dev)
-        self.r = torch.empty_like(self.l)
+    def __init__(self, B, h, w, dev, lr=False):
+        self.lr = lr
+        self.xl = torch.empty(((2 if lr else 1) * B, h, w, 3), dtype=torch.uint8, device=dev)
+        self.xr = torch.empty_like(self.xl)
+        self.l, self.r = self.xl[:B], self.xr[:B]
         self.host_l = torch.empty((B, h, w, 3), dtype=torch.uint8).pin_memory()
         self.host_r = torch.empty_like(self.host_l).pin_memory()
         self.graph = self.pred = self.sig = None
@@ -119,10 +131,11 @@ class StereoMatcher:
     skip_stage_id 3 skips the finest level (bicubic x3 of the 1/3 disparity; Middlebury, demo.sh:5)
     precision     "fp32" (3xTF32 convs) or "tf32"
     max_graphs    shapes whose graphs are kept (least recently used evicted first)
+    lr_check      None (off) or the left-right check's tolerance in pixels (a finite number >= 0); a call may override it
     """
 
     def __init__(self, state_dict=None, max_disp=192, masks="learned", thold=0.9, detail_thold=0.3, skip_stage_id=4,
-                 precision="fp32", device="cuda", max_graphs=4):
+                 precision="fp32", device="cuda", max_graphs=4, lr_check=None):
         if masks not in MASKS:
             raise ValueError(f"masks must be one of {MASKS}, got {masks!r}")
         if precision not in PRECISIONS:
@@ -131,6 +144,7 @@ class StereoMatcher:
             raise ValueError(f"skip_stage_id must be 1..4, got {skip_stage_id!r}")
         if isinstance(max_graphs, bool) or not isinstance(max_graphs, int) or max_graphs < 1:
             raise ValueError(f"max_graphs must be a positive integer, got {max_graphs!r}")
+        self.lr_check = None if lr_check is None else ops.lr_tolerance(lr_check)
         dev = torch.device(device)
         if dev.type != "cuda":
             raise ValueError(f"device must be a CUDA device (decnet_b200 has no CPU path), got {device!r}")
@@ -183,6 +197,13 @@ class StereoMatcher:
         rm = ops.detail_detection(r01, 3, self.detail_thold)[::-1]
         return self.model(fl, fr, lm, rm)[0]
 
+    def _step(self, st):
+        """What the graph of a set runs: [the reverse direction's inputs, then] the step at the set's batch."""
+        if st.lr:
+            B = st.l.shape[0]
+            ops.mirror_swap_u8(st.l, st.r, st.xl[B:], st.xr[B:])
+        return self._forward(st.xl, st.xr)
+
     def _capture(self, st, max_disp):
         """One eager run on a side stream (it rebuilds any stale weight cache), then the capture (bench.py's capture)."""
         if st.graph is not None:
@@ -195,9 +216,9 @@ class StereoMatcher:
         try:
             side.wait_stream(main)
             with torch.cuda.stream(side):
-                self._forward(st.l, st.r)
+                self._step(st)
                 with torch.cuda.graph(graph, stream=side):
-                    st.pred = self._forward(st.l, st.r)
+                    st.pred = self._step(st)
             main.wait_stream(side)
             torch.cuda.synchronize(self.dev)
         finally:
@@ -218,7 +239,7 @@ class StereoMatcher:
         self._graphs.move_to_end(key)
         B, h, w = key[:3]
         while len(sets) < n:
-            sets.append(_Set(B, h, w, self.dev))
+            sets.append(_Set(B, h, w, self.dev, lr=key[-1] == "lr"))
         return sets
 
     def _replay(self, st, max_disp):
@@ -228,8 +249,12 @@ class StereoMatcher:
         st.graph.replay()
 
     # ------------------------------------------------------------------------------------------------------------ calls
-    def _result(self, st, h, w, output):
-        """Fresh device tensor (never the graph's static buffer) in the requested format, on the current stream."""
+    def _result(self, st, h, w, output, tol=None, return_valid=False):
+        """Fresh device tensor (never the graph's static buffer) in the requested format, on the current stream; with the
+        left-right check (tol) the checked disparity, or (disparity, valid) when return_valid."""
+        if st.lr:
+            out = ops.lr_check(st.pred, h, w, tol, float_out=output == "float", u16_out=output == "u16", valid_out=return_valid)
+            return out if return_valid else out[0]
         if output == "u16":
             return ops.disp_to_u16(st.pred, h, w)
         H, W = st.pred.shape[-2:]
@@ -238,20 +263,29 @@ class StereoMatcher:
     def _max_disp(self, max_disp):
         return self.max_disp if max_disp is None else round_max_disp(max_disp)
 
-    def __call__(self, left, right, output="float", max_disp=None):
+    def _lr(self, lr_check, return_valid):
+        """The call's left-right check tolerance (None: off), validated before any device work."""
+        tol = self.lr_check if lr_check is None else ops.lr_tolerance(lr_check)
+        if return_valid and tol is None:
+            raise ValueError("return_valid=True needs a left-right check: give lr_check to the matcher or the call")
+        return tol
+
+    def __call__(self, left, right, output="float", max_disp=None, lr_check=None, return_valid=False):
         """Disparity of one pair ([h,w,3]), a batch ([B,h,w,3]) or lists of single pairs (any sizes; one batch per
         distinct size, results in input order).  output "float" (pixels) or "u16" (x256, demo.py:191-197); the result
-        has the kind of the input (numpy, CPU tensor or CUDA tensor)."""
+        has the kind of the input (numpy, CPU tensor or CUDA tensor).  lr_check (None: the matcher's) is the left-right
+        check's tolerance in pixels; pixels that fail it are 0.  return_valid: each result is (disparity, bool valid)."""
         if output not in OUTPUTS:
             raise ValueError(f"output must be one of {OUTPUTS}, got {output!r}")
         D = self._max_disp(max_disp)
+        tol = self._lr(lr_check, return_valid)
         if isinstance(left, (list, tuple)):
-            return self._call_list(left, right, output, D)
+            return self._call_list(left, right, output, D, tol, return_valid)
         kind, batched, B, h, w = check_pair(left, right)
-        out = self._run(left, right, kind, B, h, w, output, D)
-        return out if batched else out[0]
+        out = self._run(left, right, kind, B, h, w, output, D, tol, return_valid)
+        return out if batched else _index(out, 0)
 
-    def _call_list(self, lefts, rights, output, D):
+    def _call_list(self, lefts, rights, output, D, tol, return_valid):
         if not isinstance(rights, (list, tuple)) or len(rights) != len(lefts):
             raise ValueError("left and right lists must have the same length")
         groups = OrderedDict()
@@ -263,9 +297,10 @@ class StereoMatcher:
         results = [None] * len(lefts)
         for (kind, h, w), idx in groups.items():
             stack = np.stack if kind == "numpy" else torch.stack
-            out = self._run(stack([lefts[i] for i in idx]), stack([rights[i] for i in idx]), kind, len(idx), h, w, output, D)
+            out = self._run(stack([lefts[i] for i in idx]), stack([rights[i] for i in idx]), kind, len(idx), h, w, output, D,
+                            tol, return_valid)
             for j, i in enumerate(idx):
-                results[i] = out[j]
+                results[i] = _index(out, j)
         return results
 
     def _upload(self, st, left, right, kind):
@@ -282,28 +317,32 @@ class StereoMatcher:
         st.r.copy_(st.host_r, non_blocking=True)
 
     @torch.no_grad()
-    def _run(self, left, right, kind, B, h, w, output, D):
+    def _run(self, left, right, kind, B, h, w, output, D, tol=None, return_valid=False):
         if kind == "cuda" and left.device != self.dev:
             raise ValueError(f"inputs are on {left.device}, the matcher on {self.dev}")
         with torch.cuda.device(self.dev):
-            st = self._sets(cache_key(B, h, w, D, self.masks, self.precision), 1)[0]
+            st = self._sets(cache_key(B, h, w, D, self.masks, self.precision, tol is not None), 1)[0]
             self._upload(st, left, right, kind)
             self._replay(st, D)
-            out = self._result(st, h, w, output)
+            out = self._result(st, h, w, output, tol, return_valid)
             if kind == "cuda":
                 return out
-            out = out.cpu()                                               # synchronous: the staging buffers are free again
-            return out.numpy() if kind == "numpy" else out
+            out = _map(lambda t: t.cpu(), out)                            # synchronous: the staging buffers are free again
+            return _map(lambda t: t.numpy(), out) if kind == "numpy" else out
 
-    @torch.no_grad()
-    def stream(self, pairs, output="float", max_disp=None):
+    def stream(self, pairs, output="float", max_disp=None, lr_check=None, return_valid=False):
         """Yield the result of each (left, right) of `pairs` in order, software-pipelined over two buffer sets per shape:
         while the graph of item i runs, the copy stream uploads item i+1 into the other set (bench.py's pipelined_e2e).
         Host results are read back through pinned memory and yielded as fresh arrays.  A change of shape drains the
-        pipeline and continues with the new shape's sets."""
+        pipeline and continues with the new shape's sets.  lr_check / return_valid as for a call."""
         if output not in OUTPUTS:
             raise ValueError(f"output must be one of {OUTPUTS}, got {output!r}")
         D = self._max_disp(max_disp)
+        tol = self._lr(lr_check, return_valid)
+        return self._stream(pairs, output, D, tol, return_valid)          # arguments checked now, not at the first item
+
+    @torch.no_grad()
+    def _stream(self, pairs, output, D, tol, return_valid):
         with torch.cuda.device(self.dev):
             if self._copy_stream is None:
                 self._copy_stream = torch.cuda.Stream(self.dev)
@@ -313,7 +352,7 @@ class StereoMatcher:
                 kind, batched, B, h, w = check_pair(left, right)
                 if kind == "cuda" and left.device != self.dev:
                     raise ValueError(f"inputs are on {left.device}, the matcher on {self.dev}")
-                k = cache_key(B, h, w, D, self.masks, self.precision)
+                k = cache_key(B, h, w, D, self.masks, self.precision, tol is not None)
                 if k != key:
                     while pending:
                         yield self._finish(pending.popleft())
@@ -339,11 +378,9 @@ class StereoMatcher:
                     st.uploaded.record(copy)
                 main.wait_event(st.uploaded)
                 self._replay(st, D)
-                res = self._result(st, h, w, output)
+                res = self._result(st, h, w, output, tol, return_valid)
                 if kind != "cuda":
-                    host = torch.empty(res.shape, dtype=res.dtype, pin_memory=True)
-                    host.copy_(res, non_blocking=True)
-                    res = host
+                    res = _map(_to_pinned, res)
                 st.computed = torch.cuda.Event()
                 st.computed.record(main)
                 if pending:
@@ -357,7 +394,22 @@ class StereoMatcher:
         done, res, kind, batched = item
         done.synchronize()
         if kind == "numpy":
-            res = res.numpy().copy()
+            res = _map(lambda t: t.numpy().copy(), res)
         elif kind == "cpu":
-            res = res.clone()
-        return res if batched else res[0]
+            res = _map(lambda t: t.clone(), res)
+        return res if batched else _index(res, 0)
+
+
+def _map(fn, out):
+    """fn over a result: one tensor, or the (disparity, valid) pair of return_valid."""
+    return tuple(fn(t) for t in out) if isinstance(out, tuple) else fn(out)
+
+
+def _index(out, i):
+    return _map(lambda t: t[i], out)
+
+
+def _to_pinned(t):
+    host = torch.empty(t.shape, dtype=t.dtype, pin_memory=True)
+    host.copy_(t, non_blocking=True)
+    return host

@@ -419,6 +419,22 @@ int decnet_image_prepare_u8(const unsigned char *img_hwc, float *out01, float *o
 int decnet_disp_to_u16(const float *pred, unsigned short *out, int B, int H, int W, int ori_h, int ori_w, void *stream);
 int decnet_epe_3px(const float *pred, const float *gt, float max_disp, double *sums3, long long n, void *stream);
 
+/* Left-right consistency check of StereoMatcher (no counterpart in the reference; oracle/lr_check.py is the spec).
+ * The reverse disparity of a pair (L, R) is the model run on (mirror(R), mirror(L)), mirror = column flip, cropped like the
+ * forward one and mirrored back.
+ *   decnet_mirror_swap_u8: out_left[b] = mirror(right[b]), out_right[b] = mirror(left[b]) on uint8 RGB [B,h,w,3] -- the
+ *     reverse direction's input.  16-byte accesses when w % 16 == 0 and all pointers are 16-byte aligned, words when
+ *     w % 4 == 0 (4-byte aligned), bytes otherwise.
+ *   decnet_lr_check: pred fp32 [2B,H,W] padded predictions, images 0..B-1 forward, B..2B-1 the mirrored reverse.  Over the
+ *     cropped pixels (the last ori_h rows / ori_w columns), dl = forward, in fp32 without contraction:
+ *       u = floor((x - dl) + 0.5);  valid = isfinite(dl) && 0 <= u < ori_w && |dl - dr[u]| <= tol   (NaN dr: invalid)
+ *     where dr[u] is the reverse image's padded column W-1-u.  Outputs [B,ori_h,ori_w], each may be NULL (not all):
+ *     out_f32 = valid ? dl : 0, out_u16 = valid ? decnet_disp_to_u16's value of dl : 0, out_valid = valid (0 / 1 bytes). */
+int decnet_mirror_swap_u8(const unsigned char *left, const unsigned char *right, unsigned char *out_left,
+                          unsigned char *out_right, int B, int h, int w, void *stream);
+int decnet_lr_check(const float *pred, int B, int H, int W, int ori_h, int ori_w, float tol, float *out_f32,
+                    unsigned short *out_u16, unsigned char *out_valid, void *stream);
+
 /* SoftAttention conv input cat(left_fea, dense, sparse, left_mask, -var) -> [B,C+4,H,W]
  * (modules/SparseDenseNetRefinementMask.py:197).  C = 0 (left_fea may be NULL) packs only the four
  * single-channel maps -> [B,4,H,W], the second source of decnet_conv2d_tf32_nchw_cat. */

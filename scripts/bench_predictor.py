@@ -12,6 +12,12 @@
   bicubic_up3        bicubic_up3_kernel against F.interpolate(bicubic) at 675x972 -> 2025x2916: us per launch and the share of
                      the HBM bound (data-sheet 7.7 TB/s; the 23.6 MB output fits the 126 MB L2, so back-to-back launches are not
                      flushed between them)
+  *_lr               the same legs with the left-right check (lr_check=1.0: the reverse direction in the same graph at 2B,
+                     then lr_check_kernel), measured in the same process, alternating with the plain leg call by call
+                     (single pairs) or run by run (stream)
+  mirror_swap_u8,    the two kernels of the check at B = 8 SceneFlow pairs: us per launch and the share of the HBM bound on
+  lr_check           their algorithmic bytes (mirror: 2 * 2*B*h*w*3; lr_check: 4 + 4 bytes read per pixel plus the outputs),
+                     launches rotating over enough buffers (> 300 MB) that each one reads from HBM, not L2
 
     python scripts/bench_predictor.py --out DIR
 """
@@ -28,6 +34,7 @@ ROOT = Path(__file__).resolve().parents[1]
 sys.path.insert(0, str(ROOT))
 
 HBM_GBS = 7700.0
+LR_TOL = 1.0
 
 
 def gpu_info(torch):
@@ -86,6 +93,85 @@ def latency(torch, m, left, right, calls, warmup):
             "readback_host_ms": pct(down_ms, 0.5), "what_readback": "disp_to_u16 + D2H into a new numpy array, synchronised"}
 
 
+def latency_pair(torch, m, left, right, calls, warmup):
+    """latency() of the plain call and of the call with the left-right check, alternating call by call."""
+    from decnet_b200.predictor import cache_key
+    h, w = left.shape[:2]
+    legs = {"plain": {}, "lr": {"lr_check": LR_TOL}}
+    for kw in legs.values():
+        for _ in range(warmup):
+            m(left, right, output="u16", **kw)
+    ts = {k: [] for k in legs}
+    for _ in range(calls):
+        for k, kw in legs.items():
+            t0 = time.perf_counter()
+            m(left, right, output="u16", **kw)
+            ts[k].append((time.perf_counter() - t0) * 1e3)
+    sets = {k: m._graphs[cache_key(1, h, w, m.max_disp, m.masks, m.precision, k == "lr")][0] for k in legs}
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    n = max(10, calls // 8)
+    dev_ms = {k: [] for k in legs}
+    for _ in range(2):
+        for k, st in sets.items():
+            torch.cuda.synchronize()
+            e0.record()
+            for _ in range(n):
+                st.graph.replay()
+            e1.record()
+            torch.cuda.synchronize()
+            dev_ms[k].append(e0.elapsed_time(e1) / n)
+    out = {}
+    for k, st in sets.items():
+        tol = legs[k].get("lr_check")
+        down = []
+        for _ in range(20):
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            m._result(st, h, w, "u16", tol).cpu().numpy()
+            down.append((time.perf_counter() - t0) * 1e3)
+        out[k] = {"calls": calls, "warmup": warmup, "p50_ms": pct(ts[k], 0.5), "p90_ms": pct(ts[k], 0.9), "min_ms": min(ts[k]),
+                  "replay_device_ms": min(dev_ms[k]), "replay_device_ms_runs": dev_ms[k],
+                  "readback_host_ms": pct(down, 0.5),
+                  "what_readback": ("lr_check (u16) + D2H" if tol is not None else "disp_to_u16 + D2H") + ", synchronised"}
+    out["lr"]["lr_check"] = LR_TOL
+    out["lr_over_plain"] = {"p50": out["lr"]["p50_ms"] / out["plain"]["p50_ms"],
+                            "replay_device": out["lr"]["replay_device_ms"] / out["plain"]["replay_device_ms"]}
+    return out
+
+
+def kernel_us(torch, fn_of_set, nsets, n=96, reps=5):
+    """Device us per launch of fn_of_set(i), rotating i over nsets buffer sets: n launches captured in one CUDA graph (no host
+    overhead between them), best of `reps` timed replays."""
+    side = torch.cuda.Stream()
+    side.wait_stream(torch.cuda.current_stream())
+    with torch.cuda.stream(side):
+        for i in range(nsets):
+            fn_of_set(i)
+    torch.cuda.current_stream().wait_stream(side)
+    torch.cuda.synchronize()
+    g = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(g):
+        for i in range(n):
+            fn_of_set(i % nsets)
+    g.replay()
+    torch.cuda.synchronize()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    best = float("inf")
+    for _ in range(reps):
+        e0.record()
+        g.replay()
+        e1.record()
+        torch.cuda.synchronize()
+        best = min(best, e0.elapsed_time(e1) * 1e3 / n)
+    g.reset()
+    return best
+
+
+def hbm_share(nbytes, us):
+    return {"bytes": nbytes, "hbm_bound_us": nbytes / (HBM_GBS * 1e9) * 1e6,
+            "frac_of_hbm_bound": nbytes / (HBM_GBS * 1e9) / (us * 1e-6), "hbm_gbs_assumed": HBM_GBS}
+
+
 def run_bench_py():
     cmd = [sys.executable, str(ROOT / "bench.py"), "--gpus", "1", "--steps", "20", "--warmup", "5", "--no-cpu-baseline",
            "--no-extras"]
@@ -121,6 +207,8 @@ def main():
     m = StereoMatcher(max_disp=192)
     res["sceneflow_single"] = dict(latency(torch, m, l1, r1, args.calls, 10), shape="540x960 -> 540x972", max_disp=216,
                                    masks="learned")
+    res["sceneflow_single_lr"] = dict(latency_pair(torch, m, l1, r1, args.calls, 10), shape="540x960 -> 540x972",
+                                      max_disp=216, masks="learned")
     del m
     torch.cuda.empty_cache()
 
@@ -136,20 +224,35 @@ def main():
     pair = (l8.cpu(), r8.cpu())
     for _ in m.stream([pair] * 4, output="u16"):
         pass
-    n = args.stream_steps
-    torch.cuda.synchronize()
-    t0 = time.perf_counter()
-    for _ in m.stream([pair] * n, output="u16"):
+    for _ in m.stream([pair] * 4, output="u16", lr_check=LR_TOL):
         pass
-    el = time.perf_counter() - t0
+    n = args.stream_steps
+
+    def run(**kw):
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        for _ in m.stream([pair] * n, output="u16", **kw):
+            pass
+        return time.perf_counter() - t0
+    els = {"plain": [], "lr": []}
+    for _ in range(2):                                                   # alternating plain and LR runs
+        els["plain"].append(run())
+        els["lr"].append(run(lr_check=LR_TOL))
+    el = min(els["plain"])
     rate = B * n / el
+    rate_lr = B * n / min(els["lr"])
     e2e = res["bench_py"].get("e2e")
     res["sceneflow_stream"] = {"batch": B, "steps": n, "pairs_per_s": rate, "ms_per_step": el / n * 1e3,
                                "left_mask_density": [round(d, 4) for d in dens],
                                "bench_py_e2e_pairs_per_s": e2e if e2e is not None else "not measured",
                                "ratio_to_bench_py_e2e": rate / e2e if e2e else "not measured",
                                "what": "CPU uint8 tensors in -> pinned staging -> H2D on a copy stream -> graph -> disp_to_u16 -> "
-                                       "pinned D2H -> new tensor, two buffer sets; host clock over the whole loop"}
+                                       "pinned D2H -> new tensor, two buffer sets; host clock over the whole loop; best of two runs"}
+    res["sceneflow_stream_lr"] = {"batch": B, "steps": n, "lr_check": LR_TOL, "pairs_per_s": rate_lr,
+                                  "ms_per_step": min(els["lr"]) / n * 1e3,
+                                  "pairs_per_s_runs": {k: [B * n / e for e in v] for k, v in els.items()},
+                                  "lr_over_plain_step_time": rate / rate_lr,
+                                  "what": "as sceneflow_stream with the left-right check; runs alternate with the plain ones"}
     del m
     torch.cuda.empty_cache()
 
@@ -158,6 +261,8 @@ def main():
     m = StereoMatcher(max_disp=768, masks="image", skip_stage_id=3)
     res["middlebury_single"] = dict(latency(torch, m, lm, rm, 30, 3), shape="2000x2900 -> 2025x2916", max_disp=783,
                                     masks="image", skip_stage_id=3)
+    res["middlebury_single_lr"] = dict(latency_pair(torch, m, lm, rm, 30, 3), shape="2000x2900 -> 2025x2916",
+                                       max_disp=783, masks="image", skip_stage_id=3)
     del m
     torch.cuda.empty_cache()
 
@@ -187,6 +292,24 @@ def main():
                           "aten_note": "F.interpolate on pred*3 computed beforehand (the x3 multiply is not timed)",
                           "bytes": nbytes, "hbm_bound_us": nbytes / (HBM_GBS * 1e9) * 1e6,
                           "frac_of_hbm_bound": nbytes / (HBM_GBS * 1e9) / (ours * 1e-6), "hbm_gbs_assumed": HBM_GBS}
+
+    # 5. the left-right check's kernels at B = 8 SceneFlow pairs, rotating over buffer sets larger than L2 together
+    B, h, w, H, W, nsets = 8, 540, 960, 540, 972, 8
+    img = [[torch.randint(0, 256, (2 * B, h, w, 3), device=dev, dtype=torch.uint8) for _ in range(2)] for _ in range(nsets)]
+    ptr = [[t.data_ptr() for t in (a[:B], b[:B], a[B:], b[B:])] for a, b in img]
+    t_mirror = kernel_us(torch, lambda i: ops._call("decnet_mirror_swap_u8", img[i][0], *ptr[i], B, h, w), nsets)
+    res["mirror_swap_u8"] = dict(hbm_share(2 * 2 * B * h * w * 3, t_mirror), us=t_mirror, shape=f"{B}x{h}x{w}x3, both views",
+                                 path="16-byte (w % 16 == 0)", buffer_sets=nsets)
+    del img
+    preds = [torch.randn(2 * B, H, W, device=dev) * 20 + 40 for _ in range(nsets)]
+    for name, out_bytes in (("u16", 2), ("float_valid", 5)):
+        outs = [(torch.empty(B, h, w, device=dev) if name == "float_valid" else None,
+                 torch.empty(B, h, w, dtype=torch.uint16, device=dev) if name == "u16" else None,
+                 torch.empty(B, h, w, dtype=torch.bool, device=dev) if name == "float_valid" else None) for _ in range(nsets)]
+        t = kernel_us(torch, lambda i: ops._call("decnet_lr_check", preds[i], preds[i].data_ptr(), B, H, W, h, w, LR_TOL,
+                                                 *(o.data_ptr() if o is not None else None for o in outs[i])), nsets)
+        res[f"lr_check_{name}"] = dict(hbm_share(B * h * w * (8 + out_bytes), t), us=t, shape=f"pred {2 * B}x{H}x{W} -> {B}x{h}x{w}",
+                                       outputs=name, buffer_sets=nsets)
     (out / "bench_predictor.json").write_text(json.dumps(res, indent=1))
     print(json.dumps(res))
 

@@ -79,6 +79,7 @@ SIGNATURES = {
     "decnet_epe_3px": (_i, [_f32p] * 2 + [C.c_float, _f32p, C.c_longlong, C.c_void_p]),
     "decnet_mirror_swap_u8": (_i, [_f32p] * 4 + [_i] * 3 + [C.c_void_p]),
     "decnet_lr_check": (_i, [_f32p] + [_i] * 5 + [C.c_float] + [_f32p] * 3 + [C.c_void_p]),
+    "decnet_lr_check_fill": (_i, [_f32p] + [_i] * 5 + [C.c_float] + [_f32p] * 4 + [C.c_void_p]),
     "decnet_attn_pack": (_i, [_f32p] * 6 + [_i] * 4 + [C.c_void_p]),
     "decnet_blend": (_i, [_f32p] * 5 + [_i] * 3 + [C.c_void_p]),
     "decnet_warp_bilinear": (_i, [_f32p] * 3 + [_i] * 4 + [C.c_void_p]),

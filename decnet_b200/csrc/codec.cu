@@ -7,7 +7,9 @@
 //   epe_3px          : modules/loss.py:427-437 `test_loss_func`: EPE and 3-px / 5 % error over 0 < gt < max_disp.
 //   mirror_swap_u8   : the input of the reverse direction of StereoMatcher's left-right check: (mirror(right), mirror(left)).
 //   lr_check         : the left-right consistency check itself, on the forward and mirrored reverse predictions.
-//                      Neither of the last two has a counterpart in the reference.
+//   lr_check_fill    : the check fused with background hole filling of the pixels it rejects (oracle/lr_fill.py): a row
+//                      pass (check + nearest valid neighbours in the row) and a pass over the rows without a valid pixel.
+//                      None of the last three has a counterpart in the reference.
 #include "common.cuh"
 #include <algorithm>
 #include <cstdint>
@@ -40,7 +42,7 @@ image_prepare_u8_kernel(const unsigned char *__restrict__ img, float *__restrict
     }
 }
 
-// demo.py:191-197 for one value: clamp(d * 256, 0, 65535) truncated; shared by disp_to_u16 and lr_check.
+// demo.py:191-197 for one value: clamp(d * 256, 0, 65535) truncated; shared by disp_to_u16, lr_check and the fill kernels.
 __device__ __forceinline__ unsigned short disp_u16(float d)
 {
     float v = __fmul_rn(d, 256.f);
@@ -106,8 +108,19 @@ mirror_swap_u8_kernel(const unsigned char *__restrict__ left, const unsigned cha
     }
 }
 
+// Whether one cropped pixel passes the left-right check (oracle/lr_check.py): x is its column in the crop, rev the padded row
+// of the mirrored reverse prediction, whose value at crop column u sits at padded column W-1-u.
+// dl = fwd[W - ow + x] is the forward value, loaded by the caller.  Shared by lr_check and lr_check_fill_rows.
+__device__ __forceinline__ bool lr_valid(float dl, const float *rev, int W, int ow, int x, float tol)
+{
+    const float u = floorf(__fadd_rn(__fsub_rn((float)x, dl), 0.5f));      // NaN / inf dl fail every test below
+    const bool inside = isfinite(dl) && u >= 0.f && u < (float)ow;
+    const float dr = rev[W - 1 - (inside ? (int)u : 0)];                   // unconditional: a caller's loads can overlap
+    return inside && fabsf(__fsub_rn(dl, dr)) <= tol;                      // NaN dr: false
+}
+
 // Left-right consistency check over the cropped pixels of the forward half of pred [2B,H,W]; the reverse half holds the
-// mirrored run, whose cropped and mirrored-back value at column u sits at padded column W-1-u (oracle/lr_check.py).
+// mirrored run.
 __global__ void __launch_bounds__(kBlock)
 lr_check_kernel(const float *__restrict__ pred, int B, int H, int W, int oh, int ow, float tol, float *__restrict__ out_f32,
                 unsigned short *__restrict__ out_u16, unsigned char *__restrict__ out_valid, long long n)
@@ -119,12 +132,193 @@ lr_check_kernel(const float *__restrict__ pred, int B, int H, int W, int oh, int
     const float *fwd = pred + (b * H + (H - oh + y)) * (long long)W;
     const float *rev = pred + ((b + B) * H + (H - oh + y)) * (long long)W;
     const float dl = fwd[W - ow + x];
-    const float u = floorf(__fadd_rn(__fsub_rn((float)x, dl), 0.5f));      // NaN / inf dl fail every test below
-    bool valid = isfinite(dl) && u >= 0.f && u < (float)ow;
-    if (valid) valid = fabsf(__fsub_rn(dl, rev[W - 1 - (int)u])) <= tol;   // NaN dr: false
+    const bool valid = lr_valid(dl, rev, W, ow, x, tol);
     if (out_f32) out_f32[i] = valid ? dl : 0.f;
     if (out_u16) out_u16[i] = valid ? disp_u16(dl) : (unsigned short)0;
     if (out_valid) out_valid[i] = valid ? 1 : 0;
+}
+
+// Background hole filling (oracle/lr_fill.py), row phase, fused with the check: one CTA per cropped row (b, y).  An invalid
+// pixel takes the smaller value of its nearest valid neighbours L (left) and R (right) in the row -- R's only when strictly
+// smaller, so ties keep L's bits -- or the one that exists; valid pixels keep dl.
+// The row is processed in chunks of kFillChunk columns, thread t owning columns c0 + i*kBlock + t.  Per chunk the checked
+// values are staged in shared memory and the validity as one warp ballot per 32 columns; L and R come from a block-wide max
+// scan of valid column indices (carried from the previous chunks) and a min scan (carrying in the first valid column after
+// the chunk).  A row of up to kFillChunk columns (every row up to Middlebury's 2916 px) is one chunk and one pass over the
+// predictions.  For a wider row that first valid column after the chunk comes from a look-ahead that recomputes the check
+// ahead of the chunk; it only moves forward, so the row is swept at most twice.  A neighbour outside the chunk is valid, so
+// its value is its forward prediction, read back from pred.
+// out_f32 always receives the row-phase values (0 on a row without a valid pixel: lr_fill_empty_rows_kernel reads them),
+// out_u16 / out_valid when requested, row_flags[b*oh + y] whether the row has a valid pixel.
+constexpr int kFillItems = 16;                                             // columns per thread per chunk
+constexpr int kFillChunk = kBlock * kFillItems;                            // 4096 columns, 16 KB of staged values
+constexpr int kFillWarps = kBlock / 32;
+
+__global__ void __launch_bounds__(kBlock)
+lr_check_fill_rows_kernel(const float *__restrict__ pred, int B, int H, int W, int oh, int ow, float tol,
+                          float *__restrict__ out_f32, unsigned short *__restrict__ out_u16,
+                          unsigned char *__restrict__ out_valid, unsigned char *__restrict__ row_flags)
+{
+    __shared__ float sv[kFillChunk];                                       // checked values of the chunk (dl where valid)
+    __shared__ unsigned sbits[kFillItems * kFillWarps];                    // validity: ballot of entry e = i*kFillWarps + warp
+    __shared__ int spre[kFillItems * kFillWarps];                          // last valid column before entry e (-1: none)
+    __shared__ int ssuf[kFillItems * kFillWarps];                          // first valid column after entry e (ow: none)
+    __shared__ int scarry, snext;
+    const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    const long long row = blockIdx.x;                                      // b * oh + y
+    const long long b = row / oh;
+    const int y = (int)(row - b * oh);
+    const float *fwd = pred + (b * H + (H - oh + y)) * (long long)W;
+    const float *rev = pred + ((b + B) * H + (H - oh + y)) * (long long)W;
+    const float *fwd_crop = fwd + (W - ow);
+    const long long o = row * ow;
+    int carry = -1;                                                        // last valid column left of the chunk
+    int next = -1;                                                         // first valid column >= the chunk's end, once known
+
+    for (int c0 = 0; c0 < ow; c0 += kFillChunk) {
+        const int c1 = min(c0 + kFillChunk, ow);
+        if (c1 == ow) {
+            next = ow;
+        } else if (next < c1) {                                            // look ahead (rows wider than one chunk only)
+            if (t == 0) snext = ow;
+            __syncthreads();
+            for (int a = c1; a < ow; a += kFillChunk) {
+                int m = ow;
+#pragma unroll 1
+                for (int i = 0; i < kFillItems; ++i) {                     // a thread's columns ascend: its first hit is its min
+                    const int x = a + i * kBlock + t;
+                    if (x < ow && lr_valid(fwd_crop[x], rev, W, ow, x, tol)) { m = x; break; }
+                }
+                m = __reduce_min_sync(0xffffffffu, m);
+                if (lane == 0) atomicMin(&snext, m);
+                __syncthreads();
+                next = snext;
+                __syncthreads();                                           // every thread has read snext before the next atomics
+                if (next < ow) break;
+            }
+        }
+        const int nseg = (c1 - c0 + kBlock - 1) / kBlock, nent = nseg * kFillWarps;
+        unsigned vmask = 0;                                                // bit i: column c0 + i*kBlock + t is valid
+        for (int i0 = 0; i0 < nseg; i0 += 4) {                             // 4 columns per thread, their loads in flight together
+            float d[4];
+#pragma unroll
+            for (int k = 0; k < 4; ++k) d[k] = fwd_crop[min(c0 + (i0 + k) * kBlock + t, ow - 1)];
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const int x = c0 + (i0 + k) * kBlock + t, xc = min(x, ow - 1);
+                const bool v = (x < ow) & lr_valid(d[k], rev, W, ow, xc, tol);
+                vmask |= (unsigned)v << (i0 + k);
+                sv[(i0 + k) * kBlock + t] = v ? d[k] : 0.f;
+            }
+        }
+#pragma unroll
+        for (int i = 0; i < kFillItems; ++i) {
+            if (i >= nseg) break;
+            const unsigned bits = __ballot_sync(0xffffffffu, (vmask >> i) & 1u);
+            if (lane == 0) sbits[i * kFillWarps + warp] = bits;
+        }
+        __syncthreads();
+        if (warp < 2) {                                                    // warp 0: exclusive max scan, warp 1: min scan
+            // lane l owns entries 4l..4l+3 (column order); entry e covers columns c0 + (e / kFillWarps)*kBlock + (e % kFillWarps)*32 + 0..31
+            int agg[4];
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const int e = 4 * lane + k;
+                const unsigned bits = e < nent ? sbits[e] : 0u;
+                const int base = c0 + (e / kFillWarps) * kBlock + (e % kFillWarps) * 32;
+                agg[k] = warp == 0 ? (bits ? base + 31 - __clz(bits) : -1) : (bits ? base + __ffs(bits) - 1 : ow);
+            }
+            if (warp == 0) {
+                const int tot = max(max(agg[0], agg[1]), max(agg[2], agg[3]));
+                int incl = tot;
+                for (int s = 1; s < 32; s <<= 1) {
+                    const int u = __shfl_up_sync(0xffffffffu, incl, s);
+                    if (lane >= s) incl = max(incl, u);
+                }
+                int run = max(carry, __shfl_up_sync(0xffffffffu, incl, 1));
+                if (lane == 0) run = carry;
+#pragma unroll
+                for (int k = 0; k < 4; ++k) { spre[4 * lane + k] = run; run = max(run, agg[k]); }
+                if (lane == 31) scarry = run;
+            } else {
+                const int tot = min(min(agg[0], agg[1]), min(agg[2], agg[3]));
+                int incl = tot;
+                for (int s = 1; s < 32; s <<= 1) {
+                    const int u = __shfl_down_sync(0xffffffffu, incl, s);
+                    if (lane + s < 32) incl = min(incl, u);
+                }
+                int run = min(next, __shfl_down_sync(0xffffffffu, incl, 1));
+                if (lane == 31) run = next;
+#pragma unroll
+                for (int k = 3; k >= 0; --k) { ssuf[4 * lane + k] = run; run = min(run, agg[k]); }
+            }
+        }
+        __syncthreads();
+#pragma unroll
+        for (int i = 0; i < kFillItems; ++i) {
+            const int x = c0 + i * kBlock + t;
+            if (i >= nseg || x >= ow) break;
+            const int e = i * kFillWarps + warp, base = x - lane;
+            const unsigned bits = sbits[e];
+            const bool v = (bits >> lane) & 1u;
+            float d = sv[x - c0];
+            if (!v) {
+                const unsigned lo = bits & ((1u << lane) - 1u), hi = bits & ~((2u << lane) - 1u);
+                const int L = lo ? base + 31 - __clz(lo) : spre[e];
+                const int R = hi ? base + __ffs(hi) - 1 : ssuf[e];
+                const float dL = L < 0 ? 0.f : L >= c0 ? sv[L - c0] : fwd_crop[L];
+                const float dR = R >= ow ? 0.f : R < c1 ? sv[R - c0] : fwd_crop[R];
+                d = L < 0 ? dR : R >= ow ? dL : dR < dL ? dR : dL;         // neither: a row without a valid pixel, 0
+            }
+            out_f32[o + x] = d;
+            if (out_u16) out_u16[o + x] = disp_u16(d);
+            if (out_valid) out_valid[o + x] = v ? 1 : 0;
+        }
+        carry = scarry;
+        __syncthreads();                                                   // sv, sbits and scarry are rewritten by the next chunk
+    }
+    if (t == 0) row_flags[row] = carry >= 0 ? 1 : 0;
+}
+
+// Background hole filling, column phase: a row without a valid pixel (row_flags 0) in an image that has a non-empty row takes,
+// column by column, the smaller row-phase value of the nearest non-empty rows A (above) and C (below) -- C's only when
+// strictly smaller -- or the one that exists.  One CTA per cropped row; non-empty rows, the common case, exit at once.  It
+// reads the neighbours from the float rows the row phase wrote (the wrapper allocates them when only uint16 was asked for)
+// and writes disp_u16 of the chosen value: reading the uint16 rows instead would also be exact, since disp_u16 is monotone,
+// but would not give the float output.
+__global__ void __launch_bounds__(kBlock)
+lr_fill_empty_rows_kernel(int oh, int ow, float *__restrict__ out_f32, unsigned short *__restrict__ out_u16,
+                          const unsigned char *__restrict__ row_flags)
+{
+    const long long row = blockIdx.x;
+    if (row_flags[row]) return;
+    __shared__ int sa, sc;
+    const int t = threadIdx.x;
+    const long long b = row / oh;
+    const int y = (int)(row - b * oh);
+    const unsigned char *flags = row_flags + b * oh;
+    if (t == 0) { sa = -1; sc = oh; }
+    __syncthreads();
+    int a = -1, c = oh;
+    for (int yy = t; yy < oh; yy += kBlock)
+        if (flags[yy]) {
+            if (yy < y) a = yy;                                            // ascending: the last hit above is the nearest
+            else if (c == oh) c = yy;
+        }
+    a = __reduce_max_sync(0xffffffffu, a);
+    c = __reduce_min_sync(0xffffffffu, c);
+    if ((t & 31) == 0) { atomicMax(&sa, a); atomicMin(&sc, c); }
+    __syncthreads();
+    a = sa; c = sc;
+    if (a < 0 && c == oh) return;                                          // no valid pixel in the image: it stays 0
+    const float *ra = out_f32 + (b * oh + max(a, 0)) * (long long)ow, *rc = out_f32 + (b * oh + min(c, oh - 1)) * (long long)ow;
+    const long long o = row * ow;
+    for (int x = t; x < ow; x += kBlock) {
+        const float da = a < 0 ? 0.f : ra[x], dc = c == oh ? 0.f : rc[x];
+        const float d = a < 0 ? dc : c == oh ? da : dc < da ? dc : da;
+        out_f32[o + x] = d;
+        if (out_u16) out_u16[o + x] = disp_u16(d);
+    }
 }
 
 __global__ void __launch_bounds__(kBlock)
@@ -204,6 +398,22 @@ int decnet_lr_check(const float *pred, int B, int H, int W, int ori_h, int ori_w
     lr_check_kernel<<<(unsigned)((n + kBlock - 1) / kBlock), kBlock, 0, static_cast<cudaStream_t>(stream)>>>(
         pred, B, H, W, ori_h, ori_w, tol, out_f32, out_u16, out_valid, n);
     return after_launch("lr_check_kernel");
+}
+
+int decnet_lr_check_fill(const float *pred, int B, int H, int W, int ori_h, int ori_w, float tol, float *out_f32,
+                         unsigned short *out_u16, unsigned char *out_valid, unsigned char *row_flags, void *stream)
+{
+    DECNET_REQUIRE(pred && out_f32 && row_flags, "null prediction, float rows or row flags");
+    DECNET_REQUIRE(B > 0 && ori_h > 0 && ori_w > 0 && ori_h <= H && ori_w <= W, "crop %dx%d outside the %dx%d map", ori_h, ori_w, H, W);
+    DECNET_REQUIRE(tol >= 0.f && tol <= 3.402823466e38f, "tolerance must be finite and >= 0");
+    const long long rows = (long long)B * ori_h;
+    DECNET_REQUIRE(rows <= 0x7fffffffLL, "%lld rows exceed the grid", rows);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    lr_check_fill_rows_kernel<<<(unsigned)rows, kBlock, 0, st>>>(pred, B, H, W, ori_h, ori_w, tol, out_f32, out_u16, out_valid,
+                                                                 row_flags);
+    if (int s = after_launch("lr_check_fill_rows_kernel")) return s;
+    lr_fill_empty_rows_kernel<<<(unsigned)rows, kBlock, 0, st>>>(ori_h, ori_w, out_f32, out_u16, row_flags);
+    return after_launch("lr_fill_empty_rows_kernel");
 }
 
 int decnet_epe_3px(const float *pred, const float *gt, float max_disp, double *sums3, long long n, void *stream)

@@ -327,10 +327,24 @@ def lr_tolerance(tol):
     return float(tol)
 
 
-def lr_check(pred, ori_h, ori_w, tol, float_out=True, u16_out=False, valid_out=False):
+LR_FILLS = ("none", "background")
+
+
+def lr_fill(fill):
+    """A hole-filling rule of the left-right check: one of LR_FILLS, else ValueError."""
+    if not isinstance(fill, str) or fill not in LR_FILLS:
+        raise ValueError(f"fill must be one of {LR_FILLS}, got {fill!r}")
+    return fill
+
+
+def lr_check(pred, ori_h, ori_w, tol, float_out=True, u16_out=False, valid_out=False, fill="none"):
     """Left-right consistency check (oracle/lr_check.py).  pred fp32 [2B,H,W]: the forward padded predictions, then
     those of the mirrored, swapped pairs.  Returns a tuple of the requested [B,ori_h,ori_w] outputs, in this order:
-    float (the forward disparity where valid, else 0), uint16 (disp_to_u16's value where valid, else 0), bool valid."""
+    float (the forward disparity where valid, else 0), uint16 (disp_to_u16's value where valid, else 0), bool valid.
+    fill="background" fills the invalid pixels from their valid neighbours instead of 0 (oracle/lr_fill.py: the smaller
+    value of the nearest valid pixels left and right in the row, then rows without one from the rows above and below);
+    valid stays the check's mask, False on every filled pixel."""
+    fill = lr_fill(fill)
     _chk("pred", pred)
     if pred.dim() != 3 or pred.shape[0] % 2 or pred.shape[0] == 0:
         raise ValueError(f"pred must be [2B,H,W] (forward then reverse), got {tuple(pred.shape)}")
@@ -341,12 +355,17 @@ def lr_check(pred, ori_h, ori_w, tol, float_out=True, u16_out=False, valid_out=F
     if not (float_out or u16_out or valid_out):
         raise ValueError("request at least one output")
     shape, dev = (B2 // 2, int(ori_h), int(ori_w)), pred.device
-    f = torch.empty(shape, dtype=torch.float32, device=dev) if float_out else None
+    f = torch.empty(shape, dtype=torch.float32, device=dev) if float_out or fill != "none" else None
     u = torch.empty(shape, dtype=torch.uint16, device=dev) if u16_out else None
     v = torch.empty(shape, dtype=torch.bool, device=dev) if valid_out else None
-    _call("decnet_lr_check", pred, pred.data_ptr(), B2 // 2, H, W, int(ori_h), int(ori_w), float(tol),
-          *(t.data_ptr() if t is not None else None for t in (f, u, v)))
-    return tuple(t for t in (f, u, v) if t is not None)
+    if fill == "none":
+        _call("decnet_lr_check", pred, pred.data_ptr(), B2 // 2, H, W, int(ori_h), int(ori_w), float(tol),
+              *(t.data_ptr() if t is not None else None for t in (f, u, v)))
+    else:                                                                  # the float rows are the fill's scratch too
+        flags = torch.empty(shape[:2], dtype=torch.uint8, device=dev)
+        _call("decnet_lr_check_fill", pred, pred.data_ptr(), B2 // 2, H, W, int(ori_h), int(ori_w), float(tol),
+              *(t.data_ptr() if t is not None else None for t in (f, u, v)), flags.data_ptr())
+    return tuple(t for t, want in ((f, float_out), (u, u16_out), (v, valid_out)) if want)
 
 
 def epe_3px(pred, gt, max_disp):

@@ -5,6 +5,7 @@
     png16 = m(left, right, output="u16")          # demo.py:191-197 (x256, uint16)
     for out in m.stream(pairs, output="u16"): ...
     disp, valid = StereoMatcher(lr_check=1.0)(left, right, return_valid=True)   # left-right check: 0 where it fails
+    dense = StereoMatcher(lr_check=1.0, fill="background")(left, right)         # ... and its holes filled
 
 Every call of one shape (B, h, w, max_disp) replays one CUDA graph of the whole step: uint8 -> pad / normalise ->
 feature extractor (both views, the right one on a forked stream) -> [image-space detail masks] -> decomposed matching.
@@ -18,6 +19,10 @@ buffer set then holds 2B pairs: the upload fills the first B, ops.mirror_swap_u8
 the unchanged step runs at batch 2B.  ops.lr_check compares the two directions outside the graph, so the tolerance is a
 per-call argument that never re-captures.  It keeps the forward disparity where |dl - dr| <= tol at the matched column of
 the right view and writes 0 (KITTI's "no value") elsewhere: occluded pixels and matches outside the right image.
+fill="background" fills those pixels instead, in the same pass over the predictions (oracle/lr_fill.py): each takes the
+smaller disparity of its nearest valid neighbours in the row, because an occluded pixel belongs to the surface behind; a row
+without a valid pixel takes the rows above and below.  The mask `valid` stays the check's, so filled pixels are still told
+apart from measured ones.  The fill is also outside the graph: changing it never re-captures either.
 
 The capture and the double-buffered loop of `stream()` restate bench.py's `capture` / `pipelined_e2e` on purpose:
 bench.py is the fixed measuring stick of the project and does not import the package's public API.
@@ -132,10 +137,12 @@ class StereoMatcher:
     precision     "fp32" (3xTF32 convs) or "tf32"
     max_graphs    shapes whose graphs are kept (least recently used evicted first)
     lr_check      None (off) or the left-right check's tolerance in pixels (a finite number >= 0); a call may override it
+    fill          "none" (failing pixels are 0) or "background" (failing pixels filled from their valid neighbours; needs
+                  a left-right check); a call may override it
     """
 
     def __init__(self, state_dict=None, max_disp=192, masks="learned", thold=0.9, detail_thold=0.3, skip_stage_id=4,
-                 precision="fp32", device="cuda", max_graphs=4, lr_check=None):
+                 precision="fp32", device="cuda", max_graphs=4, lr_check=None, fill="none"):
         if masks not in MASKS:
             raise ValueError(f"masks must be one of {MASKS}, got {masks!r}")
         if precision not in PRECISIONS:
@@ -145,6 +152,7 @@ class StereoMatcher:
         if isinstance(max_graphs, bool) or not isinstance(max_graphs, int) or max_graphs < 1:
             raise ValueError(f"max_graphs must be a positive integer, got {max_graphs!r}")
         self.lr_check = None if lr_check is None else ops.lr_tolerance(lr_check)
+        self.fill = ops.lr_fill(fill)
         dev = torch.device(device)
         if dev.type != "cuda":
             raise ValueError(f"device must be a CUDA device (decnet_b200 has no CPU path), got {device!r}")
@@ -249,11 +257,12 @@ class StereoMatcher:
         st.graph.replay()
 
     # ------------------------------------------------------------------------------------------------------------ calls
-    def _result(self, st, h, w, output, tol=None, return_valid=False):
+    def _result(self, st, h, w, output, tol=None, return_valid=False, fill="none"):
         """Fresh device tensor (never the graph's static buffer) in the requested format, on the current stream; with the
-        left-right check (tol) the checked disparity, or (disparity, valid) when return_valid."""
+        left-right check (tol) the checked disparity, holes filled by `fill`, or (disparity, valid) when return_valid."""
         if st.lr:
-            out = ops.lr_check(st.pred, h, w, tol, float_out=output == "float", u16_out=output == "u16", valid_out=return_valid)
+            out = ops.lr_check(st.pred, h, w, tol, float_out=output == "float", u16_out=output == "u16", valid_out=return_valid,
+                               fill=fill)
             return out if return_valid else out[0]
         if output == "u16":
             return ops.disp_to_u16(st.pred, h, w)
@@ -263,29 +272,34 @@ class StereoMatcher:
     def _max_disp(self, max_disp):
         return self.max_disp if max_disp is None else round_max_disp(max_disp)
 
-    def _lr(self, lr_check, return_valid):
-        """The call's left-right check tolerance (None: off), validated before any device work."""
+    def _lr(self, lr_check, return_valid, fill=None):
+        """The call's left-right check tolerance (None: off) and fill rule, validated before any device work."""
+        fill = None if fill is None else ops.lr_fill(fill)
         tol = self.lr_check if lr_check is None else ops.lr_tolerance(lr_check)
         if return_valid and tol is None:
             raise ValueError("return_valid=True needs a left-right check: give lr_check to the matcher or the call")
-        return tol
+        fill = self.fill if fill is None else fill
+        if fill != "none" and tol is None:
+            raise ValueError(f"fill needs a left-right check: give lr_check to the matcher or the call (fill={fill!r})")
+        return tol, fill
 
-    def __call__(self, left, right, output="float", max_disp=None, lr_check=None, return_valid=False):
+    def __call__(self, left, right, output="float", max_disp=None, lr_check=None, return_valid=False, fill=None):
         """Disparity of one pair ([h,w,3]), a batch ([B,h,w,3]) or lists of single pairs (any sizes; one batch per
         distinct size, results in input order).  output "float" (pixels) or "u16" (x256, demo.py:191-197); the result
         has the kind of the input (numpy, CPU tensor or CUDA tensor).  lr_check (None: the matcher's) is the left-right
-        check's tolerance in pixels; pixels that fail it are 0.  return_valid: each result is (disparity, bool valid)."""
+        check's tolerance in pixels; pixels that fail it are 0, or filled from their neighbours with fill="background"
+        (None: the matcher's fill).  return_valid: each result is (disparity, bool valid), valid False on filled pixels."""
         if output not in OUTPUTS:
             raise ValueError(f"output must be one of {OUTPUTS}, got {output!r}")
         D = self._max_disp(max_disp)
-        tol = self._lr(lr_check, return_valid)
+        tol, fill = self._lr(lr_check, return_valid, fill)
         if isinstance(left, (list, tuple)):
-            return self._call_list(left, right, output, D, tol, return_valid)
+            return self._call_list(left, right, output, D, tol, return_valid, fill)
         kind, batched, B, h, w = check_pair(left, right)
-        out = self._run(left, right, kind, B, h, w, output, D, tol, return_valid)
+        out = self._run(left, right, kind, B, h, w, output, D, tol, return_valid, fill)
         return out if batched else _index(out, 0)
 
-    def _call_list(self, lefts, rights, output, D, tol, return_valid):
+    def _call_list(self, lefts, rights, output, D, tol, return_valid, fill):
         if not isinstance(rights, (list, tuple)) or len(rights) != len(lefts):
             raise ValueError("left and right lists must have the same length")
         groups = OrderedDict()
@@ -298,7 +312,7 @@ class StereoMatcher:
         for (kind, h, w), idx in groups.items():
             stack = np.stack if kind == "numpy" else torch.stack
             out = self._run(stack([lefts[i] for i in idx]), stack([rights[i] for i in idx]), kind, len(idx), h, w, output, D,
-                            tol, return_valid)
+                            tol, return_valid, fill)
             for j, i in enumerate(idx):
                 results[i] = _index(out, j)
         return results
@@ -317,32 +331,32 @@ class StereoMatcher:
         st.r.copy_(st.host_r, non_blocking=True)
 
     @torch.no_grad()
-    def _run(self, left, right, kind, B, h, w, output, D, tol=None, return_valid=False):
+    def _run(self, left, right, kind, B, h, w, output, D, tol=None, return_valid=False, fill="none"):
         if kind == "cuda" and left.device != self.dev:
             raise ValueError(f"inputs are on {left.device}, the matcher on {self.dev}")
         with torch.cuda.device(self.dev):
             st = self._sets(cache_key(B, h, w, D, self.masks, self.precision, tol is not None), 1)[0]
             self._upload(st, left, right, kind)
             self._replay(st, D)
-            out = self._result(st, h, w, output, tol, return_valid)
+            out = self._result(st, h, w, output, tol, return_valid, fill)
             if kind == "cuda":
                 return out
             out = _map(lambda t: t.cpu(), out)                            # synchronous: the staging buffers are free again
             return _map(lambda t: t.numpy(), out) if kind == "numpy" else out
 
-    def stream(self, pairs, output="float", max_disp=None, lr_check=None, return_valid=False):
+    def stream(self, pairs, output="float", max_disp=None, lr_check=None, return_valid=False, fill=None):
         """Yield the result of each (left, right) of `pairs` in order, software-pipelined over two buffer sets per shape:
         while the graph of item i runs, the copy stream uploads item i+1 into the other set (bench.py's pipelined_e2e).
         Host results are read back through pinned memory and yielded as fresh arrays.  A change of shape drains the
-        pipeline and continues with the new shape's sets.  lr_check / return_valid as for a call."""
+        pipeline and continues with the new shape's sets.  lr_check / return_valid / fill as for a call."""
         if output not in OUTPUTS:
             raise ValueError(f"output must be one of {OUTPUTS}, got {output!r}")
         D = self._max_disp(max_disp)
-        tol = self._lr(lr_check, return_valid)
-        return self._stream(pairs, output, D, tol, return_valid)          # arguments checked now, not at the first item
+        tol, fill = self._lr(lr_check, return_valid, fill)
+        return self._stream(pairs, output, D, tol, return_valid, fill)    # arguments checked now, not at the first item
 
     @torch.no_grad()
-    def _stream(self, pairs, output, D, tol, return_valid):
+    def _stream(self, pairs, output, D, tol, return_valid, fill):
         with torch.cuda.device(self.dev):
             if self._copy_stream is None:
                 self._copy_stream = torch.cuda.Stream(self.dev)
@@ -378,7 +392,7 @@ class StereoMatcher:
                     st.uploaded.record(copy)
                 main.wait_event(st.uploaded)
                 self._replay(st, D)
-                res = self._result(st, h, w, output, tol, return_valid)
+                res = self._result(st, h, w, output, tol, return_valid, fill)
                 if kind != "cuda":
                     res = _map(_to_pinned, res)
                 st.computed = torch.cuda.Event()

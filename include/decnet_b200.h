@@ -429,11 +429,21 @@ int decnet_epe_3px(const float *pred, const float *gt, float max_disp, double *s
  *     cropped pixels (the last ori_h rows / ori_w columns), dl = forward, in fp32 without contraction:
  *       u = floor((x - dl) + 0.5);  valid = isfinite(dl) && 0 <= u < ori_w && |dl - dr[u]| <= tol   (NaN dr: invalid)
  *     where dr[u] is the reverse image's padded column W-1-u.  Outputs [B,ori_h,ori_w], each may be NULL (not all):
- *     out_f32 = valid ? dl : 0, out_u16 = valid ? decnet_disp_to_u16's value of dl : 0, out_valid = valid (0 / 1 bytes). */
+ *     out_f32 = valid ? dl : 0, out_u16 = valid ? decnet_disp_to_u16's value of dl : 0, out_valid = valid (0 / 1 bytes).
+ *   decnet_lr_check_fill: the same check, then background hole filling of the invalid pixels (oracle/lr_fill.py is the
+ *     spec), each output a copy of a valid dl.  Row phase: an invalid pixel with valid neighbours L (nearest to the left)
+ *     and R (nearest to the right) in its row takes dl[R] if dl[R] < dl[L], else dl[L]; with one of them, its value.
+ *     Column phase: a row without a valid pixel takes, column by column, the same rule on the row-phase values of the
+ *     nearest rows above and below that have one.  An image without a valid pixel stays 0.  out_f32 and row_flags
+ *     [B,ori_h] are required (the column phase reads the float rows; row_flags = the row has a valid pixel); out_u16 =
+ *     decnet_disp_to_u16's value of the float output; out_valid is the check's mask, 0 on every filled pixel.  No limit on
+ *     ori_w beyond the check's. */
 int decnet_mirror_swap_u8(const unsigned char *left, const unsigned char *right, unsigned char *out_left,
                           unsigned char *out_right, int B, int h, int w, void *stream);
 int decnet_lr_check(const float *pred, int B, int H, int W, int ori_h, int ori_w, float tol, float *out_f32,
                     unsigned short *out_u16, unsigned char *out_valid, void *stream);
+int decnet_lr_check_fill(const float *pred, int B, int H, int W, int ori_h, int ori_w, float tol, float *out_f32,
+                         unsigned short *out_u16, unsigned char *out_valid, unsigned char *row_flags, void *stream);
 
 /* SoftAttention conv input cat(left_fea, dense, sparse, left_mask, -var) -> [B,C+4,H,W]
  * (modules/SparseDenseNetRefinementMask.py:197).  C = 0 (left_fea may be NULL) packs only the four

@@ -18,6 +18,11 @@
   mirror_swap_u8,    the two kernels of the check at B = 8 SceneFlow pairs: us per launch and the share of the HBM bound on
   lr_check           their algorithmic bytes (mirror: 2 * 2*B*h*w*3; lr_check: 4 + 4 bytes read per pixel plus the outputs),
                      launches rotating over enough buffers (> 300 MB) that each one reads from HBM, not L2
+  lr_fill_*          the check fused with background hole filling (decnet_lr_check_fill: lr_check_fill_rows_kernel +
+                     lr_fill_empty_rows_kernel) at B = 8 SceneFlow pairs and one Middlebury pair, timed as lr_check_* in the
+                     same process beside an lr_check leg of the same shape; bytes: 8 read per pixel, written the float rows
+                     (always: the column phase reads them), the requested uint16 / valid outputs and one flag per row
+  sceneflow_stream_lr_fill  sceneflow_stream with the check and fill="background", runs alternating with the plain and _lr ones
 
     python scripts/bench_predictor.py --out DIR
 """
@@ -226,6 +231,8 @@ def main():
         pass
     for _ in m.stream([pair] * 4, output="u16", lr_check=LR_TOL):
         pass
+    for _ in m.stream([pair] * 4, output="u16", lr_check=LR_TOL, fill="background"):
+        pass
     n = args.stream_steps
 
     def run(**kw):
@@ -234,10 +241,11 @@ def main():
         for _ in m.stream([pair] * n, output="u16", **kw):
             pass
         return time.perf_counter() - t0
-    els = {"plain": [], "lr": []}
-    for _ in range(2):                                                   # alternating plain and LR runs
+    els = {"plain": [], "lr": [], "lr_fill": []}
+    for _ in range(2):                                                   # alternating plain, LR and LR + fill runs
         els["plain"].append(run())
         els["lr"].append(run(lr_check=LR_TOL))
+        els["lr_fill"].append(run(lr_check=LR_TOL, fill="background"))
     el = min(els["plain"])
     rate = B * n / el
     rate_lr = B * n / min(els["lr"])
@@ -253,6 +261,13 @@ def main():
                                   "pairs_per_s_runs": {k: [B * n / e for e in v] for k, v in els.items()},
                                   "lr_over_plain_step_time": rate / rate_lr,
                                   "what": "as sceneflow_stream with the left-right check; runs alternate with the plain ones"}
+    rate_fill = B * n / min(els["lr_fill"])
+    res["sceneflow_stream_lr_fill"] = {"batch": B, "steps": n, "lr_check": LR_TOL, "fill": "background", "pairs_per_s": rate_fill,
+                                       "ms_per_step": min(els["lr_fill"]) / n * 1e3,
+                                       "lr_fill_over_lr_step_time": rate_lr / rate_fill,
+                                       "what": "as sceneflow_stream_lr with fill=\"background\" (lr_check_fill_rows_kernel + "
+                                               "lr_fill_empty_rows_kernel instead of lr_check_kernel); runs alternate with the "
+                                               "plain and _lr ones"}
     del m
     torch.cuda.empty_cache()
 
@@ -310,6 +325,40 @@ def main():
                                                  *(o.data_ptr() if o is not None else None for o in outs[i])), nsets)
         res[f"lr_check_{name}"] = dict(hbm_share(B * h * w * (8 + out_bytes), t), us=t, shape=f"pred {2 * B}x{H}x{W} -> {B}x{h}x{w}",
                                        outputs=name, buffer_sets=nsets)
+    del preds
+    torch.cuda.empty_cache()
+
+    # 6. the check with background hole filling beside the check alone, at B = 8 SceneFlow pairs and one Middlebury pair
+    for tag, (B, h, w, H, W, nsets) in (("", (8, 540, 960, 540, 972, 8)), ("_middlebury", (1, 2000, 2900, 2025, 2916, 8))):
+        preds = [torch.randn(2 * B, H, W, device=dev) * 20 + 40 for _ in range(nsets)]
+        for name, out_bytes in (("u16", 2), ("float_valid", 5)):
+            outs = [(torch.empty(B, h, w, device=dev),
+                     torch.empty(B, h, w, dtype=torch.uint16, device=dev) if name == "u16" else None,
+                     torch.empty(B, h, w, dtype=torch.bool, device=dev) if name == "float_valid" else None,
+                     torch.empty(B, h, dtype=torch.uint8, device=dev)) for _ in range(nsets)]
+            chk = lambda i: ops._call("decnet_lr_check", preds[i], preds[i].data_ptr(), B, H, W, h, w, LR_TOL,
+                                      outs[i][0].data_ptr() if name == "float_valid" else None,
+                                      *(o.data_ptr() if o is not None else None for o in outs[i][1:3]))
+            fil = lambda i: ops._call("decnet_lr_check_fill", preds[i], preds[i].data_ptr(), B, H, W, h, w, LR_TOL,
+                                      *(o.data_ptr() if o is not None else None for o in outs[i]))
+            runs = {"check": [], "fill": []}
+            for _ in range(2):                                           # alternating, best of each
+                runs["check"].append(kernel_us(torch, chk, nsets))
+                runs["fill"].append(kernel_us(torch, fil, nsets))
+            t_chk, t_fill = min(runs["check"]), min(runs["fill"])
+            (valid,) = ops.lr_check(preds[0], h, w, LR_TOL, float_out=False, valid_out=True)
+            shape = f"pred {2 * B}x{H}x{W} -> {B}x{h}x{w}"
+            if tag:
+                res[f"lr_check_{name}{tag}"] = dict(hbm_share(B * h * w * (8 + out_bytes), t_chk), us=t_chk, shape=shape,
+                                                    outputs=name, buffer_sets=nsets, us_runs=runs["check"])
+            fill_bytes = B * h * w * (8 + 4 + (2 if name == "u16" else 1)) + B * h
+            res[f"lr_fill_{name}{tag}"] = dict(hbm_share(fill_bytes, t_fill), us=t_fill, shape=shape, outputs=name,
+                                               buffer_sets=nsets, us_runs=runs["fill"], lr_check_us=t_chk,
+                                               fill_over_check=t_fill / t_chk,
+                                               valid_fraction=float(valid.float().mean()),
+                                               what="decnet_lr_check_fill (both kernels) vs decnet_lr_check, alternating")
+        del preds
+        torch.cuda.empty_cache()
     (out / "bench_predictor.json").write_text(json.dumps(res, indent=1))
     print(json.dumps(res))
 

@@ -5,7 +5,7 @@ from __future__ import annotations
 
 import torch
 
-from . import _lib, ops
+from . import ops
 
 
 def _pad16(n: int) -> int:
@@ -42,21 +42,14 @@ def conv3d_layer(x, w, bias, np_, relu, residual=None, out=None, out_f32=False, 
     if out is None:
         out = (torch.empty((B, D, H, W), dtype=torch.float32, device=x.device) if out_f32
                else torch.empty((B, D, H, W, np_), dtype=torch.bfloat16, device=x.device))
+    res = residual.data_ptr() if residual is not None else None
     if band:
         assert not out_f32
-        with torch.cuda.device_of(x):
-            st = _lib.lib().decnet_conv3d_bf16_band(x.data_ptr(), w.data_ptr(), bias.data_ptr(),
-                                                    residual.data_ptr() if residual is not None else None, out.data_ptr(),
-                                                    B, D, H, W, cp, np_, 1 if relu else 0,
-                                                    torch.cuda.current_stream(x.device).cuda_stream)
-        _lib.check(st, "decnet_conv3d_bf16_band")
-        return out
-    with torch.cuda.device_of(x):
-        st = _lib.lib().decnet_conv3d_bf16(x.data_ptr(), w.data_ptr(), bias.data_ptr(),
-                                           residual.data_ptr() if residual is not None else None,
-                                           out.data_ptr(), 1 if out_f32 else 0, B, D, H, W, cp, np_, 1 if relu else 0,
-                                           torch.cuda.current_stream(x.device).cuda_stream)
-    _lib.check(st, "decnet_conv3d_bf16")
+        ops._call("decnet_conv3d_bf16_band", x, x.data_ptr(), w.data_ptr(), bias.data_ptr(), res, out.data_ptr(),
+                  B, D, H, W, cp, np_, 1 if relu else 0)
+    else:
+        ops._call("decnet_conv3d_bf16", x, x.data_ptr(), w.data_ptr(), bias.data_ptr(), res, out.data_ptr(),
+                  1 if out_f32 else 0, B, D, H, W, cp, np_, 1 if relu else 0)
     return out
 
 
@@ -78,11 +71,8 @@ def run_stack(reg, vol, with_pred=False):
     B, D, H, W, cp = t1.shape
     cost = torch.empty((B, D, H, W), dtype=torch.float32, device=t1.device)
     pred = torch.empty((B, H, W), dtype=torch.float32, device=t1.device)
-    with torch.cuda.device_of(t1):
-        st = _lib.lib().decnet_conv3d_bf16_softargmin(t1.data_ptr(), u[7][0].data_ptr(), u[7][1].data_ptr(), cost.data_ptr(),
-                                                      pred.data_ptr(), B, D, H, W, cp, u[7][2], 0,
-                                                      torch.cuda.current_stream(t1.device).cuda_stream)
-    _lib.check(st, "decnet_conv3d_bf16_softargmin")
+    ops._call("decnet_conv3d_bf16_softargmin", t1, t1.data_ptr(), u[7][0].data_ptr(), u[7][1].data_ptr(), cost.data_ptr(),
+              pred.data_ptr(), B, D, H, W, cp, u[7][2], 0)
     return pred, cost
 
 

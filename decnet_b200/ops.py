@@ -3,6 +3,7 @@ the current CUDA stream.  PyTorch is plumbing here (memory + streams), not the p
 """
 from __future__ import annotations
 
+import ctypes
 import math
 import numbers
 import os
@@ -15,6 +16,13 @@ from . import _lib
 
 def _stream(t: torch.Tensor) -> int:
     return torch.cuda.current_stream(t.device).cuda_stream
+
+
+def _call(name, t, *args):
+    """Call C entry `name` with args and the current stream, on t's device; raise DecnetError on a failed status."""
+    with torch.cuda.device_of(t):
+        st = getattr(_lib.lib(), name)(*args, _stream(t))
+    _lib.check(st, name)
 
 
 def _chk(name: str, t: torch.Tensor, ref: torch.Tensor | None = None, shape=None) -> None:
@@ -51,12 +59,10 @@ def spamat_forward(ref_feas, tar_feas, ref_mask, tar_mask, max_disp, output=None
     max_cost = torch.empty_like(ref_mask) if max_cost is None else max_cost
     for n, t in (("output", output), ("sum_similarities", sum_sim), ("max_cost", max_cost)):
         _chk(n, t, ref_feas, (B, H, W))
-    with torch.cuda.device_of(ref_feas):
-        st = _lib.lib().decnet_spamat_fwd(
-            ref_feas.data_ptr(), tar_feas.data_ptr(), ref_mask.data_ptr(), tar_mask.data_ptr(),
-            output.data_ptr(), sum_sim.data_ptr(), max_cost.data_ptr(),
-            B, Cc, H, W, int(max_disp), _stream(ref_feas))
-    _lib.check(st, "decnet_spamat_fwd")
+    _call("decnet_spamat_fwd", ref_feas,
+          ref_feas.data_ptr(), tar_feas.data_ptr(), ref_mask.data_ptr(), tar_mask.data_ptr(),
+          output.data_ptr(), sum_sim.data_ptr(), max_cost.data_ptr(),
+          B, Cc, H, W, int(max_disp))
     return output, sum_sim, max_cost
 
 
@@ -70,12 +76,10 @@ def spavar_forward(ref_feas, tar_feas, ref_mask, tar_mask, disparity, max_disp,
     max_cost = torch.empty_like(ref_mask) if max_cost is None else max_cost
     for n, t in (("output", output), ("sum_similarities", sum_sim), ("max_cost", max_cost)):
         _chk(n, t, ref_feas, (B, H, W))
-    with torch.cuda.device_of(ref_feas):
-        st = _lib.lib().decnet_spavar_fwd(
-            ref_feas.data_ptr(), tar_feas.data_ptr(), ref_mask.data_ptr(), tar_mask.data_ptr(),
-            disparity.data_ptr(), output.data_ptr(), sum_sim.data_ptr(), max_cost.data_ptr(),
-            B, Cc, H, W, int(max_disp), _stream(ref_feas))
-    _lib.check(st, "decnet_spavar_fwd")
+    _call("decnet_spavar_fwd", ref_feas,
+          ref_feas.data_ptr(), tar_feas.data_ptr(), ref_mask.data_ptr(), tar_mask.data_ptr(),
+          disparity.data_ptr(), output.data_ptr(), sum_sim.data_ptr(), max_cost.data_ptr(),
+          B, Cc, H, W, int(max_disp))
     return output, sum_sim, max_cost
 
 
@@ -83,19 +87,16 @@ def spamat_spavar_forward(ref_feas, tar_feas, ref_mask, tar_mask, max_disp):
     """Fused SpaMat + SpaVar(disparity = SpaMat output) -> (disp, var, sum_sim, max_cost)."""
     B, Cc, H, W = _feat_args(ref_feas, tar_feas, ref_mask, tar_mask)
     outs = [torch.empty_like(ref_mask) for _ in range(4)]
-    with torch.cuda.device_of(ref_feas):
-        st = _lib.lib().decnet_spamat_spavar_fwd(
-            ref_feas.data_ptr(), tar_feas.data_ptr(), ref_mask.data_ptr(), tar_mask.data_ptr(),
-            outs[0].data_ptr(), outs[1].data_ptr(), outs[2].data_ptr(), outs[3].data_ptr(),
-            B, Cc, H, W, int(max_disp), _stream(ref_feas))
-    _lib.check(st, "decnet_spamat_spavar_fwd")
+    _call("decnet_spamat_spavar_fwd", ref_feas,
+          ref_feas.data_ptr(), tar_feas.data_ptr(), ref_mask.data_ptr(), tar_mask.data_ptr(),
+          outs[0].data_ptr(), outs[1].data_ptr(), outs[2].data_ptr(), outs[3].data_ptr(),
+          B, Cc, H, W, int(max_disp))
     return tuple(outs)
 
 
 def spamat_spavar_forward_levels(levels):
     """Fused SpaMat + SpaVar of several pyramid levels in ONE launch.  levels: [(ref_feas, tar_feas, ref_mask, tar_mask,
     max_disp), ...] (finest level first for the best schedule) -> [(disp, var, sum_sim, max_cost), ...] in the same order."""
-    import ctypes
     n = len(levels)
     if not 1 <= n <= 4:
         raise ValueError("1..4 levels")
@@ -107,11 +108,10 @@ def spamat_spavar_forward_levels(levels):
         outs.append(tuple(torch.empty_like(ml) for _ in range(4)))
     vp = ctypes.c_void_p * n
     ia = ctypes.c_int * n
-    ptrs = [vp(*[lv[k].data_ptr() for lv in levels]) for k in range(4)] + [vp(*[o[k].data_ptr() for o in outs]) for k in range(4)]
-    ints = [ia(*[d[k] for d in dims]) for k in range(5)]
-    t0 = levels[0][0]
-    _call("decnet_spamat_spavar_fwd_levels", t0, n, *[ctypes.cast(p, ctypes.c_void_p) for p in ptrs],
-          *[ctypes.cast(i, ctypes.c_void_p) for i in ints])
+    _call("decnet_spamat_spavar_fwd_levels", levels[0][0], n,
+          *[vp(*[lv[k].data_ptr() for lv in levels]) for k in range(4)],
+          *[vp(*[o[k].data_ptr() for o in outs]) for k in range(4)],
+          *[ia(*[d[k] for d in dims]) for k in range(5)])
     return outs
 
 
@@ -125,12 +125,10 @@ def spamat_backward(ref_feas, tar_feas, ref_mask, tar_mask, output, sum_sim, max
     grad_tar = torch.zeros_like(tar_feas) if grad_tar is None else grad_tar
     _chk("grad_ref_feas", grad_ref, ref_feas, (B, Cc, H, W))
     _chk("grad_tar_feas", grad_tar, ref_feas, (B, Cc, H, W))
-    with torch.cuda.device_of(ref_feas):
-        st = _lib.lib().decnet_spamat_bwd(
-            ref_feas.data_ptr(), tar_feas.data_ptr(), ref_mask.data_ptr(), tar_mask.data_ptr(),
-            output.data_ptr(), sum_sim.data_ptr(), max_cost.data_ptr(), grad_output.data_ptr(),
-            grad_ref.data_ptr(), grad_tar.data_ptr(), B, Cc, H, W, int(max_disp), _stream(ref_feas))
-    _lib.check(st, "decnet_spamat_bwd")
+    _call("decnet_spamat_bwd", ref_feas,
+          ref_feas.data_ptr(), tar_feas.data_ptr(), ref_mask.data_ptr(), tar_mask.data_ptr(),
+          output.data_ptr(), sum_sim.data_ptr(), max_cost.data_ptr(), grad_output.data_ptr(),
+          grad_ref.data_ptr(), grad_tar.data_ptr(), B, Cc, H, W, int(max_disp))
     return grad_ref, grad_tar
 
 
@@ -146,13 +144,11 @@ def spavar_backward(ref_feas, tar_feas, ref_mask, tar_mask, disparity, output, s
     _chk("grad_ref_feas", grad_ref, ref_feas, (B, Cc, H, W))
     _chk("grad_tar_feas", grad_tar, ref_feas, (B, Cc, H, W))
     _chk("grad_disparity", grad_disp, ref_feas, (B, H, W))
-    with torch.cuda.device_of(ref_feas):
-        st = _lib.lib().decnet_spavar_bwd(
-            ref_feas.data_ptr(), tar_feas.data_ptr(), ref_mask.data_ptr(), tar_mask.data_ptr(),
-            disparity.data_ptr(), output.data_ptr(), sum_sim.data_ptr(), max_cost.data_ptr(),
-            grad_output.data_ptr(), grad_ref.data_ptr(), grad_tar.data_ptr(), grad_disp.data_ptr(),
-            B, Cc, H, W, int(max_disp), _stream(ref_feas))
-    _lib.check(st, "decnet_spavar_bwd")
+    _call("decnet_spavar_bwd", ref_feas,
+          ref_feas.data_ptr(), tar_feas.data_ptr(), ref_mask.data_ptr(), tar_mask.data_ptr(),
+          disparity.data_ptr(), output.data_ptr(), sum_sim.data_ptr(), max_cost.data_ptr(),
+          grad_output.data_ptr(), grad_ref.data_ptr(), grad_tar.data_ptr(), grad_disp.data_ptr(),
+          B, Cc, H, W, int(max_disp))
     return grad_ref, grad_tar, grad_disp
 
 
@@ -163,23 +159,14 @@ def candidate_signature(ref_mask, tar_mask, max_disp):
     B, H, W = ref_mask.shape
     count = torch.empty((B, H, W), dtype=torch.int32, device=ref_mask.device)
     hsh = torch.empty((B, H, W), dtype=torch.int64, device=ref_mask.device)
-    with torch.cuda.device_of(ref_mask):
-        st = _lib.lib().decnet_candidate_signature(
-            ref_mask.data_ptr(), tar_mask.data_ptr(), count.data_ptr(), hsh.data_ptr(),
-            B, H, W, int(max_disp), _stream(ref_mask))
-    _lib.check(st, "decnet_candidate_signature")
+    _call("decnet_candidate_signature", ref_mask,
+          ref_mask.data_ptr(), tar_mask.data_ptr(), count.data_ptr(), hsh.data_ptr(), B, H, W, int(max_disp))
     return count, hsh
 
 
 # --------------------------------------------------------------------------------------
 # dense stage + glue (SURVEY.md section 8 rows a2, a4, a6, a8, a13, a14)
 # --------------------------------------------------------------------------------------
-def _call(name, t, *args):
-    with torch.cuda.device_of(t):
-        st = getattr(_lib.lib(), name)(*args, _stream(t))
-    _lib.check(st, name)
-
-
 def cost_volume(left_fea, right_fea, D):
     """fp32 NCDHW cost volume [B,C,D,H,W] (reference layout)."""
     _chk("left_fea", left_fea)
@@ -261,7 +248,6 @@ def sigmoid_logit_threshold(thold, device):
 
 def detail_head(x_l, x_r, w3, bias, logit_thold):
     """masks (left, right) from the 3-channel maps in front of GenerateSparseMask's last 1x1 conv."""
-    import ctypes
     _chk("x_l", x_l)
     B, c, H, W = x_l.shape
     if c != 3:
@@ -269,9 +255,8 @@ def detail_head(x_l, x_r, w3, bias, logit_thold):
     _chk("x_r", x_r, x_l, (B, 3, H, W))
     ml = torch.empty((B, H, W), dtype=torch.float32, device=x_l.device)
     mr = torch.empty_like(ml)
-    w = (ctypes.c_float * 3)(*[float(v) for v in w3])
-    _call("decnet_detail_head", x_l, x_l.data_ptr(), x_r.data_ptr(), ctypes.cast(w, ctypes.c_void_p), float(bias),
-          float(logit_thold), ml.data_ptr(), mr.data_ptr(), B, H, W)
+    _call("decnet_detail_head", x_l, x_l.data_ptr(), x_r.data_ptr(), (ctypes.c_float * 3)(*[float(v) for v in w3]),
+          float(bias), float(logit_thold), ml.data_ptr(), mr.data_ptr(), B, H, W)
     return ml, mr
 
 
@@ -281,7 +266,6 @@ IMAGENET_MEAN, IMAGENET_STD = (0.485, 0.456, 0.406), (0.229, 0.224, 0.225)      
 def image_prepare_u8(img_u8, multiple=27, want01=True, want_norm=True, mean=IMAGENET_MEAN, std=IMAGENET_STD):
     """uint8 RGB [B,h,w,3] (CUDA) -> (img01, img_norm) fp32 [B,3,H,W], top/left zero-padded to multiples of
     `multiple` like demo.py:75-81; img01 = v/255, img_norm = (v/255 - mean)/std (demo.py:82-88)."""
-    import ctypes
     if not (isinstance(img_u8, torch.Tensor) and img_u8.is_cuda and img_u8.dtype == torch.uint8 and img_u8.is_contiguous()
             and img_u8.dim() == 4 and img_u8.shape[3] == 3):
         raise ValueError("img_u8 must be a contiguous CUDA uint8 tensor [B,h,w,3]")
@@ -289,10 +273,8 @@ def image_prepare_u8(img_u8, multiple=27, want01=True, want_norm=True, mean=IMAG
     H, W = -(-h // multiple) * multiple, -(-w // multiple) * multiple
     o01 = torch.empty((B, 3, H, W), dtype=torch.float32, device=img_u8.device) if want01 else None
     onm = torch.empty((B, 3, H, W), dtype=torch.float32, device=img_u8.device) if want_norm else None
-    m = (ctypes.c_float * 3)(*mean)
-    s = (ctypes.c_float * 3)(*std)
     _call("decnet_image_prepare_u8", img_u8, img_u8.data_ptr(), o01.data_ptr() if want01 else None,
-          onm.data_ptr() if want_norm else None, ctypes.cast(m, ctypes.c_void_p), ctypes.cast(s, ctypes.c_void_p), B, h, w, H, W)
+          onm.data_ptr() if want_norm else None, (ctypes.c_float * 3)(*mean), (ctypes.c_float * 3)(*std), B, h, w, H, W)
     return o01, onm
 
 
@@ -482,8 +464,6 @@ def refine_pack(left_fea, right_fea, disp):
 
 def haar_detail_masks(x, levels):
     """Haar lost-detail masks (row a7): x [B,1,H,W] -> ([mask_level1, ...] each [B,1,H/2^k,W/2^k], LL)."""
-    import ctypes
-    import numpy as np
     _chk("x", x)
     if x.dim() != 4 or x.shape[1] != 1:
         raise ValueError("x must be [B,1,H,W]")
@@ -496,8 +476,8 @@ def haar_detail_masks(x, levels):
         det = torch.empty_like(ll)
         mask = torch.empty_like(ll)
         ws = torch.empty(B * 12, dtype=torch.int32, device=x.device)
-        _call("decnet_haar_level", cur, cur.data_ptr(), ll.data_ptr(), det.data_ptr(), mask.data_ptr(), ws.data_ptr(),
-              ctypes.cast(th, ctypes.c_void_p), B, H, W)
+        _call("decnet_haar_level", cur, cur.data_ptr(), ll.data_ptr(), det.data_ptr(), mask.data_ptr(), ws.data_ptr(), th,
+              B, H, W)
         masks.append(mask)
         cur = ll
     return masks, cur
@@ -574,6 +554,18 @@ def _split_arg(split):
     return SPLIT_KIND if split else 0
 
 
+def _fp16_split(hi, lo):
+    """(sw, fp16(hi * 2^sw), fp16(lo * 2^(11+sw))): the weight halves of split kind 2's fp16 correction MMA.  sw is a 0-dim
+    int32 tensor on hi's device (no host sync: packing may run under stream capture) with max|hi| * 2^sw just below 2^13,
+    which brings the weights into fp16's exponent range with room on both sides."""
+    m = hi.abs().max()
+    e = torch.frexp(torch.where(torch.isfinite(m) & (m > 0), m, torch.ones_like(m)))[1]
+    sw = (13 - e).clamp(-40, 40).to(torch.int32)
+    wh = torch.ldexp(hi, sw).clamp(-65504.0, 65504.0).to(torch.float16)
+    wl = torch.ldexp(lo, sw + 11).clamp(-65504.0, 65504.0).to(torch.float16)
+    return sw, wh, wl
+
+
 def _pack_split_weights(out, bias_np):
     """out fp32 [T][NP][cp] -> ([2T][NP][cp] for the split modes of the channels-last kernel, bias [NP + 4]).
     Taps 0..T-1: the TF32 hi parts.  Taps T..2T-1, SPLIT_KIND 1: the TF32 lo parts; SPLIT_KIND 2: per 32-channel chunk of cl
@@ -587,9 +579,7 @@ def _pack_split_weights(out, bias_np):
         b[bias_np.numel()] = 1.0
         return torch.cat((hi, lo), 0).contiguous(), b
     T, np_, cp = out.shape
-    sw = _weight_scale_exp(hi)
-    wh = torch.ldexp(hi, sw).clamp(-65504.0, 65504.0).to(torch.float16)
-    wl = torch.ldexp(lo, sw + 11).clamp(-65504.0, 65504.0).to(torch.float16)
+    sw, wh, wl = _fp16_split(hi, lo)
     b2 = torch.zeros((T, np_, 2 * cp), dtype=torch.float16, device=out.device)
     for c0 in range(0, cp, 32):
         cl = min(32, cp - c0)
@@ -636,22 +626,26 @@ def padded_cat_channels(src_channels):
     return sum((c + 7) // 8 * 8 for c in src_channels)
 
 
+def _pad_cat_weights(w, src_channels, rows):
+    """[Cout,Cin,3,3] -> fp32 [rows >= Cout, padded_cat_channels(src_channels), 3, 3], zero-filled: the input is a
+    concatenation of tensors with these channel counts (sum = Cin), each padded to whole 8-channel chunks."""
+    cout, cin = w.shape[:2]
+    assert sum(src_channels) == cin, (src_channels, cin)
+    wp = torch.zeros((rows, padded_cat_channels(src_channels), 3, 3), dtype=torch.float32, device=w.device)
+    for j, c in enumerate(src_channels):
+        o, i = padded_cat_channels(src_channels[:j]), sum(src_channels[:j])
+        wp[:cout, o:o + c] = w[:, i:i + c].float()
+    return wp
+
+
 def pack_conv2d_tf32_nchw_weights(w, bias, src_channels=None, split=False):
     """[Cout,Cin,3,3] (+ bias [Cout]) -> (rows of 32 floats as include/decnet_b200.h describes, bias [CP]).
     src_channels: the input is a concatenation of tensors with these channel counts (sum = Cin), each
     padded to whole 8-channel chunks for decnet_conv2d_tc_nchw_cat.
     split: the hi rows followed by the lo rows (3xTF32 mode)."""
-    cout, cin = w.shape[:2]
-    wf = w.float()
-    if src_channels is not None and len(src_channels) > 1:
-        assert sum(src_channels) == cin, (src_channels, cin)
-        wp_ = torch.zeros((cout, padded_cat_channels(src_channels), 3, 3), dtype=torch.float32, device=w.device)
-        o = i = 0
-        for c in src_channels:
-            wp_[:, o:o + c] = wf[:, i:i + c]
-            o += (c + 7) // 8 * 8
-            i += c
-        wf, cin = wp_, wp_.shape[1]
+    cout = w.shape[0]
+    wf = _pad_cat_weights(w, src_channels, cout) if src_channels is not None and len(src_channels) > 1 else w.float()
+    cin = wf.shape[1]
     nck, cp = (cin + 7) // 8, (4 if cout <= 4 else (cout + 7) // 8 * 8)
     natoms = (3 * cp + 31) // 32
     # B[kh][ci][col = kw*CP + co]
@@ -673,14 +667,6 @@ def pack_conv2d_tf32_nchw_weights(w, bias, src_channels=None, split=False):
     return out.contiguous(), b.contiguous()
 
 
-def _weight_scale_exp(hi):
-    """sw (0-dim int32 tensor on hi's device, no host sync: packing may run under stream capture) with max|hi| * 2^sw just below
-    2^13: brings the weights into fp16's exponent range with room on both sides."""
-    m = hi.abs().max()
-    e = torch.frexp(torch.where(torch.isfinite(m) & (m > 0), m, torch.ones_like(m)))[1]
-    return (13 - e).clamp(-40, 40).to(torch.int32)
-
-
 def _pack_nchw_split16(blocks):
     """blocks fp32 [kh][chunk][atom][8 k][32 n] -> (hi rows then fp16 correction rows, 2^-(11+sw)): split kind 2 of the thin
     NCHW kernel.  All three products of a pixel carry the factor S = 2^(11+sw): the TF32 hi rows hold hi(w) * S, and each 1 KB
@@ -689,9 +675,7 @@ def _pack_nchw_split16(blocks):
     rows (SWIZZLE_128B_ATOM_32B: 32-byte unit ^= bits 7-8 of the address), so the 16-byte units of a block are stored
     pre-permuted: unit g of the global block holds logical unit s64(s128a32(g)), s64 = 16-byte unit ^= bits 7-8."""
     hi, lo = split_tf32(blocks)
-    sw = _weight_scale_exp(hi)
-    wh = torch.ldexp(hi, sw).clamp(-65504.0, 65504.0).to(torch.float16)
-    wl = torch.ldexp(lo, sw + 11).clamp(-65504.0, 65504.0).to(torch.float16)
+    sw, wh, wl = _fp16_split(hi, lo)
     kh, nck, natoms = blocks.shape[:3]
     logical = torch.stack((wh, wl), 3).contiguous()                                    # [kh][chunk][atom][2][8 k][32 n] halves
     units = logical.view(kh, nck, natoms, 64, 8)                                       # 64 sixteen-byte units per 1 KB block
@@ -711,32 +695,35 @@ def conv2d_tf32_nchw(x, w_packed, bias_padded, cout, dilation=1, relu=False):
     return out
 
 
-def conv2d_tf32_nchw_cat(srcs, w_packed, bias_padded, cout, dilation=1, relu=False, w_valid=0, split=False, addend=None):
-    """Conv over torch.cat(srcs, 1) without building it; srcs: 1..3 tensors [B,Ci,H,W] or [B,H,W] (one channel).
-    split: fp32-class operand split (w_packed from pack_conv2d_tf32_nchw_weights(split=True)).
-    addend [B,H,W] (cout == 1): added after the activation in the epilogue."""
-    import ctypes
+def _cat_srcs(srcs):
+    """The inputs of a convolution over torch.cat(srcs, 1): each [B,Ci,H,W] or [B,H,W] (one channel), on srcs[0]'s device
+    -> (srcs[0], B, H, W, device pointer array, channel count array, n) as the *_cat entry points take them."""
     x0 = srcs[0]
     _chk("srcs[0]", x0)
     B, H, W = x0.shape[0], x0.shape[-2], x0.shape[-1]
     chans = []
     for i, t in enumerate(srcs):
         _chk(f"srcs[{i}]", t, x0)
-        c = 1 if t.dim() == 3 else t.shape[1]
         if (t.shape[0], t.shape[-2], t.shape[-1]) != (B, H, W):
             raise ValueError(f"srcs[{i}] {tuple(t.shape)} does not match srcs[0] {tuple(x0.shape)}")
-        chans.append(int(c))
+        chans.append(1 if t.dim() == 3 else int(t.shape[1]))
     n = len(srcs)
-    ptrs = (ctypes.c_void_p * n)(*[t.data_ptr() for t in srcs])
-    cs = (ctypes.c_int * n)(*chans)
+    return x0, B, H, W, (ctypes.c_void_p * n)(*[t.data_ptr() for t in srcs]), (ctypes.c_int * n)(*chans), n
+
+
+def conv2d_tf32_nchw_cat(srcs, w_packed, bias_padded, cout, dilation=1, relu=False, w_valid=0, split=False, addend=None):
+    """Conv over torch.cat(srcs, 1) without building it; srcs: 1..3 tensors [B,Ci,H,W] or [B,H,W] (one channel).
+    split: fp32-class operand split (w_packed from pack_conv2d_tf32_nchw_weights(split=True)).
+    addend [B,H,W] (cout == 1): added after the activation in the epilogue."""
+    x0, B, H, W, ptrs, cs, n = _cat_srcs(srcs)
     out = torch.empty((B, int(cout), H, W), dtype=torch.float32, device=x0.device)
     if addend is not None:
         _chk("addend", addend, x0, (B, H, W))
         if int(cout) != 1:
             raise ValueError("addend only for single-channel outputs")
-    _call("decnet_conv2d_tc_nchw_cat_add", x0, ctypes.cast(ptrs, ctypes.c_void_p), ctypes.cast(cs, ctypes.c_void_p), n,
-          w_packed.data_ptr(), bias_padded.data_ptr(), addend.data_ptr() if addend is not None else None, out.data_ptr(),
-          B, int(cout), H, W, int(dilation), 1 if relu else 0, int(w_valid), _split_arg(split))
+    _call("decnet_conv2d_tc_nchw_cat_add", x0, ptrs, cs, n, w_packed.data_ptr(), bias_padded.data_ptr(),
+          addend.data_ptr() if addend is not None else None, out.data_ptr(), B, int(cout), H, W, int(dilation),
+          1 if relu else 0, int(w_valid), _split_arg(split))
     return out
 
 
@@ -749,40 +736,19 @@ def pack_conv2d_tf32_rows_weights(w, bias, src_channels=None):
     decnet_conv2d_tf32_rows_nchw_cat; every source of a concatenated input is padded to whole 8-channel chunks."""
     cout, cin = w.shape[:2]
     assert cout <= 8
-    chans = tuple(src_channels) if src_channels else (cin,)
-    assert sum(chans) == cin, (chans, cin)
-    cpad = padded_cat_channels(chans)
-    wf = torch.zeros((8, cpad, 3, 3), dtype=torch.float32, device=w.device)
-    o = i = 0
-    for c in chans:
-        wf[:cout, o:o + c] = w[:, i:i + c].float()
-        o += (c + 7) // 8 * 8
-        i += c
-    nck = cpad // 8
-    out = wf.view(8, nck, 8, 3, 3).permute(3, 4, 1, 0, 2).contiguous()          # [kh][kw][ck][co][ci]
-    out = ((out.view(torch.int32) + 0x1000) & ~0x1FFF).view(torch.float32)       # cvt.rna to TF32
+    wf = _pad_cat_weights(w, tuple(src_channels) if src_channels else (cin,), 8)
+    nck = wf.shape[1] // 8
+    out = rna_tf32(wf.view(8, nck, 8, 3, 3).permute(3, 4, 1, 0, 2))             # [kh][kw][ck][co][ci]
     b = torch.zeros(8, dtype=torch.float32, device=w.device)
     b[:cout] = bias.float()
     return out.contiguous(), b.contiguous()
 
 
 def conv2d_tf32_rows_nchw_cat(srcs, w_compact, bias8, cout, dilation=1, relu=False):
-    import ctypes
-    x0 = srcs[0]
-    _chk("srcs[0]", x0)
-    B, H, W = x0.shape[0], x0.shape[-2], x0.shape[-1]
-    chans = []
-    for i, t in enumerate(srcs):
-        _chk(f"srcs[{i}]", t, x0)
-        if (t.shape[0], t.shape[-2], t.shape[-1]) != (B, H, W):
-            raise ValueError(f"srcs[{i}] {tuple(t.shape)} does not match srcs[0] {tuple(x0.shape)}")
-        chans.append(1 if t.dim() == 3 else int(t.shape[1]))
-    n = len(srcs)
-    ptrs = (ctypes.c_void_p * n)(*[t.data_ptr() for t in srcs])
-    cs = (ctypes.c_int * n)(*chans)
+    x0, B, H, W, ptrs, cs, n = _cat_srcs(srcs)
     out = torch.empty((B, int(cout), H, W), dtype=torch.float32, device=x0.device)
-    _call("decnet_conv2d_tf32_rows_nchw_cat", x0, ctypes.cast(ptrs, ctypes.c_void_p), ctypes.cast(cs, ctypes.c_void_p), n,
-          w_compact.data_ptr(), bias8.data_ptr(), out.data_ptr(), B, int(cout), H, W, int(dilation), 1 if relu else 0)
+    _call("decnet_conv2d_tf32_rows_nchw_cat", x0, ptrs, cs, n, w_compact.data_ptr(), bias8.data_ptr(), out.data_ptr(),
+          B, int(cout), H, W, int(dilation), 1 if relu else 0)
     return out
 
 
@@ -803,22 +769,9 @@ def conv2d_tf32_nhwc_halo(x_pad, w_packed, bias, relu, round_out=False, split=Fa
 def nchw_cat_to_nhwc_pad(srcs, cp, round_tf32=True):
     """cat(srcs, 1) (NCHW, single-channel maps as [B,H,W]) -> zero-bordered channels-last [B,H+2,W+2,cp]
     (round_tf32: values rounded to TF32 for the halo kernel's plain-TF32 mode; its 3xTF32 mode takes them unrounded)."""
-    import ctypes
-    x0 = srcs[0]
-    _chk("srcs[0]", x0)
-    B, H, W = x0.shape[0], x0.shape[-2], x0.shape[-1]
-    chans = []
-    for i, t in enumerate(srcs):
-        _chk(f"srcs[{i}]", t, x0)
-        if (t.shape[0], t.shape[-2], t.shape[-1]) != (B, H, W):
-            raise ValueError(f"srcs[{i}] {tuple(t.shape)} does not match srcs[0] {tuple(x0.shape)}")
-        chans.append(1 if t.dim() == 3 else int(t.shape[1]))
-    n = len(srcs)
-    ptrs = (ctypes.c_void_p * n)(*[t.data_ptr() for t in srcs])
-    cs = (ctypes.c_int * n)(*chans)
+    x0, B, H, W, ptrs, cs, n = _cat_srcs(srcs)
     out = torch.empty((B, H + 2, W + 2, int(cp)), dtype=torch.float32, device=x0.device)
-    _call("decnet_nchw_cat_to_nhwc_pad", x0, ctypes.cast(ptrs, ctypes.c_void_p), ctypes.cast(cs, ctypes.c_void_p), n,
-          out.data_ptr(), B, H, W, int(cp), 1 if round_tf32 else 0)
+    _call("decnet_nchw_cat_to_nhwc_pad", x0, ptrs, cs, n, out.data_ptr(), B, H, W, int(cp), 1 if round_tf32 else 0)
     return out
 
 

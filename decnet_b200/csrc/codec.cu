@@ -9,7 +9,9 @@
 //   lr_check         : the left-right consistency check itself, on the forward and mirrored reverse predictions.
 //   lr_check_fill    : the check fused with background hole filling of the pixels it rejects (oracle/lr_fill.py): a row
 //                      pass (check + nearest valid neighbours in the row) and a pass over the rows without a valid pixel.
-//                      None of the last three has a counterpart in the reference.
+//   lr_check_guided_fill : lr_check_fill, then edge-aware filling guided by the left image (oracle/lr_guided.py): three
+//                      iterations of tridiagonal solves along every row and every column, and a compose pass.
+//                      None of the last four has a counterpart in the reference.
 #include "common.cuh"
 #include <algorithm>
 #include <cstdint>
@@ -321,6 +323,207 @@ lr_fill_empty_rows_kernel(int oh, int ow, float *__restrict__ out_f32, unsigned 
     }
 }
 
+// Edge-aware ("guided") hole filling (oracle/lr_guided.py): the fast global smoother's line solves over the background-
+// filled output of the two kernels above.  Every operation is an explicitly rounded intrinsic in the oracle's order, so
+// nothing is contracted into an FMA; subnormals are kept (the build has no -ftz), which the weight table and den need.
+// Scratch (decnet_lr_guided_fill_scratch_floats): the weight table, then five planes of B*h*w floats: the row and column
+// edge weights wh (pixel x to x+1, 0 in the last column) and wv (y to y+1, 0 in the last row), num, den and g (the solver's
+// g_i, kept for the back substitution).
+constexpr int kGuideTable = 766;                                           // k = sum_c |dI_c| in 0..765
+constexpr int kGuideTableFloats = 768;                                     // the planes after it stay 16-byte aligned
+constexpr int kGuideIters = 3;
+
+// w(k) = float32(exp(-k / sigma)) in double: every entry of sigma = 2.6 but w(0) = 1 lies more than 6e5 double ulps from a
+// float32 rounding boundary, so any double exp within a few ulps gives the oracle's table.
+__global__ void guided_table_kernel(double sigma, float *__restrict__ table)
+{
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k < kGuideTable) table[k] = (float)exp(-(double)k / sigma);
+}
+
+__device__ __forceinline__ int guide_l1(const unsigned char *p, const unsigned char *q)
+{
+    return abs((int)p[0] - (int)q[0]) + abs((int)p[1] - (int)q[1]) + abs((int)p[2] - (int)q[2]);
+}
+
+// Per cropped pixel: the edge weights to its right and lower neighbours, and the right-hand sides num = valid ? f : 0 and
+// den = valid ? 1 : 0 (f is the check's value on valid pixels).
+__global__ void __launch_bounds__(kBlock)
+guided_prep_kernel(const unsigned char *__restrict__ guide, const float *__restrict__ f, const unsigned char *__restrict__ valid,
+                   const float *__restrict__ table, int h, int w, long long n, float *__restrict__ wh, float *__restrict__ wv,
+                   float *__restrict__ num, float *__restrict__ den)
+{
+    const long long i = (long long)blockIdx.x * kBlock + threadIdx.x;      // over B*h*w pixels
+    if (i >= n) return;
+    const int x = (int)(i % w), y = (int)((i / w) % h);
+    const unsigned char *p = guide + i * 3;
+    wh[i] = x < w - 1 ? table[guide_l1(p, p + 3)] : 0.f;
+    wv[i] = y < h - 1 ? table[guide_l1(p, p + 3ll * w)] : 0.f;
+    const bool v = valid[i];
+    num[i] = v ? f[i] : 0.f;
+    den[i] = v ? 1.f : 0.f;
+}
+
+// One forward-elimination step of oracle.lr_guided.solve_line for both right-hand sides: a = lam_t * w(k_i), the carried
+// state is (a_(i-1), g_(i-1), y_(i-1) of num and den); in place: w -> g_i, fn -> y_i of num, fd -> y_i of den.
+__device__ __forceinline__ void thomas_step(float lt, float &w, float &fn, float &fd, float &ap, float &gp, float &yn, float &yd)
+{
+    const float a = __fmul_rn(lt, w);
+    const float m = __fsub_rn(__fadd_rn(__fadd_rn(1.f, ap), a), __fmul_rn(ap, gp));
+    const float r = __frcp_rn(m);
+    const float g = __fmul_rn(a, r);
+    yn = __fmul_rn(__fadd_rn(fn, __fmul_rn(ap, yn)), r);
+    yd = __fmul_rn(__fadd_rn(fd, __fmul_rn(ap, yd)), r);
+    ap = a; gp = g;
+    w = g; fn = yn; fd = yd;
+}
+
+// Back substitution x_i = y_i + g_i x_(i+1) (x_(n-1) = y_(n-1): last), in place on y.
+__device__ __forceinline__ void thomas_back(bool last, float g, float &yn, float &yd, float &xn, float &xd)
+{
+    if (!last) {
+        yn = __fadd_rn(yn, __fmul_rn(g, xn));
+        yd = __fadd_rn(yd, __fmul_rn(g, xd));
+    }
+    xn = yn; xd = yd;
+}
+
+__device__ __forceinline__ void cp_async_wait_one() { asm volatile("cp.async.wait_group 1;\n" ::: "memory"); }
+
+// Row solves of one iteration: one warp per 32 consecutive rows of the [B*h, w] planes, lane l solving row r0 + l.  The rows
+// pass through shared memory in 32 x 32 tiles (a warp's loads and stores stay coalesced, the lanes' reads are conflict-free
+// with the padded stride), double-buffered with cp.async: the next tile's loads are in flight while the current tile's
+// dependent chain of steps runs.  Forward: (w, num, den) -> (g, y_num, y_den), then backward over the tiles in reverse:
+// (g, y_num, y_den) -> x into num and den.
+constexpr int kRowTile = 32;
+
+__global__ void __launch_bounds__(32)
+guided_rows_kernel(const float *__restrict__ wh, float *num, float *den, float *gbuf, float lt, long long rows, int n)
+{
+    __shared__ float s[2][3][kRowTile][kRowTile + 1];
+    const int lane = threadIdx.x;
+    const long long r0 = (long long)blockIdx.x * kRowTile;
+    const int ntiles = (n + kRowTile - 1) / kRowTile;
+    auto load = [&](int tile, int buf, const float *p0, const float *p1, const float *p2) {
+        const int x = min(tile * kRowTile + lane, n - 1);
+#pragma unroll 4
+        for (int j = 0; j < kRowTile; ++j) {
+            const long long o = min(r0 + j, rows - 1) * n + x;
+            cp_async_4(&s[buf][0][j][lane], p0 + o);
+            cp_async_4(&s[buf][1][j][lane], p1 + o);
+            cp_async_4(&s[buf][2][j][lane], p2 + o);
+        }
+        cp_async_commit();
+    };
+    auto store = [&](int tile, int buf, float *p0, float *p1, float *p2) {
+        const int x = tile * kRowTile + lane;
+        __syncwarp();
+        if (x < n)
+            for (int j = 0; j < kRowTile && r0 + j < rows; ++j) {
+                const long long o = (r0 + j) * n + x;
+                if (p0) p0[o] = s[buf][0][j][lane];
+                p1[o] = s[buf][1][j][lane];
+                p2[o] = s[buf][2][j][lane];
+            }
+        __syncwarp();                                                      // the tile is read before a copy refills it
+    };
+
+    float ap = 0.f, gp = 0.f, yn = 0.f, yd = 0.f;
+    load(0, 0, wh, num, den);
+    for (int t = 0; t < ntiles; ++t) {
+        const int buf = t & 1;
+        if (t + 1 < ntiles) { load(t + 1, buf ^ 1, wh, num, den); cp_async_wait_one(); }
+        else cp_async_wait_all();
+        __syncwarp();
+        const int cnt = min(kRowTile, n - t * kRowTile);
+        float (*sw)[kRowTile + 1] = s[buf][0], (*sn)[kRowTile + 1] = s[buf][1], (*sd)[kRowTile + 1] = s[buf][2];
+#pragma unroll 8
+        for (int k = 0; k < cnt; ++k) thomas_step(lt, sw[lane][k], sn[lane][k], sd[lane][k], ap, gp, yn, yd);
+        store(t, buf, gbuf, num, den);
+    }
+    float xn = 0.f, xd = 0.f;
+    load(ntiles - 1, 0, gbuf, num, den);
+    for (int t = ntiles - 1, i = 0; t >= 0; --t, ++i) {
+        const int buf = i & 1;
+        if (t > 0) { load(t - 1, buf ^ 1, gbuf, num, den); cp_async_wait_one(); }
+        else cp_async_wait_all();
+        __syncwarp();
+        const int cnt = min(kRowTile, n - t * kRowTile);
+        float (*sg)[kRowTile + 1] = s[buf][0], (*sn)[kRowTile + 1] = s[buf][1], (*sd)[kRowTile + 1] = s[buf][2];
+#pragma unroll 8
+        for (int k = cnt - 1; k >= 0; --k) thomas_back(t * kRowTile + k == n - 1, sg[lane][k], sn[lane][k], sd[lane][k], xn, xd);
+        store(t, buf, nullptr, num, den);
+    }
+}
+
+// Column solves of one iteration: one thread per column of the [B, h, w] planes (a warp's accesses are 32 consecutive
+// columns of one row).  The next kColGroup rows' loads are issued before the current group's chain of steps.
+constexpr int kColGroup = 8;
+constexpr int kColBlock = 128;
+
+__global__ void __launch_bounds__(kColBlock)
+guided_cols_kernel(const float *__restrict__ wv, float *num, float *den, float *gbuf, float lt, int B, int h, int w)
+{
+    const long long col = (long long)blockIdx.x * kColBlock + threadIdx.x;
+    if (col >= (long long)B * w) return;
+    const long long b = col / w;
+    const long long base = b * h * (long long)w + (col - b * w);
+    auto at = [&](int y) { return base + (long long)min(max(y, 0), h - 1) * w; };
+    float cw[kColGroup], cn[kColGroup], cd[kColGroup];
+#pragma unroll
+    for (int k = 0; k < kColGroup; ++k) { const long long o = at(k); cw[k] = wv[o]; cn[k] = num[o]; cd[k] = den[o]; }
+    float ap = 0.f, gp = 0.f, yn = 0.f, yd = 0.f;
+    for (int y0 = 0; y0 < h; y0 += kColGroup) {
+        float nw[kColGroup], nn[kColGroup], nd[kColGroup];
+#pragma unroll
+        for (int k = 0; k < kColGroup; ++k) { const long long o = at(y0 + kColGroup + k); nw[k] = wv[o]; nn[k] = num[o]; nd[k] = den[o]; }
+#pragma unroll
+        for (int k = 0; k < kColGroup; ++k) {
+            if (y0 + k >= h) break;
+            thomas_step(lt, cw[k], cn[k], cd[k], ap, gp, yn, yd);
+            const long long o = at(y0 + k);
+            gbuf[o] = cw[k]; num[o] = cn[k]; den[o] = cd[k];
+        }
+#pragma unroll
+        for (int k = 0; k < kColGroup; ++k) { cw[k] = nw[k]; cn[k] = nn[k]; cd[k] = nd[k]; }
+    }
+    // backward, groups of kColGroup rows from the bottom: group q covers rows top - k, k = 0..kColGroup-1
+    int top = h - 1;
+#pragma unroll
+    for (int k = 0; k < kColGroup; ++k) { const long long o = at(top - k); cw[k] = gbuf[o]; cn[k] = num[o]; cd[k] = den[o]; }
+    float xn = 0.f, xd = 0.f;
+    for (; top >= 0; top -= kColGroup) {
+        float nw[kColGroup], nn[kColGroup], nd[kColGroup];
+#pragma unroll
+        for (int k = 0; k < kColGroup; ++k) { const long long o = at(top - kColGroup - k); nw[k] = gbuf[o]; nn[k] = num[o]; nd[k] = den[o]; }
+#pragma unroll
+        for (int k = 0; k < kColGroup; ++k) {
+            if (top - k < 0) break;
+            thomas_back(top - k == h - 1, cw[k], cn[k], cd[k], xn, xd);
+            const long long o = at(top - k);
+            num[o] = cn[k]; den[o] = cd[k];
+        }
+#pragma unroll
+        for (int k = 0; k < kColGroup; ++k) { cw[k] = nw[k]; cn[k] = nn[k]; cd[k] = nd[k]; }
+    }
+}
+
+// Compose: an invalid pixel whose den is a normal float takes num / den, any other keeps the background value out_f32
+// already holds (valid pixels keep their bits); out_u16 = disp_u16 of the result.
+__global__ void __launch_bounds__(kBlock)
+guided_compose_kernel(const float *__restrict__ num, const float *__restrict__ den, const unsigned char *__restrict__ valid,
+                      float *__restrict__ out_f32, unsigned short *__restrict__ out_u16, long long n)
+{
+    const long long i = (long long)blockIdx.x * kBlock + threadIdx.x;
+    if (i >= n) return;
+    float d = out_f32[i];
+    if (!valid[i]) {
+        const float c = den[i];
+        if (c >= 1.17549435e-38f) { d = __fdiv_rn(num[i], c); out_f32[i] = d; }   // 2^-126; NaN compares false
+    }
+    if (out_u16) out_u16[i] = disp_u16(d);
+}
+
 __global__ void __launch_bounds__(kBlock)
 epe_3px_kernel(const float *__restrict__ pred, const float *__restrict__ gt, float max_disp, double *__restrict__ sums, long long n)
 {
@@ -414,6 +617,45 @@ int decnet_lr_check_fill(const float *pred, int B, int H, int W, int ori_h, int 
     if (int s = after_launch("lr_check_fill_rows_kernel")) return s;
     lr_fill_empty_rows_kernel<<<(unsigned)rows, kBlock, 0, st>>>(ori_h, ori_w, out_f32, out_u16, row_flags);
     return after_launch("lr_fill_empty_rows_kernel");
+}
+
+long long decnet_lr_guided_fill_scratch_floats(int B, int ori_h, int ori_w)
+{
+    return kGuideTableFloats + 5 * (long long)B * ori_h * ori_w;           // table, wh, wv, num, den, g
+}
+
+int decnet_lr_check_guided_fill(const float *pred, const unsigned char *guide, int B, int H, int W, int ori_h, int ori_w,
+                                float tol, double lambda, double sigma_color, float *out_f32, unsigned short *out_u16,
+                                unsigned char *out_valid, unsigned char *row_flags, float *scratch, void *stream)
+{
+    DECNET_REQUIRE(pred && guide && out_f32 && out_valid && row_flags && scratch,
+                   "null prediction, guide, float rows, mask, row flags or scratch");
+    DECNET_REQUIRE(B > 0 && ori_h > 0 && ori_w > 0 && ori_h <= H && ori_w <= W, "crop %dx%d outside the %dx%d map", ori_h, ori_w, H, W);
+    DECNET_REQUIRE(tol >= 0.f && tol <= 3.402823466e38f, "tolerance must be finite and >= 0");
+    DECNET_REQUIRE(lambda >= 0.0 && lambda <= 1.7976931348623157e308, "lambda must be finite and >= 0");
+    DECNET_REQUIRE(sigma_color > 0.0 && sigma_color <= 1.7976931348623157e308, "sigma_color must be finite and > 0");
+    const long long rows = (long long)B * ori_h, n = rows * ori_w;
+    DECNET_REQUIRE(rows <= 0x7fffffffLL, "%lld rows exceed the grid", rows);
+    if (int s = decnet_lr_check_fill(pred, B, H, W, ori_h, ori_w, tol, out_f32, nullptr, out_valid, row_flags, stream)) return s;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    float *table = scratch, *wh = table + kGuideTableFloats, *wv = wh + n, *num = wv + n, *den = num + n, *g = den + n;
+    guided_table_kernel<<<(kGuideTable + kBlock - 1) / kBlock, kBlock, 0, st>>>(sigma_color, table);
+    if (int s = after_launch("guided_table_kernel")) return s;
+    const unsigned pix_grid = (unsigned)((n + kBlock - 1) / kBlock);
+    guided_prep_kernel<<<pix_grid, kBlock, 0, st>>>(guide, out_f32, out_valid, table, ori_h, ori_w, n, wh, wv, num, den);
+    if (int s = after_launch("guided_prep_kernel")) return s;
+    for (int t = 1; t <= kGuideIters; ++t) {
+        double q = 1.0;                                                    // 4^(T-t), exact
+        for (int k = t; k < kGuideIters; ++k) q *= 4.0;
+        const float lt = (float)(lambda * 1.5 * q / 63.0);                 // 63 = 4^T - 1; in the oracle's order
+        guided_rows_kernel<<<(unsigned)((rows + kRowTile - 1) / kRowTile), 32, 0, st>>>(wh, num, den, g, lt, rows, ori_w);
+        if (int s = after_launch("guided_rows_kernel")) return s;
+        guided_cols_kernel<<<(unsigned)(((long long)B * ori_w + kColBlock - 1) / kColBlock), kColBlock, 0, st>>>(
+            wv, num, den, g, lt, B, ori_h, ori_w);
+        if (int s = after_launch("guided_cols_kernel")) return s;
+    }
+    guided_compose_kernel<<<pix_grid, kBlock, 0, st>>>(num, den, out_valid, out_f32, out_u16, n);
+    return after_launch("guided_compose_kernel");
 }
 
 int decnet_epe_3px(const float *pred, const float *gt, float max_disp, double *sums3, long long n, void *stream)

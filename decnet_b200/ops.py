@@ -309,7 +309,9 @@ def lr_tolerance(tol):
     return float(tol)
 
 
-LR_FILLS = ("none", "background")
+LR_FILLS = ("none", "background", "guided")
+GUIDED_LAMBDA = 8000.0         # fill="guided": smoothness weight lambda of the fast global smoother (OpenCV's default)
+GUIDED_SIGMA = 2.6             # and its colour scale on the L1 colour distance (OpenCV's 1.5 on the Euclidean one, x sqrt(3))
 
 
 def lr_fill(fill):
@@ -319,14 +321,20 @@ def lr_fill(fill):
     return fill
 
 
-def lr_check(pred, ori_h, ori_w, tol, float_out=True, u16_out=False, valid_out=False, fill="none"):
+def lr_check(pred, ori_h, ori_w, tol, float_out=True, u16_out=False, valid_out=False, fill="none", guide=None):
     """Left-right consistency check (oracle/lr_check.py).  pred fp32 [2B,H,W]: the forward padded predictions, then
     those of the mirrored, swapped pairs.  Returns a tuple of the requested [B,ori_h,ori_w] outputs, in this order:
     float (the forward disparity where valid, else 0), uint16 (disp_to_u16's value where valid, else 0), bool valid.
     fill="background" fills the invalid pixels from their valid neighbours instead of 0 (oracle/lr_fill.py: the smaller
     value of the nearest valid pixels left and right in the row, then rows without one from the rows above and below);
-    valid stays the check's mask, False on every filled pixel."""
+    fill="guided" spreads the valid disparities along the left images `guide` (contiguous CUDA uint8 [B,ori_h,ori_w,3],
+    required for it and rejected otherwise), stopping at colour edges (oracle/lr_guided.py, GUIDED_LAMBDA and
+    GUIDED_SIGMA), with the background value where no valid pixel reaches; valid stays the check's mask, False on every
+    filled pixel."""
     fill = lr_fill(fill)
+    if (guide is not None) != (fill == "guided"):
+        raise ValueError(f"guide is required for fill=\"guided\" and only for it (fill={fill!r}, guide "
+                         f"{'given' if guide is not None else 'missing'})")
     _chk("pred", pred)
     if pred.dim() != 3 or pred.shape[0] % 2 or pred.shape[0] == 0:
         raise ValueError(f"pred must be [2B,H,W] (forward then reverse), got {tuple(pred.shape)}")
@@ -337,16 +345,27 @@ def lr_check(pred, ori_h, ori_w, tol, float_out=True, u16_out=False, valid_out=F
     if not (float_out or u16_out or valid_out):
         raise ValueError("request at least one output")
     shape, dev = (B2 // 2, int(ori_h), int(ori_w)), pred.device
+    if guide is not None and not (isinstance(guide, torch.Tensor) and guide.is_cuda and guide.dtype == torch.uint8
+                                  and guide.is_contiguous() and tuple(guide.shape) == shape + (3,) and guide.device == dev):
+        raise ValueError(f"guide must be a contiguous CUDA uint8 tensor {list(shape) + [3]} on {dev}, got "
+                         + (f"{guide.dtype} {tuple(guide.shape)} on {guide.device}" if isinstance(guide, torch.Tensor)
+                            else type(guide).__name__))
     f = torch.empty(shape, dtype=torch.float32, device=dev) if float_out or fill != "none" else None
     u = torch.empty(shape, dtype=torch.uint16, device=dev) if u16_out else None
-    v = torch.empty(shape, dtype=torch.bool, device=dev) if valid_out else None
+    v = torch.empty(shape, dtype=torch.bool, device=dev) if valid_out or fill == "guided" else None
+    args = (B2 // 2, H, W, int(ori_h), int(ori_w), float(tol))
+    outs = tuple(t.data_ptr() if t is not None else None for t in (f, u, v))
     if fill == "none":
-        _call("decnet_lr_check", pred, pred.data_ptr(), B2 // 2, H, W, int(ori_h), int(ori_w), float(tol),
-              *(t.data_ptr() if t is not None else None for t in (f, u, v)))
+        _call("decnet_lr_check", pred, pred.data_ptr(), *args, *outs)
     else:                                                                  # the float rows are the fill's scratch too
         flags = torch.empty(shape[:2], dtype=torch.uint8, device=dev)
-        _call("decnet_lr_check_fill", pred, pred.data_ptr(), B2 // 2, H, W, int(ori_h), int(ori_w), float(tol),
-              *(t.data_ptr() if t is not None else None for t in (f, u, v)), flags.data_ptr())
+        if fill == "background":
+            _call("decnet_lr_check_fill", pred, pred.data_ptr(), *args, *outs, flags.data_ptr())
+        else:
+            scratch = torch.empty(int(_lib.lib().decnet_lr_guided_fill_scratch_floats(*shape)), dtype=torch.float32,
+                                  device=dev)
+            _call("decnet_lr_check_guided_fill", pred, pred.data_ptr(), guide.data_ptr(), *args, GUIDED_LAMBDA,
+                  GUIDED_SIGMA, *outs, flags.data_ptr(), scratch.data_ptr())
     return tuple(t for t, want in ((f, float_out), (u, u16_out), (v, valid_out)) if want)
 
 

@@ -6,6 +6,7 @@
     for out in m.stream(pairs, output="u16"): ...
     disp, valid = StereoMatcher(lr_check=1.0)(left, right, return_valid=True)   # left-right check: 0 where it fails
     dense = StereoMatcher(lr_check=1.0, fill="background")(left, right)         # ... and its holes filled
+    dense = StereoMatcher(lr_check=1.0, fill="guided")(left, right)             # ... filled along the left image
 
 Every call of one shape (B, h, w, max_disp) replays one CUDA graph of the whole step: uint8 -> pad / normalise ->
 feature extractor (both views, the right one on a forked stream) -> [image-space detail masks] -> decomposed matching.
@@ -22,7 +23,12 @@ the right view and writes 0 (KITTI's "no value") elsewhere: occluded pixels and 
 fill="background" fills those pixels instead, in the same pass over the predictions (oracle/lr_fill.py): each takes the
 smaller disparity of its nearest valid neighbours in the row, because an occluded pixel belongs to the surface behind; a row
 without a valid pixel takes the rows above and below.  The mask `valid` stays the check's, so filled pixels are still told
-apart from measured ones.  The fill is also outside the graph: changing it never re-captures either.
+apart from measured ones.  fill="guided" spreads the valid disparities along the left image instead, stopping at its
+colour edges (oracle/lr_guided.py: the fast global smoother's row and column solves as normalised interpolation), so the
+filled strips follow object outlines rather than one value per row; a pixel that no valid disparity reaches keeps its
+background value.  It reads the uploaded left images st.l, on the main stream before the set's `computed` event, so the
+next upload into that set cannot overwrite them first.  The fill is also outside the graph: changing it never re-captures
+either.
 
 The capture and the double-buffered loop of `stream()` restate bench.py's `capture` / `pipelined_e2e` on purpose:
 bench.py is the fixed measuring stick of the project and does not import the package's public API.
@@ -137,8 +143,9 @@ class StereoMatcher:
     precision     "fp32" (3xTF32 convs) or "tf32"
     max_graphs    shapes whose graphs are kept (least recently used evicted first)
     lr_check      None (off) or the left-right check's tolerance in pixels (a finite number >= 0); a call may override it
-    fill          "none" (failing pixels are 0) or "background" (failing pixels filled from their valid neighbours; needs
-                  a left-right check); a call may override it
+    fill          "none" (failing pixels are 0), "background" (failing pixels filled from their valid neighbours in the
+                  row) or "guided" (filled along the left image, stopping at its edges); a fill needs a left-right check;
+                  a call may override it
     """
 
     def __init__(self, state_dict=None, max_disp=192, masks="learned", thold=0.9, detail_thold=0.3, skip_stage_id=4,
@@ -262,7 +269,7 @@ class StereoMatcher:
         left-right check (tol) the checked disparity, holes filled by `fill`, or (disparity, valid) when return_valid."""
         if st.lr:
             out = ops.lr_check(st.pred, h, w, tol, float_out=output == "float", u16_out=output == "u16", valid_out=return_valid,
-                               fill=fill)
+                               fill=fill, guide=st.l if fill == "guided" else None)
             return out if return_valid else out[0]
         if output == "u16":
             return ops.disp_to_u16(st.pred, h, w)
@@ -287,8 +294,8 @@ class StereoMatcher:
         """Disparity of one pair ([h,w,3]), a batch ([B,h,w,3]) or lists of single pairs (any sizes; one batch per
         distinct size, results in input order).  output "float" (pixels) or "u16" (x256, demo.py:191-197); the result
         has the kind of the input (numpy, CPU tensor or CUDA tensor).  lr_check (None: the matcher's) is the left-right
-        check's tolerance in pixels; pixels that fail it are 0, or filled from their neighbours with fill="background"
-        (None: the matcher's fill).  return_valid: each result is (disparity, bool valid), valid False on filled pixels."""
+        check's tolerance in pixels; pixels that fail it are 0, or filled from their neighbours with fill="background" or
+        along the left image with fill="guided" (None: the matcher's fill).  return_valid: each result is (disparity, bool valid), valid False on filled pixels."""
         if output not in OUTPUTS:
             raise ValueError(f"output must be one of {OUTPUTS}, got {output!r}")
         D = self._max_disp(max_disp)

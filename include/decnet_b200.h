@@ -437,13 +437,29 @@ int decnet_epe_3px(const float *pred, const float *gt, float max_disp, double *s
  *     nearest rows above and below that have one.  An image without a valid pixel stays 0.  out_f32 and row_flags
  *     [B,ori_h] are required (the column phase reads the float rows; row_flags = the row has a valid pixel); out_u16 =
  *     decnet_disp_to_u16's value of the float output; out_valid is the check's mask, 0 on every filled pixel.  No limit on
- *     ori_w beyond the check's. */
+ *     ori_w beyond the check's.
+ *   decnet_lr_check_guided_fill: decnet_lr_check_fill, then edge-aware filling guided by the left images guide (uint8 RGB
+ *     [B,ori_h,ori_w,3]; oracle/lr_guided.py is the spec), in fp32 with every operation rounded separately.  Edge weights
+ *     w(k) = (float)exp(-k / sigma_color) in double, k = sum_c |guide_c(p) - guide_c(q)| of neighbours p, q.  Three
+ *     iterations t = 1..3 with lam_t = (float)(lambda * 1.5 * 4^(3-t) / 63) (double) each solve every row, then every
+ *     column: (I + L) x = f on a line of n pixels, a_i = lam_t * w(k_i) between pixels i and i+1 (a_-1 = a_(n-1) = 0), by
+ *     b_i = (1 + a_(i-1)) + a_i, m_i = b_i - a_(i-1) g_(i-1), r_i = 1 / m_i, g_i = a_i r_i, y_i = (f_i + a_(i-1) y_(i-1)) r_i,
+ *     x_(n-1) = y_(n-1), x_i = y_i + g_i x_(i+1), for num (starting as valid ? dl : 0) and den (valid ? 1 : 0).  Then an
+ *     invalid pixel whose den >= 2^-126 takes num / den; every other pixel keeps its decnet_lr_check_fill value (an image
+ *     without a valid pixel stays 0).  lambda must be finite and >= 0 (0: the background fill), sigma_color finite and
+ *     > 0.  guide, out_f32, out_valid, row_flags [B,ori_h] and scratch (decnet_lr_guided_fill_scratch_floats floats) are
+ *     required; out_u16 = decnet_disp_to_u16's value of the float output; out_valid is the check's mask.  No limit on ori_h
+ *     or ori_w beyond the check's. */
 int decnet_mirror_swap_u8(const unsigned char *left, const unsigned char *right, unsigned char *out_left,
                           unsigned char *out_right, int B, int h, int w, void *stream);
 int decnet_lr_check(const float *pred, int B, int H, int W, int ori_h, int ori_w, float tol, float *out_f32,
                     unsigned short *out_u16, unsigned char *out_valid, void *stream);
 int decnet_lr_check_fill(const float *pred, int B, int H, int W, int ori_h, int ori_w, float tol, float *out_f32,
                          unsigned short *out_u16, unsigned char *out_valid, unsigned char *row_flags, void *stream);
+long long decnet_lr_guided_fill_scratch_floats(int B, int ori_h, int ori_w);
+int decnet_lr_check_guided_fill(const float *pred, const unsigned char *guide, int B, int H, int W, int ori_h, int ori_w,
+                                float tol, double lambda, double sigma_color, float *out_f32, unsigned short *out_u16,
+                                unsigned char *out_valid, unsigned char *row_flags, float *scratch, void *stream);
 
 /* SoftAttention conv input cat(left_fea, dense, sparse, left_mask, -var) -> [B,C+4,H,W]
  * (modules/SparseDenseNetRefinementMask.py:197).  C = 0 (left_fea may be NULL) packs only the four

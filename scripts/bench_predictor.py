@@ -23,6 +23,13 @@
                      same process beside an lr_check leg of the same shape; bytes: 8 read per pixel, written the float rows
                      (always: the column phase reads them), the requested uint16 / valid outputs and one flag per row
   sceneflow_stream_lr_fill  sceneflow_stream with the check and fill="background", runs alternating with the plain and _lr ones
+  lr_guided_*        the check with guided hole filling (decnet_lr_check_guided_fill: the two kernels of lr_fill, then the
+                     weight table, the prep pass, three iterations of guided_rows_kernel + guided_cols_kernel and the compose
+                     pass) at B = 8 and B = 1 SceneFlow pairs and one Middlebury pair, uint16 output, alternating with
+                     decnet_lr_check_fill on the same buffers; the line solves are chains of dependent steps, so the time is
+                     reported as is, not as a share of the HBM bound
+  sceneflow_stream_lr_guided  sceneflow_stream with the check and fill="guided", runs alternating with the _lr and _lr_fill ones
+  *_single_lr        also hold an lr_guided leg: the single-pair call with fill="guided", alternating with the other two
 
     python scripts/bench_predictor.py --out DIR
 """
@@ -102,7 +109,7 @@ def latency_pair(torch, m, left, right, calls, warmup):
     """latency() of the plain call and of the call with the left-right check, alternating call by call."""
     from decnet_b200.predictor import cache_key
     h, w = left.shape[:2]
-    legs = {"plain": {}, "lr": {"lr_check": LR_TOL}}
+    legs = {"plain": {}, "lr": {"lr_check": LR_TOL}, "lr_guided": {"lr_check": LR_TOL, "fill": "guided"}}
     for kw in legs.values():
         for _ in range(warmup):
             m(left, right, output="u16", **kw)
@@ -112,7 +119,7 @@ def latency_pair(torch, m, left, right, calls, warmup):
             t0 = time.perf_counter()
             m(left, right, output="u16", **kw)
             ts[k].append((time.perf_counter() - t0) * 1e3)
-    sets = {k: m._graphs[cache_key(1, h, w, m.max_disp, m.masks, m.precision, k == "lr")][0] for k in legs}
+    sets = {k: m._graphs[cache_key(1, h, w, m.max_disp, m.masks, m.precision, k != "plain")][0] for k in legs}
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     n = max(10, calls // 8)
     dev_ms = {k: [] for k in legs}
@@ -127,18 +134,21 @@ def latency_pair(torch, m, left, right, calls, warmup):
             dev_ms[k].append(e0.elapsed_time(e1) / n)
     out = {}
     for k, st in sets.items():
-        tol = legs[k].get("lr_check")
+        tol, fill = legs[k].get("lr_check"), legs[k].get("fill", "none")
         down = []
         for _ in range(20):
             torch.cuda.synchronize()
             t0 = time.perf_counter()
-            m._result(st, h, w, "u16", tol).cpu().numpy()
+            m._result(st, h, w, "u16", tol, False, fill).cpu().numpy()
             down.append((time.perf_counter() - t0) * 1e3)
         out[k] = {"calls": calls, "warmup": warmup, "p50_ms": pct(ts[k], 0.5), "p90_ms": pct(ts[k], 0.9), "min_ms": min(ts[k]),
                   "replay_device_ms": min(dev_ms[k]), "replay_device_ms_runs": dev_ms[k],
                   "readback_host_ms": pct(down, 0.5),
-                  "what_readback": ("lr_check (u16) + D2H" if tol is not None else "disp_to_u16 + D2H") + ", synchronised"}
-    out["lr"]["lr_check"] = LR_TOL
+                  "what_readback": (f"lr_check (u16, fill={fill}) + D2H" if tol is not None else "disp_to_u16 + D2H")
+                                   + ", synchronised"}
+    out["lr"]["lr_check"] = out["lr_guided"]["lr_check"] = LR_TOL
+    out["lr_guided"]["fill"] = "guided"
+    out["lr_guided_over_lr"] = {"p50": out["lr_guided"]["p50_ms"] / out["lr"]["p50_ms"]}
     out["lr_over_plain"] = {"p50": out["lr"]["p50_ms"] / out["plain"]["p50_ms"],
                             "replay_device": out["lr"]["replay_device_ms"] / out["plain"]["replay_device_ms"]}
     return out
@@ -202,6 +212,7 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("bench_predictor.py needs a CUDA device")
     from decnet_b200 import StereoMatcher, ops
+    from decnet_b200._lib import lib
     dev = torch.device("cuda", 0)
     res = {"gpu": gpu_info(torch)}
     res["bench_py"] = run_bench_py()
@@ -233,6 +244,8 @@ def main():
         pass
     for _ in m.stream([pair] * 4, output="u16", lr_check=LR_TOL, fill="background"):
         pass
+    for _ in m.stream([pair] * 4, output="u16", lr_check=LR_TOL, fill="guided"):
+        pass
     n = args.stream_steps
 
     def run(**kw):
@@ -241,11 +254,12 @@ def main():
         for _ in m.stream([pair] * n, output="u16", **kw):
             pass
         return time.perf_counter() - t0
-    els = {"plain": [], "lr": [], "lr_fill": []}
+    els = {"plain": [], "lr": [], "lr_fill": [], "lr_guided": []}
     for _ in range(2):                                                   # alternating plain, LR and LR + fill runs
         els["plain"].append(run())
         els["lr"].append(run(lr_check=LR_TOL))
         els["lr_fill"].append(run(lr_check=LR_TOL, fill="background"))
+        els["lr_guided"].append(run(lr_check=LR_TOL, fill="guided"))
     el = min(els["plain"])
     rate = B * n / el
     rate_lr = B * n / min(els["lr"])
@@ -268,6 +282,13 @@ def main():
                                        "what": "as sceneflow_stream_lr with fill=\"background\" (lr_check_fill_rows_kernel + "
                                                "lr_fill_empty_rows_kernel instead of lr_check_kernel); runs alternate with the "
                                                "plain and _lr ones"}
+    rate_guided = B * n / min(els["lr_guided"])
+    res["sceneflow_stream_lr_guided"] = {"batch": B, "steps": n, "lr_check": LR_TOL, "fill": "guided",
+                                         "pairs_per_s": rate_guided, "ms_per_step": min(els["lr_guided"]) / n * 1e3,
+                                         "lr_guided_over_lr_fill_step_time": rate_fill / rate_guided,
+                                         "what": "as sceneflow_stream_lr_fill with fill=\"guided\" "
+                                                 "(decnet_lr_check_guided_fill); runs alternate with the plain, _lr and "
+                                                 "_lr_fill ones"}
     del m
     torch.cuda.empty_cache()
 
@@ -358,6 +379,32 @@ def main():
                                                valid_fraction=float(valid.float().mean()),
                                                what="decnet_lr_check_fill (both kernels) vs decnet_lr_check, alternating")
         del preds
+        torch.cuda.empty_cache()
+
+    # 7. guided hole filling beside background hole filling, uint16 output
+    for tag, (B, h, w, H, W, nsets) in (("", (8, 540, 960, 540, 972, 4)), ("_b1", (1, 540, 960, 540, 972, 8)),
+                                        ("_middlebury", (1, 2000, 2900, 2025, 2916, 4))):
+        preds = [torch.randn(2 * B, H, W, device=dev) * 20 + 40 for _ in range(nsets)]
+        guides = [torch.randint(0, 256, (B, h, w, 3), device=dev, dtype=torch.uint8) for _ in range(nsets)]
+        nscratch = int(lib().decnet_lr_guided_fill_scratch_floats(B, h, w))
+        outs = [(torch.empty(B, h, w, device=dev), torch.empty(B, h, w, dtype=torch.uint16, device=dev),
+                 torch.empty(B, h, w, dtype=torch.bool, device=dev), torch.empty(B, h, dtype=torch.uint8, device=dev),
+                 torch.empty(nscratch, device=dev)) for _ in range(nsets)]
+        bg = lambda i: ops._call("decnet_lr_check_fill", preds[i], preds[i].data_ptr(), B, H, W, h, w, LR_TOL,
+                                 *(o.data_ptr() for o in outs[i][:4]))
+        gf = lambda i: ops._call("decnet_lr_check_guided_fill", preds[i], preds[i].data_ptr(), guides[i].data_ptr(), B, H, W,
+                                 h, w, LR_TOL, ops.GUIDED_LAMBDA, ops.GUIDED_SIGMA, *(o.data_ptr() for o in outs[i]))
+        runs = {"background": [], "guided": []}
+        for _ in range(2):                                               # alternating, best of each
+            runs["background"].append(kernel_us(torch, bg, nsets, n=32))
+            runs["guided"].append(kernel_us(torch, gf, nsets, n=32))
+        t_bg, t_g = min(runs["background"]), min(runs["guided"])
+        res[f"lr_guided_u16{tag}"] = {"us": t_g, "background_us": t_bg, "guided_over_background": t_g / t_bg,
+                                      "us_runs": runs, "shape": f"pred {2 * B}x{H}x{W} -> {B}x{h}x{w}", "buffer_sets": nsets,
+                                      "scratch_mb_per_set": nscratch * 4 / 1e6, "guide": "uniform random uint8",
+                                      "what": "decnet_lr_check_guided_fill (check, background fill, 3 x rows + columns, "
+                                              "compose) vs decnet_lr_check_fill, alternating; 32 launches per graph"}
+        del preds, guides, outs
         torch.cuda.empty_cache()
     (out / "bench_predictor.json").write_text(json.dumps(res, indent=1))
     print(json.dumps(res))

@@ -82,6 +82,9 @@ SIGNATURES = {
     "decnet_lr_check_fill": (_i, [_ptr] + [_i] * 5 + [C.c_float] + [_ptr] * 4 + [C.c_void_p]),
     "decnet_lr_guided_fill_scratch_floats": (C.c_longlong, [_i] * 3),
     "decnet_lr_check_guided_fill": (_i, [_ptr] * 2 + [_i] * 5 + [C.c_float] + [C.c_double] * 2 + [_ptr] * 5 + [C.c_void_p]),
+    "decnet_lr_speckle_scratch_bytes": (C.c_longlong, [_i] * 4),
+    "decnet_lr_check_speckle": (_i, [_ptr] * 2 + [_i] * 5 + [C.c_float, _i, C.c_float, _i] + [C.c_double] * 2 + [_ptr] * 5
+                                + [C.c_void_p]),
     "decnet_attn_pack": (_i, [_ptr] * 6 + [_i] * 4 + [C.c_void_p]),
     "decnet_blend": (_i, [_ptr] * 5 + [_i] * 3 + [C.c_void_p]),
     "decnet_warp_bilinear": (_i, [_ptr] * 3 + [_i] * 4 + [C.c_void_p]),

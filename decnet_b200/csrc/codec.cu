@@ -11,7 +11,9 @@
 //                      pass (check + nearest valid neighbours in the row) and a pass over the rows without a valid pixel.
 //   lr_check_guided_fill : lr_check_fill, then edge-aware filling guided by the left image (oracle/lr_guided.py): three
 //                      iterations of tridiagonal solves along every row and every column, and a compose pass.
-//                      None of the last four has a counterpart in the reference.
+//   lr_check_speckle : the check, then a speckle filter (oracle/lr_speckle.py: small connected regions invalidated) by a
+//                      block-based union-find labeller, then either fill or none.
+//                      None of the last five has a counterpart in the reference.
 #include "common.cuh"
 #include <algorithm>
 #include <cstdint>
@@ -152,14 +154,24 @@ lr_check_kernel(const float *__restrict__ pred, int B, int H, int W, int oh, int
 // its value is its forward prediction, read back from pred.
 // out_f32 always receives the row-phase values (0 on a row without a valid pixel: lr_fill_empty_rows_kernel reads them),
 // out_u16 / out_valid when requested, row_flags[b*oh + y] whether the row has a valid pixel.
+// valid_of(d, rev, W, ow, x, tol, o) says whether crop column x of the row (value d, row offset o = row * ow) is valid:
+// CheckValid runs the check, SpeckleValid (below) reads the speckle filter's planes.
 constexpr int kFillItems = 16;                                             // columns per thread per chunk
 constexpr int kFillChunk = kBlock * kFillItems;                            // 4096 columns, 16 KB of staged values
 constexpr int kFillWarps = kBlock / 32;
 
+struct CheckValid {
+    __device__ bool operator()(float d, const float *rev, int W, int ow, int x, float tol, long long) const
+    {
+        return lr_valid(d, rev, W, ow, x, tol);
+    }
+};
+
+template <class Valid>
 __global__ void __launch_bounds__(kBlock)
 lr_check_fill_rows_kernel(const float *__restrict__ pred, int B, int H, int W, int oh, int ow, float tol,
                           float *__restrict__ out_f32, unsigned short *__restrict__ out_u16,
-                          unsigned char *__restrict__ out_valid, unsigned char *__restrict__ row_flags)
+                          unsigned char *__restrict__ out_valid, unsigned char *__restrict__ row_flags, const Valid valid_of)
 {
     __shared__ float sv[kFillChunk];                                       // checked values of the chunk (dl where valid)
     __shared__ unsigned sbits[kFillItems * kFillWarps];                    // validity: ballot of entry e = i*kFillWarps + warp
@@ -189,7 +201,7 @@ lr_check_fill_rows_kernel(const float *__restrict__ pred, int B, int H, int W, i
 #pragma unroll 1
                 for (int i = 0; i < kFillItems; ++i) {                     // a thread's columns ascend: its first hit is its min
                     const int x = a + i * kBlock + t;
-                    if (x < ow && lr_valid(fwd_crop[x], rev, W, ow, x, tol)) { m = x; break; }
+                    if (x < ow && valid_of(fwd_crop[x], rev, W, ow, x, tol, o)) { m = x; break; }
                 }
                 m = __reduce_min_sync(0xffffffffu, m);
                 if (lane == 0) atomicMin(&snext, m);
@@ -208,7 +220,7 @@ lr_check_fill_rows_kernel(const float *__restrict__ pred, int B, int H, int W, i
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
                 const int x = c0 + (i0 + k) * kBlock + t, xc = min(x, ow - 1);
-                const bool v = (x < ow) & lr_valid(d[k], rev, W, ow, xc, tol);
+                const bool v = (x < ow) & valid_of(d[k], rev, W, ow, xc, tol, o);
                 vmask |= (unsigned)v << (i0 + k);
                 sv[(i0 + k) * kBlock + t] = v ? d[k] : 0.f;
             }
@@ -321,6 +333,200 @@ lr_fill_empty_rows_kernel(int oh, int ow, float *__restrict__ out_f32, unsigned 
         out_f32[o + x] = d;
         if (out_u16) out_u16[o + x] = disp_u16(d);
     }
+}
+
+// Speckle filter (oracle/lr_speckle.py) between the check and the fill: valid 4-neighbours whose values differ by at most
+// max_diff (|a - b| in fp32) are joined, and every region of at most max_size pixels is invalidated.  A block-based
+// union-find labeller over the cropped pixels, with int32 labels (a pixel index, -1 on an invalid pixel) in three passes:
+//   speckle_tile_kernel   one CTA per kTile x kTile tile: the check, then the tile's unions in shared memory; writes the
+//                         checked values val (dl where valid, else 0), each pixel's tile-local root as a global index, and
+//                         zeroes the region sizes
+//   speckle_merge_kernel  one thread per pair of 4-neighbours across a tile border: unions of the global trees
+//   speckle_count_kernel  one CTA per tile: each pixel's label becomes its root, and the region sizes are counted, per CTA
+//                         into one shared counter for the root most of the tile shares, so a region covering the image
+//                         costs about one global atomic per tile rather than one per pixel
+// Both unions are the lock-free atomic-min union of Playne & Hawick (IEEE TPDS 2018): a root is linked under the smaller
+// one with atomicMin, and a link that lost a race is retried from the value it found.  Labels only ever point to smaller
+// indices, so every chain ends.  Which pixel is a region's root depends on the race, the regions and sizes do not.
+// Then valid' = valid && size[root] > max_size, applied by speckle_apply_kernel (no fill) or by
+// lr_check_fill_rows_kernel<SpeckleValid> (the fills).
+constexpr int kTile = 32;
+constexpr int kTileRows = 8;                                               // a CTA is kTile x kTileRows threads, 4 rows each
+
+__device__ __forceinline__ bool speckle_joined(float a, float b, float max_diff)
+{
+    return fabsf(__fsub_rn(a, b)) <= max_diff;                             // an overflow to inf does not join
+}
+
+template <class P>
+__device__ __forceinline__ int uf_find(P lab, int x)
+{
+    for (int p = lab[x]; p != x; p = lab[x]) x = p;
+    return x;
+}
+
+// Join the trees of a and b in lab (shared or global), concurrently with other threads' unions.
+__device__ __forceinline__ void uf_union(int *lab, int a, int b)
+{
+    volatile int *v = lab;
+    for (;;) {
+        a = uf_find(v, a);
+        b = uf_find(v, b);
+        if (a == b) return;
+        if (a > b) { const int t = a; a = b; b = t; }
+        const int old = atomicMin(lab + b, a);                             // link the larger root under the smaller
+        if (old == b) return;
+        b = old;                                                           // b was linked meanwhile: continue from there
+    }
+}
+
+// Tile t of the [B, oh, ow] crop -> its image b and its first row y0 and column x0.
+__device__ __forceinline__ void speckle_tile(int oh, int ow, long long &b, int &y0, int &x0)
+{
+    const int tx = (ow + kTile - 1) / kTile, ty = (oh + kTile - 1) / kTile;
+    const long long t = blockIdx.x;
+    b = t / ((long long)tx * ty);
+    const int r = (int)(t - b * tx * ty);
+    y0 = r / tx * kTile;
+    x0 = (r - r / tx * tx) * kTile;
+}
+
+__global__ void __launch_bounds__(kTile * kTileRows)
+speckle_tile_kernel(const float *__restrict__ pred, int B, int H, int W, int oh, int ow, float tol, float max_diff,
+                    float *__restrict__ val, int *__restrict__ label, int *__restrict__ size)
+{
+    __shared__ float sv[kTile * kTile];
+    __shared__ int sl[kTile * kTile];                                      // tile-local parent, -1: invalid
+    long long b;
+    int y0, x0;
+    speckle_tile(oh, ow, b, y0, x0);
+    const int lx = threadIdx.x, x = x0 + lx;
+#pragma unroll
+    for (int k = 0; k < kTile / kTileRows; ++k) {
+        const int ly = threadIdx.y + k * kTileRows, y = y0 + ly, i = ly * kTile + lx;
+        bool v = false;
+        float d = 0.f;
+        if (x < ow && y < oh) {
+            const float *fwd = pred + (b * H + (H - oh + y)) * (long long)W;
+            const float *rev = pred + ((b + B) * H + (H - oh + y)) * (long long)W;
+            const float dl = fwd[W - ow + x];
+            v = lr_valid(dl, rev, W, ow, x, tol);
+            d = v ? dl : 0.f;
+        }
+        sv[i] = d;
+        sl[i] = v ? i : -1;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int k = 0; k < kTile / kTileRows; ++k) {                          // join each pixel to its left and upper neighbours
+        const int ly = threadIdx.y + k * kTileRows, i = ly * kTile + lx;
+        if (sl[i] < 0) continue;                                           // a valid pixel's parent stays >= 0
+        if (lx > 0 && sl[i - 1] >= 0 && speckle_joined(sv[i], sv[i - 1], max_diff)) uf_union(sl, i - 1, i);
+        if (ly > 0 && sl[i - kTile] >= 0 && speckle_joined(sv[i], sv[i - kTile], max_diff)) uf_union(sl, i - kTile, i);
+    }
+    __syncthreads();
+#pragma unroll
+    for (int k = 0; k < kTile / kTileRows; ++k) {
+        const int ly = threadIdx.y + k * kTileRows, y = y0 + ly, i = ly * kTile + lx;
+        if (x >= ow || y >= oh) continue;
+        const long long g = (b * oh + y) * ow + x;
+        int root = -1;
+        if (sl[i] >= 0) {
+            const int r = uf_find(sl, i);
+            root = (int)((b * oh + y0 + r / kTile) * ow + x0 + r % kTile);
+        }
+        val[g] = sv[i];
+        label[g] = root;
+        size[g] = 0;
+    }
+}
+
+// Pair e of 4-neighbours across a tile border: the first nv pairs straddle the vertical borders (row, kTile*k - 1 | kTile*k),
+// the rest the horizontal ones (kTile*k - 1 | kTile*k, x).
+__global__ void __launch_bounds__(kBlock)
+speckle_merge_kernel(const float *__restrict__ val, int *label, int oh, int ow, float max_diff, long long nv, long long n)
+{
+    const long long e = (long long)blockIdx.x * kBlock + threadIdx.x;
+    if (e >= n) return;
+    const int tx = (ow + kTile - 1) / kTile, ty = (oh + kTile - 1) / kTile;
+    long long c, a;
+    if (e < nv) {
+        const long long row = e / (tx - 1);
+        c = row * ow + (long long)(e - row * (tx - 1) + 1) * kTile;
+        a = c - 1;
+    } else {
+        const long long j = e - nv, q = j / ow, b = q / (ty - 1);
+        c = (b * oh + (q - b * (ty - 1) + 1) * kTile) * ow + (j - q * ow);
+        a = c - ow;
+    }
+    if (label[a] < 0 || label[c] < 0 || !speckle_joined(val[a], val[c], max_diff)) return;
+    uf_union(label, (int)a, (int)c);
+}
+
+__global__ void __launch_bounds__(kTile * kTileRows)
+speckle_count_kernel(int *label, int *__restrict__ size, int oh, int ow)
+{
+    __shared__ int sdom, scount;                                           // a root of the tile and its pixel count
+    long long b;
+    int y0, x0;
+    speckle_tile(oh, ow, b, y0, x0);
+    const int lx = threadIdx.x, x = x0 + lx;
+    if (lx == 0 && threadIdx.y == 0) { sdom = -1; scount = 0; }
+    __syncthreads();
+    int roots[kTile / kTileRows];
+#pragma unroll
+    for (int k = 0; k < kTile / kTileRows; ++k) {
+        const int y = y0 + threadIdx.y + k * kTileRows;
+        roots[k] = -1;
+        if (x >= ow || y >= oh) continue;
+        const long long g = (b * oh + y) * ow + x;
+        const int l = label[g];
+        if (l < 0) continue;
+        const int r = uf_find(label, l);                                   // the trees no longer change: concurrent
+        if (r != l) label[g] = r;                                          // compressions only store ancestors
+        roots[k] = r;
+        if (sdom < 0) atomicCAS(&sdom, -1, r);
+    }
+    __syncthreads();
+    const int dom = sdom;
+#pragma unroll
+    for (int k = 0; k < kTile / kTileRows; ++k) {
+        const int r = roots[k];
+        const unsigned peers = __match_any_sync(0xffffffffu, r);
+        if (r < 0 || lx != __ffs(peers) - 1) continue;
+        if (r == dom) atomicAdd(&scount, __popc(peers));
+        else atomicAdd(size + r, __popc(peers));
+    }
+    __syncthreads();
+    if (lx == 0 && threadIdx.y == 0 && scount) atomicAdd(size + dom, scount);
+}
+
+// lr_check_fill_rows_kernel's validity under the speckle filter; the kernel then reads its values from the plane val, passed
+// as pred with H = oh, W = ow and no reverse half (B = 0).
+struct SpeckleValid {
+    const int *label, *size;
+    int max_size;
+    __device__ bool operator()(float, const float *, int, int, int x, float, long long o) const
+    {
+        const int r = label[o + x];
+        return r >= 0 && size[r] > max_size;
+    }
+};
+
+// The speckle filter without a fill: the requested outputs of valid' and its values.
+__global__ void __launch_bounds__(kBlock)
+speckle_apply_kernel(const float *__restrict__ val, const int *__restrict__ label, const int *__restrict__ size, int max_size,
+                     float *__restrict__ out_f32, unsigned short *__restrict__ out_u16, unsigned char *__restrict__ out_valid,
+                     long long n)
+{
+    const long long i = (long long)blockIdx.x * kBlock + threadIdx.x;
+    if (i >= n) return;
+    const int r = label[i];
+    const bool v = r >= 0 && size[r] > max_size;
+    const float d = v ? val[i] : 0.f;
+    if (out_f32) out_f32[i] = d;
+    if (out_u16) out_u16[i] = disp_u16(d);
+    if (out_valid) out_valid[i] = v ? 1 : 0;
 }
 
 // Edge-aware ("guided") hole filling (oracle/lr_guided.py): the fast global smoother's line solves over the background-
@@ -613,31 +819,18 @@ int decnet_lr_check_fill(const float *pred, int B, int H, int W, int ori_h, int 
     DECNET_REQUIRE(rows <= 0x7fffffffLL, "%lld rows exceed the grid", rows);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     lr_check_fill_rows_kernel<<<(unsigned)rows, kBlock, 0, st>>>(pred, B, H, W, ori_h, ori_w, tol, out_f32, out_u16, out_valid,
-                                                                 row_flags);
+                                                                 row_flags, CheckValid{});
     if (int s = after_launch("lr_check_fill_rows_kernel")) return s;
     lr_fill_empty_rows_kernel<<<(unsigned)rows, kBlock, 0, st>>>(ori_h, ori_w, out_f32, out_u16, row_flags);
     return after_launch("lr_fill_empty_rows_kernel");
 }
 
-long long decnet_lr_guided_fill_scratch_floats(int B, int ori_h, int ori_w)
+// The guided fill's stages after the background fill of out_f32 (valid: out_valid), for decnet_lr_check_guided_fill and
+// decnet_lr_check_speckle; the callers validate the arguments.
+static int guided_stages(const unsigned char *guide, int B, int ori_h, int ori_w, double lambda, double sigma_color,
+                         float *out_f32, unsigned short *out_u16, const unsigned char *out_valid, float *scratch, cudaStream_t st)
 {
-    return kGuideTableFloats + 5 * (long long)B * ori_h * ori_w;           // table, wh, wv, num, den, g
-}
-
-int decnet_lr_check_guided_fill(const float *pred, const unsigned char *guide, int B, int H, int W, int ori_h, int ori_w,
-                                float tol, double lambda, double sigma_color, float *out_f32, unsigned short *out_u16,
-                                unsigned char *out_valid, unsigned char *row_flags, float *scratch, void *stream)
-{
-    DECNET_REQUIRE(pred && guide && out_f32 && out_valid && row_flags && scratch,
-                   "null prediction, guide, float rows, mask, row flags or scratch");
-    DECNET_REQUIRE(B > 0 && ori_h > 0 && ori_w > 0 && ori_h <= H && ori_w <= W, "crop %dx%d outside the %dx%d map", ori_h, ori_w, H, W);
-    DECNET_REQUIRE(tol >= 0.f && tol <= 3.402823466e38f, "tolerance must be finite and >= 0");
-    DECNET_REQUIRE(lambda >= 0.0 && lambda <= 1.7976931348623157e308, "lambda must be finite and >= 0");
-    DECNET_REQUIRE(sigma_color > 0.0 && sigma_color <= 1.7976931348623157e308, "sigma_color must be finite and > 0");
     const long long rows = (long long)B * ori_h, n = rows * ori_w;
-    DECNET_REQUIRE(rows <= 0x7fffffffLL, "%lld rows exceed the grid", rows);
-    if (int s = decnet_lr_check_fill(pred, B, H, W, ori_h, ori_w, tol, out_f32, nullptr, out_valid, row_flags, stream)) return s;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
     float *table = scratch, *wh = table + kGuideTableFloats, *wv = wh + n, *num = wv + n, *den = num + n, *g = den + n;
     guided_table_kernel<<<(kGuideTable + kBlock - 1) / kBlock, kBlock, 0, st>>>(sigma_color, table);
     if (int s = after_launch("guided_table_kernel")) return s;
@@ -656,6 +849,96 @@ int decnet_lr_check_guided_fill(const float *pred, const unsigned char *guide, i
     }
     guided_compose_kernel<<<pix_grid, kBlock, 0, st>>>(num, den, out_valid, out_f32, out_u16, n);
     return after_launch("guided_compose_kernel");
+}
+
+long long decnet_lr_guided_fill_scratch_floats(int B, int ori_h, int ori_w)
+{
+    return kGuideTableFloats + 5 * (long long)B * ori_h * ori_w;           // table, wh, wv, num, den, g
+}
+
+int decnet_lr_check_guided_fill(const float *pred, const unsigned char *guide, int B, int H, int W, int ori_h, int ori_w,
+                                float tol, double lambda, double sigma_color, float *out_f32, unsigned short *out_u16,
+                                unsigned char *out_valid, unsigned char *row_flags, float *scratch, void *stream)
+{
+    DECNET_REQUIRE(pred && guide && out_f32 && out_valid && row_flags && scratch,
+                   "null prediction, guide, float rows, mask, row flags or scratch");
+    DECNET_REQUIRE(B > 0 && ori_h > 0 && ori_w > 0 && ori_h <= H && ori_w <= W, "crop %dx%d outside the %dx%d map", ori_h, ori_w, H, W);
+    DECNET_REQUIRE(tol >= 0.f && tol <= 3.402823466e38f, "tolerance must be finite and >= 0");
+    DECNET_REQUIRE(lambda >= 0.0 && lambda <= 1.7976931348623157e308, "lambda must be finite and >= 0");
+    DECNET_REQUIRE(sigma_color > 0.0 && sigma_color <= 1.7976931348623157e308, "sigma_color must be finite and > 0");
+    const long long rows = (long long)B * ori_h;
+    DECNET_REQUIRE(rows <= 0x7fffffffLL, "%lld rows exceed the grid", rows);
+    if (int s = decnet_lr_check_fill(pred, B, H, W, ori_h, ori_w, tol, out_f32, nullptr, out_valid, row_flags, stream)) return s;
+    return guided_stages(guide, B, ori_h, ori_w, lambda, sigma_color, out_f32, out_u16, out_valid, scratch,
+                         static_cast<cudaStream_t>(stream));
+}
+
+// Speckle planes: val (fp32), label and size (int32), n each, rounded up to 16 bytes; then the guided fill's scratch.
+static long long speckle_planes_bytes(long long n) { return (12 * n + 15) / 16 * 16; }
+
+long long decnet_lr_speckle_scratch_bytes(int B, int ori_h, int ori_w, int fill)
+{
+    const long long n = (long long)B * ori_h * ori_w;
+    return speckle_planes_bytes(n) + (fill == 2 ? 4 * decnet_lr_guided_fill_scratch_floats(B, ori_h, ori_w) : 0);
+}
+
+int decnet_lr_check_speckle(const float *pred, const unsigned char *guide, int B, int H, int W, int ori_h, int ori_w,
+                            float tol, int max_size, float max_diff, int fill, double lambda, double sigma_color,
+                            float *out_f32, unsigned short *out_u16, unsigned char *out_valid, unsigned char *row_flags,
+                            void *scratch, void *stream)
+{
+    DECNET_REQUIRE(fill >= 0 && fill <= 2, "fill must be 0 (none), 1 (background) or 2 (guided), got %d", fill);
+    DECNET_REQUIRE((guide != nullptr) == (fill == 2), "guide is required for fill 2 (guided) and only for it");
+    DECNET_REQUIRE(pred && (out_f32 || out_u16 || out_valid), "null prediction or no output requested");
+    DECNET_REQUIRE(fill == 0 || (out_f32 && row_flags), "a fill needs the float rows and row flags");
+    DECNET_REQUIRE(fill < 2 || out_valid, "the guided fill needs the mask");
+    DECNET_REQUIRE(B > 0 && ori_h > 0 && ori_w > 0 && ori_h <= H && ori_w <= W, "crop %dx%d outside the %dx%d map", ori_h, ori_w, H, W);
+    DECNET_REQUIRE(tol >= 0.f && tol <= 3.402823466e38f, "tolerance must be finite and >= 0");
+    DECNET_REQUIRE(max_size >= 0, "speckle size must be >= 0, got %d", max_size);
+    DECNET_REQUIRE(max_diff >= 0.f && max_diff <= 3.402823466e38f, "speckle range must be finite and >= 0");
+    DECNET_REQUIRE(fill < 2 || (lambda >= 0.0 && lambda <= 1.7976931348623157e308), "lambda must be finite and >= 0");
+    DECNET_REQUIRE(fill < 2 || (sigma_color > 0.0 && sigma_color <= 1.7976931348623157e308), "sigma_color must be finite and > 0");
+    const long long rows = (long long)B * ori_h, n = rows * ori_w;
+    DECNET_REQUIRE(n <= 0x7fffffffLL, "%lld pixels exceed the int32 labels", n);
+    const long long planes = speckle_planes_bytes(n);
+    if (max_size == 0) {                                                   // off: the entries without the filter, as they are
+        if (fill == 0) return decnet_lr_check(pred, B, H, W, ori_h, ori_w, tol, out_f32, out_u16, out_valid, stream);
+        if (fill == 1) return decnet_lr_check_fill(pred, B, H, W, ori_h, ori_w, tol, out_f32, out_u16, out_valid, row_flags, stream);
+        DECNET_REQUIRE(scratch, "null scratch");
+        return decnet_lr_check_guided_fill(pred, guide, B, H, W, ori_h, ori_w, tol, lambda, sigma_color, out_f32, out_u16,
+                                           out_valid, row_flags, reinterpret_cast<float *>(static_cast<char *>(scratch) + planes),
+                                           stream);
+    }
+    DECNET_REQUIRE(scratch, "null scratch");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    float *val = static_cast<float *>(scratch);
+    int *label = reinterpret_cast<int *>(val + n), *size = label + n;
+    const long long tx = (ori_w + kTile - 1) / kTile, ty = (ori_h + kTile - 1) / kTile;
+    const unsigned tiles = (unsigned)(B * tx * ty);
+    speckle_tile_kernel<<<tiles, dim3(kTile, kTileRows), 0, st>>>(pred, B, H, W, ori_h, ori_w, tol, max_diff, val, label, size);
+    if (int s = after_launch("speckle_tile_kernel")) return s;
+    const long long nv = rows * (tx - 1), edges = nv + B * (ty - 1) * ori_w;
+    if (edges > 0) {
+        speckle_merge_kernel<<<(unsigned)((edges + kBlock - 1) / kBlock), kBlock, 0, st>>>(val, label, ori_h, ori_w, max_diff, nv,
+                                                                                          edges);
+        if (int s = after_launch("speckle_merge_kernel")) return s;
+    }
+    speckle_count_kernel<<<tiles, dim3(kTile, kTileRows), 0, st>>>(label, size, ori_h, ori_w);
+    if (int s = after_launch("speckle_count_kernel")) return s;
+    if (fill == 0) {
+        speckle_apply_kernel<<<(unsigned)((n + kBlock - 1) / kBlock), kBlock, 0, st>>>(val, label, size, max_size, out_f32, out_u16,
+                                                                                      out_valid, n);
+        return after_launch("speckle_apply_kernel");
+    }
+    lr_check_fill_rows_kernel<<<(unsigned)rows, kBlock, 0, st>>>(val, 0, ori_h, ori_w, ori_h, ori_w, 0.f, out_f32,
+                                                                 fill == 2 ? nullptr : out_u16, out_valid, row_flags,
+                                                                 SpeckleValid{label, size, max_size});
+    if (int s = after_launch("lr_check_fill_rows_kernel")) return s;
+    lr_fill_empty_rows_kernel<<<(unsigned)rows, kBlock, 0, st>>>(ori_h, ori_w, out_f32, fill == 2 ? nullptr : out_u16, row_flags);
+    if (int s = after_launch("lr_fill_empty_rows_kernel")) return s;
+    if (fill == 1) return 0;
+    return guided_stages(guide, B, ori_h, ori_w, lambda, sigma_color, out_f32, out_u16, out_valid,
+                         reinterpret_cast<float *>(static_cast<char *>(scratch) + planes), st);
 }
 
 int decnet_epe_3px(const float *pred, const float *gt, float max_disp, double *sums3, long long n, void *stream)

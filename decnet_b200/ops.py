@@ -321,7 +321,19 @@ def lr_fill(fill):
     return fill
 
 
-def lr_check(pred, ori_h, ori_w, tol, float_out=True, u16_out=False, valid_out=False, fill="none", guide=None):
+def lr_speckle(size, rng):
+    """Speckle filter settings of the left-right check -> (size, range): size an int >= 0 (not a bool; 0: off), range a
+    number of disparity pixels that is finite as a float32 and >= 0 (not a bool), else ValueError."""
+    if isinstance(size, (bool, np.bool_)) or not isinstance(size, numbers.Integral) or size < 0:
+        raise ValueError(f"speckle_size must be an integer number of pixels >= 0 (0: off), got {size!r}")
+    if (isinstance(rng, (bool, np.bool_)) or not isinstance(rng, numbers.Real) or not math.isfinite(rng) or rng < 0
+            or abs(float(rng)) > float(np.finfo(np.float32).max)):
+        raise ValueError(f"speckle_range must be a finite number of disparity pixels >= 0, got {rng!r}")
+    return int(size), float(rng)
+
+
+def lr_check(pred, ori_h, ori_w, tol, float_out=True, u16_out=False, valid_out=False, fill="none", guide=None,
+             speckle_size=0, speckle_range=1.0):
     """Left-right consistency check (oracle/lr_check.py).  pred fp32 [2B,H,W]: the forward padded predictions, then
     those of the mirrored, swapped pairs.  Returns a tuple of the requested [B,ori_h,ori_w] outputs, in this order:
     float (the forward disparity where valid, else 0), uint16 (disp_to_u16's value where valid, else 0), bool valid.
@@ -330,8 +342,11 @@ def lr_check(pred, ori_h, ori_w, tol, float_out=True, u16_out=False, valid_out=F
     fill="guided" spreads the valid disparities along the left images `guide` (contiguous CUDA uint8 [B,ori_h,ori_w,3],
     required for it and rejected otherwise), stopping at colour edges (oracle/lr_guided.py, GUIDED_LAMBDA and
     GUIDED_SIGMA), with the background value where no valid pixel reaches; valid stays the check's mask, False on every
-    filled pixel."""
+    filled pixel.  speckle_size > 0 removes speckles before the fill (oracle/lr_speckle.py): valid 4-neighbours whose
+    disparities differ by at most speckle_range join a region, and every region of at most speckle_size pixels becomes
+    invalid (0, or filled); valid is then the check's mask minus the speckles.  speckle_size = 0 runs no filter."""
     fill = lr_fill(fill)
+    speckle_size, speckle_range = lr_speckle(speckle_size, speckle_range)
     if (guide is not None) != (fill == "guided"):
         raise ValueError(f"guide is required for fill=\"guided\" and only for it (fill={fill!r}, guide "
                          f"{'given' if guide is not None else 'missing'})")
@@ -355,7 +370,15 @@ def lr_check(pred, ori_h, ori_w, tol, float_out=True, u16_out=False, valid_out=F
     v = torch.empty(shape, dtype=torch.bool, device=dev) if valid_out or fill == "guided" else None
     args = (B2 // 2, H, W, int(ori_h), int(ori_w), float(tol))
     outs = tuple(t.data_ptr() if t is not None else None for t in (f, u, v))
-    if fill == "none":
+    if speckle_size:
+        kind = LR_FILLS.index(fill)
+        flags = torch.empty(shape[:2], dtype=torch.uint8, device=dev) if fill != "none" else None
+        scratch = torch.empty(int(_lib.lib().decnet_lr_speckle_scratch_bytes(*shape, kind)), dtype=torch.uint8, device=dev)
+        size = min(speckle_size, 2**31 - 1)                                # a region has fewer pixels: the same filter
+        _call("decnet_lr_check_speckle", pred, pred.data_ptr(), guide.data_ptr() if guide is not None else None, *args,
+              size, speckle_range, kind, GUIDED_LAMBDA, GUIDED_SIGMA, *outs, flags.data_ptr() if flags is not None else None,
+              scratch.data_ptr())
+    elif fill == "none":
         _call("decnet_lr_check", pred, pred.data_ptr(), *args, *outs)
     else:                                                                  # the float rows are the fill's scratch too
         flags = torch.empty(shape[:2], dtype=torch.uint8, device=dev)

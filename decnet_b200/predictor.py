@@ -7,6 +7,7 @@
     disp, valid = StereoMatcher(lr_check=1.0)(left, right, return_valid=True)   # left-right check: 0 where it fails
     dense = StereoMatcher(lr_check=1.0, fill="background")(left, right)         # ... and its holes filled
     dense = StereoMatcher(lr_check=1.0, fill="guided")(left, right)             # ... filled along the left image
+    dense = StereoMatcher(lr_check=1.0, speckle_size=100, fill="background")(left, right)   # ... speckles removed first
 
 Every call of one shape (B, h, w, max_disp) replays one CUDA graph of the whole step: uint8 -> pad / normalise ->
 feature extractor (both views, the right one on a forked stream) -> [image-space detail masks] -> decomposed matching.
@@ -29,6 +30,13 @@ filled strips follow object outlines rather than one value per row; a pixel that
 background value.  It reads the uploaded left images st.l, on the main stream before the set's `computed` event, so the
 next upload into that set cannot overwrite them first.  The fill is also outside the graph: changing it never re-captures
 either.
+
+Between the check and the fill, speckle_size > 0 removes speckles (OpenCV's speckleWindowSize / speckleRange, i.e.
+cv2.filterSpeckles; oracle/lr_speckle.py): in textureless and repetitive areas, and in occluded strips, some pixels pass
+the check by coincidence and form small islands, which either fill would spread as if they were measured.  Valid
+4-neighbours whose disparities differ by at most speckle_range join a region, and every region of at most speckle_size
+pixels becomes invalid: 0 without a fill, filled with one, False in `valid`.  It runs outside the graph with the check, so
+it never re-captures either.
 
 The capture and the double-buffered loop of `stream()` restate bench.py's `capture` / `pipelined_e2e` on purpose:
 bench.py is the fixed measuring stick of the project and does not import the package's public API.
@@ -146,10 +154,15 @@ class StereoMatcher:
     fill          "none" (failing pixels are 0), "background" (failing pixels filled from their valid neighbours in the
                   row) or "guided" (filled along the left image, stopping at its edges); a fill needs a left-right check;
                   a call may override it
+    speckle_size  0 (off) or the largest region, in pixels of the input image, that the speckle filter removes after the
+                  check and before the fill; needs a left-right check; a call may override it
+    speckle_range the largest disparity difference, in pixels, between neighbours of one region (a finite number >= 0);
+                  a call may override it
     """
 
     def __init__(self, state_dict=None, max_disp=192, masks="learned", thold=0.9, detail_thold=0.3, skip_stage_id=4,
-                 precision="fp32", device="cuda", max_graphs=4, lr_check=None, fill="none"):
+                 precision="fp32", device="cuda", max_graphs=4, lr_check=None, fill="none", speckle_size=0,
+                 speckle_range=1.0):
         if masks not in MASKS:
             raise ValueError(f"masks must be one of {MASKS}, got {masks!r}")
         if precision not in PRECISIONS:
@@ -160,6 +173,7 @@ class StereoMatcher:
             raise ValueError(f"max_graphs must be a positive integer, got {max_graphs!r}")
         self.lr_check = None if lr_check is None else ops.lr_tolerance(lr_check)
         self.fill = ops.lr_fill(fill)
+        self.speckle_size, self.speckle_range = ops.lr_speckle(speckle_size, speckle_range)
         dev = torch.device(device)
         if dev.type != "cuda":
             raise ValueError(f"device must be a CUDA device (decnet_b200 has no CPU path), got {device!r}")
@@ -264,12 +278,14 @@ class StereoMatcher:
         st.graph.replay()
 
     # ------------------------------------------------------------------------------------------------------------ calls
-    def _result(self, st, h, w, output, tol=None, return_valid=False, fill="none"):
+    def _result(self, st, h, w, output, tol=None, return_valid=False, fill="none", speckle=(0, 1.0)):
         """Fresh device tensor (never the graph's static buffer) in the requested format, on the current stream; with the
-        left-right check (tol) the checked disparity, holes filled by `fill`, or (disparity, valid) when return_valid."""
+        left-right check (tol) the checked disparity, speckles (size, range) removed, holes filled by `fill`, or
+        (disparity, valid) when return_valid."""
         if st.lr:
             out = ops.lr_check(st.pred, h, w, tol, float_out=output == "float", u16_out=output == "u16", valid_out=return_valid,
-                               fill=fill, guide=st.l if fill == "guided" else None)
+                               fill=fill, guide=st.l if fill == "guided" else None, speckle_size=speckle[0],
+                               speckle_range=speckle[1])
             return out if return_valid else out[0]
         if output == "u16":
             return ops.disp_to_u16(st.pred, h, w)
@@ -290,23 +306,36 @@ class StereoMatcher:
             raise ValueError(f"fill needs a left-right check: give lr_check to the matcher or the call (fill={fill!r})")
         return tol, fill
 
-    def __call__(self, left, right, output="float", max_disp=None, lr_check=None, return_valid=False, fill=None):
+    def _speckle(self, tol, speckle_size=None, speckle_range=None):
+        """The call's speckle filter (size, range) under the call's tolerance tol, validated before any device work."""
+        size = self.speckle_size if speckle_size is None else speckle_size
+        rng = self.speckle_range if speckle_range is None else speckle_range
+        size, rng = ops.lr_speckle(size, rng)
+        if size and tol is None:
+            raise ValueError(f"speckle_size needs a left-right check: give lr_check to the matcher or the call "
+                             f"(speckle_size={size})")
+        return size, rng
+
+    def __call__(self, left, right, output="float", max_disp=None, lr_check=None, return_valid=False, fill=None,
+                 speckle_size=None, speckle_range=None):
         """Disparity of one pair ([h,w,3]), a batch ([B,h,w,3]) or lists of single pairs (any sizes; one batch per
         distinct size, results in input order).  output "float" (pixels) or "u16" (x256, demo.py:191-197); the result
         has the kind of the input (numpy, CPU tensor or CUDA tensor).  lr_check (None: the matcher's) is the left-right
         check's tolerance in pixels; pixels that fail it are 0, or filled from their neighbours with fill="background" or
-        along the left image with fill="guided" (None: the matcher's fill).  return_valid: each result is (disparity, bool valid), valid False on filled pixels."""
+        along the left image with fill="guided" (None: the matcher's fill).  return_valid: each result is (disparity, bool valid), valid False on filled pixels.
+        speckle_size / speckle_range (None: the matcher's) remove speckles between the check and the fill."""
         if output not in OUTPUTS:
             raise ValueError(f"output must be one of {OUTPUTS}, got {output!r}")
         D = self._max_disp(max_disp)
         tol, fill = self._lr(lr_check, return_valid, fill)
+        speckle = self._speckle(tol, speckle_size, speckle_range)
         if isinstance(left, (list, tuple)):
-            return self._call_list(left, right, output, D, tol, return_valid, fill)
+            return self._call_list(left, right, output, D, tol, return_valid, fill, speckle)
         kind, batched, B, h, w = check_pair(left, right)
-        out = self._run(left, right, kind, B, h, w, output, D, tol, return_valid, fill)
+        out = self._run(left, right, kind, B, h, w, output, D, tol, return_valid, fill, speckle)
         return out if batched else _index(out, 0)
 
-    def _call_list(self, lefts, rights, output, D, tol, return_valid, fill):
+    def _call_list(self, lefts, rights, output, D, tol, return_valid, fill, speckle):
         if not isinstance(rights, (list, tuple)) or len(rights) != len(lefts):
             raise ValueError("left and right lists must have the same length")
         groups = OrderedDict()
@@ -319,7 +348,7 @@ class StereoMatcher:
         for (kind, h, w), idx in groups.items():
             stack = np.stack if kind == "numpy" else torch.stack
             out = self._run(stack([lefts[i] for i in idx]), stack([rights[i] for i in idx]), kind, len(idx), h, w, output, D,
-                            tol, return_valid, fill)
+                            tol, return_valid, fill, speckle)
             for j, i in enumerate(idx):
                 results[i] = _index(out, j)
         return results
@@ -338,32 +367,35 @@ class StereoMatcher:
         st.r.copy_(st.host_r, non_blocking=True)
 
     @torch.no_grad()
-    def _run(self, left, right, kind, B, h, w, output, D, tol=None, return_valid=False, fill="none"):
+    def _run(self, left, right, kind, B, h, w, output, D, tol=None, return_valid=False, fill="none", speckle=(0, 1.0)):
         if kind == "cuda" and left.device != self.dev:
             raise ValueError(f"inputs are on {left.device}, the matcher on {self.dev}")
         with torch.cuda.device(self.dev):
             st = self._sets(cache_key(B, h, w, D, self.masks, self.precision, tol is not None), 1)[0]
             self._upload(st, left, right, kind)
             self._replay(st, D)
-            out = self._result(st, h, w, output, tol, return_valid, fill)
+            out = self._result(st, h, w, output, tol, return_valid, fill, speckle)
             if kind == "cuda":
                 return out
             out = _map(lambda t: t.cpu(), out)                            # synchronous: the staging buffers are free again
             return _map(lambda t: t.numpy(), out) if kind == "numpy" else out
 
-    def stream(self, pairs, output="float", max_disp=None, lr_check=None, return_valid=False, fill=None):
+    def stream(self, pairs, output="float", max_disp=None, lr_check=None, return_valid=False, fill=None, speckle_size=None,
+               speckle_range=None):
         """Yield the result of each (left, right) of `pairs` in order, software-pipelined over two buffer sets per shape:
         while the graph of item i runs, the copy stream uploads item i+1 into the other set (bench.py's pipelined_e2e).
         Host results are read back through pinned memory and yielded as fresh arrays.  A change of shape drains the
-        pipeline and continues with the new shape's sets.  lr_check / return_valid / fill as for a call."""
+        pipeline and continues with the new shape's sets.  lr_check / return_valid / fill / speckle_size / speckle_range as
+        for a call."""
         if output not in OUTPUTS:
             raise ValueError(f"output must be one of {OUTPUTS}, got {output!r}")
         D = self._max_disp(max_disp)
         tol, fill = self._lr(lr_check, return_valid, fill)
-        return self._stream(pairs, output, D, tol, return_valid, fill)    # arguments checked now, not at the first item
+        speckle = self._speckle(tol, speckle_size, speckle_range)
+        return self._stream(pairs, output, D, tol, return_valid, fill, speckle)   # arguments checked now, not at the first item
 
     @torch.no_grad()
-    def _stream(self, pairs, output, D, tol, return_valid, fill):
+    def _stream(self, pairs, output, D, tol, return_valid, fill, speckle):
         with torch.cuda.device(self.dev):
             if self._copy_stream is None:
                 self._copy_stream = torch.cuda.Stream(self.dev)
@@ -399,7 +431,7 @@ class StereoMatcher:
                     st.uploaded.record(copy)
                 main.wait_event(st.uploaded)
                 self._replay(st, D)
-                res = self._result(st, h, w, output, tol, return_valid, fill)
+                res = self._result(st, h, w, output, tol, return_valid, fill, speckle)
                 if kind != "cuda":
                     res = _map(_to_pinned, res)
                 st.computed = torch.cuda.Event()

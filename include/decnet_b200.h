@@ -449,7 +449,15 @@ int decnet_epe_3px(const float *pred, const float *gt, float max_disp, double *s
  *     without a valid pixel stays 0).  lambda must be finite and >= 0 (0: the background fill), sigma_color finite and
  *     > 0.  guide, out_f32, out_valid, row_flags [B,ori_h] and scratch (decnet_lr_guided_fill_scratch_floats floats) are
  *     required; out_u16 = decnet_disp_to_u16's value of the float output; out_valid is the check's mask.  No limit on ori_h
- *     or ori_w beyond the check's. */
+ *     or ori_w beyond the check's.
+ *   decnet_lr_check_speckle: the same check, then a speckle filter (oracle/lr_speckle.py is the spec), then fill 0 (none,
+ *     as decnet_lr_check), 1 (background, as decnet_lr_check_fill) or 2 (guided, as decnet_lr_check_guided_fill with
+ *     lambda and sigma_color) on the filtered mask.  Per image, two valid 4-neighbours (never diagonal) are joined when
+ *     |dl_a - dl_b| <= max_diff in fp32; every pixel of a connected region of at most max_size pixels becomes invalid (its
+ *     value 0 before the fill).  out_valid is the filtered mask, every output a copy of a valid dl.  max_size must be
+ *     >= 0 (0: exactly the entry without the filter), max_diff finite and >= 0, B*ori_h*ori_w < 2^31 (int32 labels).
+ *     guide is required for fill 2 and only for it; the other outputs as for that fill's entry.  scratch holds
+ *     decnet_lr_speckle_scratch_bytes(B, ori_h, ori_w, fill) bytes, 16-byte aligned.  No other limit on ori_h or ori_w. */
 int decnet_mirror_swap_u8(const unsigned char *left, const unsigned char *right, unsigned char *out_left,
                           unsigned char *out_right, int B, int h, int w, void *stream);
 int decnet_lr_check(const float *pred, int B, int H, int W, int ori_h, int ori_w, float tol, float *out_f32,
@@ -460,6 +468,11 @@ long long decnet_lr_guided_fill_scratch_floats(int B, int ori_h, int ori_w);
 int decnet_lr_check_guided_fill(const float *pred, const unsigned char *guide, int B, int H, int W, int ori_h, int ori_w,
                                 float tol, double lambda, double sigma_color, float *out_f32, unsigned short *out_u16,
                                 unsigned char *out_valid, unsigned char *row_flags, float *scratch, void *stream);
+long long decnet_lr_speckle_scratch_bytes(int B, int ori_h, int ori_w, int fill);
+int decnet_lr_check_speckle(const float *pred, const unsigned char *guide, int B, int H, int W, int ori_h, int ori_w,
+                            float tol, int max_size, float max_diff, int fill, double lambda, double sigma_color,
+                            float *out_f32, unsigned short *out_u16, unsigned char *out_valid, unsigned char *row_flags,
+                            void *scratch, void *stream);
 
 /* SoftAttention conv input cat(left_fea, dense, sparse, left_mask, -var) -> [B,C+4,H,W]
  * (modules/SparseDenseNetRefinementMask.py:197).  C = 0 (left_fea may be NULL) packs only the four

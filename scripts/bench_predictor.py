@@ -30,6 +30,15 @@
                      reported as is, not as a share of the HBM bound
   sceneflow_stream_lr_guided  sceneflow_stream with the check and fill="guided", runs alternating with the _lr and _lr_fill ones
   *_single_lr        also hold an lr_guided leg: the single-pair call with fill="guided", alternating with the other two
+  lr_speckle_*       the check with the speckle filter (speckle_size 100, speckle_range 1) and background hole filling
+                     (decnet_lr_check_speckle: speckle_tile / _merge / _count_kernel, then the two kernels of lr_fill) against
+                     decnet_lr_check_fill on the same buffers, alternating, uint16 output, at B = 8 SceneFlow pairs and one
+                     Middlebury pair, on two kinds of prediction: "random" (randn * 20 + 40, about 3 % of the pixels pass the
+                     check: many one-pixel regions) and "planar" (a few planes of values in (-0.5, 0.5] against a zero
+                     reverse map with tolerance 3e38, 97 % valid: one region per image, the count's contention case);
+                     the HBM share is taken on lr_fill's algorithmic bytes (the check's 8 bytes read per pixel and the
+                     outputs), so it also shows what the labeller's planes cost
+  sceneflow_stream_lr_speckle  sceneflow_stream_lr_fill with speckle_size=100, runs alternating with the _lr_fill ones
 
     python scripts/bench_predictor.py --out DIR
 """
@@ -47,6 +56,7 @@ sys.path.insert(0, str(ROOT))
 
 HBM_GBS = 7700.0
 LR_TOL = 1.0
+SPECKLE = (100, 1.0)           # speckle_size, speckle_range of the lr_speckle legs
 
 
 def gpu_info(torch):
@@ -187,6 +197,56 @@ def hbm_share(nbytes, us):
             "frac_of_hbm_bound": nbytes / (HBM_GBS * 1e9) / (us * 1e-6), "hbm_gbs_assumed": HBM_GBS}
 
 
+def lr_speckle_legs(torch, res):
+    """8. the speckle filter with background hole filling beside background hole filling alone, uint16 output."""
+    from decnet_b200 import ops
+    from decnet_b200._lib import lib
+    dev = torch.device("cuda", 0)
+    for tag, (B, h, w, H, W, nsets) in (("", (8, 540, 960, 540, 972, 6)), ("_middlebury", (1, 2000, 2900, 2025, 2916, 6))):
+        for kind in ("random", "planar"):
+            if kind == "random":
+                tol = LR_TOL
+                preds = [torch.randn(2 * B, H, W, device=dev) * 20 + 40 for _ in range(nsets)]
+            else:
+                tol = 3e38
+                yy = torch.arange(H, device=dev).view(1, H, 1).float()
+                xx = torch.arange(W, device=dev).view(1, 1, W).float()
+                planes = torch.where(xx < W // 3, 0.4 - 1e-4 * xx - 5e-5 * yy, torch.where(yy < H // 2, 1e-4 * xx - 0.45,
+                                                                                           -2e-5 * yy + 0.1))
+                preds = []
+                for i in range(nsets):
+                    fwd = (planes.expand(B, H, W) * 64).round() / 64
+                    holes = torch.rand(B, H, W, device=dev, generator=torch.Generator(device=dev).manual_seed(i)) < 0.03
+                    preds.append(torch.cat([fwd.masked_fill(holes, float("nan")), torch.zeros(B, H, W, device=dev)]))
+            nscratch = int(lib().decnet_lr_speckle_scratch_bytes(B, h, w, 1))
+            outs = [(torch.empty(B, h, w, device=dev), torch.empty(B, h, w, dtype=torch.uint16, device=dev), None,
+                     torch.empty(B, h, dtype=torch.uint8, device=dev)) for _ in range(nsets)]
+            scratch = [torch.empty(nscratch, dtype=torch.uint8, device=dev) for _ in range(nsets)]
+            ptrs = [tuple(o.data_ptr() if o is not None else None for o in outs[i]) for i in range(nsets)]
+            bg = lambda i: ops._call("decnet_lr_check_fill", preds[i], preds[i].data_ptr(), B, H, W, h, w, tol, *ptrs[i])
+            sp = lambda i: ops._call("decnet_lr_check_speckle", preds[i], preds[i].data_ptr(), None, B, H, W, h, w, tol,
+                                     SPECKLE[0], SPECKLE[1], 1, ops.GUIDED_LAMBDA, ops.GUIDED_SIGMA, *ptrs[i],
+                                     scratch[i].data_ptr())
+            runs = {"background": [], "speckle": []}
+            for _ in range(2):                                           # alternating, best of each
+                runs["background"].append(kernel_us(torch, bg, nsets, n=48))
+                runs["speckle"].append(kernel_us(torch, sp, nsets, n=48))
+            t_bg, t_sp = min(runs["background"]), min(runs["speckle"])
+            (valid,) = ops.lr_check(preds[0], h, w, tol, float_out=False, valid_out=True)
+            (kept,) = ops.lr_check(preds[0], h, w, tol, float_out=False, valid_out=True, fill="background",
+                                   speckle_size=SPECKLE[0], speckle_range=SPECKLE[1])
+            nbytes = B * h * w * (8 + 4 + 2) + B * h
+            res[f"lr_speckle_{kind}_u16{tag}"] = dict(
+                hbm_share(nbytes, t_sp), us=t_sp, background_us=t_bg, speckle_over_background=t_sp / t_bg,
+                background_frac_of_hbm_bound=hbm_share(nbytes, t_bg)["frac_of_hbm_bound"], us_runs=runs,
+                shape=f"pred {2 * B}x{H}x{W} -> {B}x{h}x{w}", buffer_sets=nsets, scratch_mb_per_set=nscratch / 1e6,
+                speckle_size=SPECKLE[0], speckle_range=SPECKLE[1], tol=tol, valid_fraction=float(valid.float().mean()),
+                kept_fraction=float(kept.float().mean()),
+                what="decnet_lr_check_speckle (fill 1) vs decnet_lr_check_fill, alternating; 48 launches per graph")
+            del preds, outs, scratch
+            torch.cuda.empty_cache()
+
+
 def run_bench_py():
     cmd = [sys.executable, str(ROOT / "bench.py"), "--gpus", "1", "--steps", "20", "--warmup", "5", "--no-cpu-baseline",
            "--no-extras"]
@@ -246,6 +306,9 @@ def main():
         pass
     for _ in m.stream([pair] * 4, output="u16", lr_check=LR_TOL, fill="guided"):
         pass
+    for _ in m.stream([pair] * 4, output="u16", lr_check=LR_TOL, fill="background", speckle_size=SPECKLE[0],
+                      speckle_range=SPECKLE[1]):
+        pass
     n = args.stream_steps
 
     def run(**kw):
@@ -254,12 +317,14 @@ def main():
         for _ in m.stream([pair] * n, output="u16", **kw):
             pass
         return time.perf_counter() - t0
-    els = {"plain": [], "lr": [], "lr_fill": [], "lr_guided": []}
+    els = {"plain": [], "lr": [], "lr_fill": [], "lr_guided": [], "lr_speckle": []}
     for _ in range(2):                                                   # alternating plain, LR and LR + fill runs
         els["plain"].append(run())
         els["lr"].append(run(lr_check=LR_TOL))
         els["lr_fill"].append(run(lr_check=LR_TOL, fill="background"))
         els["lr_guided"].append(run(lr_check=LR_TOL, fill="guided"))
+        els["lr_speckle"].append(run(lr_check=LR_TOL, fill="background", speckle_size=SPECKLE[0], speckle_range=SPECKLE[1]))
+        els["lr_fill"].append(run(lr_check=LR_TOL, fill="background"))
     el = min(els["plain"])
     rate = B * n / el
     rate_lr = B * n / min(els["lr"])
@@ -289,6 +354,13 @@ def main():
                                          "what": "as sceneflow_stream_lr_fill with fill=\"guided\" "
                                                  "(decnet_lr_check_guided_fill); runs alternate with the plain, _lr and "
                                                  "_lr_fill ones"}
+    rate_speckle = B * n / min(els["lr_speckle"])
+    res["sceneflow_stream_lr_speckle"] = {"batch": B, "steps": n, "lr_check": LR_TOL, "fill": "background",
+                                          "speckle_size": SPECKLE[0], "speckle_range": SPECKLE[1], "pairs_per_s": rate_speckle,
+                                          "ms_per_step": min(els["lr_speckle"]) / n * 1e3,
+                                          "lr_speckle_over_lr_fill_rate": rate_speckle / rate_fill,
+                                          "what": "as sceneflow_stream_lr_fill with the speckle filter (decnet_lr_check_speckle); "
+                                                  "each speckle run sits between two _lr_fill runs"}
     del m
     torch.cuda.empty_cache()
 
@@ -406,6 +478,8 @@ def main():
                                               "compose) vs decnet_lr_check_fill, alternating; 32 launches per graph"}
         del preds, guides, outs
         torch.cuda.empty_cache()
+
+    lr_speckle_legs(torch, res)
     (out / "bench_predictor.json").write_text(json.dumps(res, indent=1))
     print(json.dumps(res))
 

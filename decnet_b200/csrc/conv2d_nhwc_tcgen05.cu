@@ -34,7 +34,18 @@
 // activation tile completes its own mbarrier, so the converters start while the (4x larger) weight part of the stage is still in
 // flight (DESIGN.md section 3.4).
 //
-// Warp roles as in conv3d_tcgen05.cu: 0 TMA producer, 1 MMA issuer, 2-5 epilogue, 6-9 converters (split mode only);
+// split = 3 (split16 input, the default inside the DynamicUpsampling and wide Refinement stacks): the activations arrive already
+// as the operand the fp16 MMAs read, stored by the producing kernel as [fp16(2^11 * (x - h)) x cl | h x cl], h = fp16(x)
+// (common.cuh: split16_store; same 4 bytes per channel as fp32, so the same tensor map loads it).  The converters idle, the hi
+// taps of the weights are gone ([9][NP][cp]: only the fp16 taps of split = 2), and per column tap the issuer runs
+//   small terms: [lo | h] * [hi16(w) ; lo16(w)]   (split = 2's correction MMA, cl/8 K-steps)  -> small-term accumulator
+//   big term:    h * hi16(w)                       (A at +2*cl bytes, the hi16 half of B, cl/16 K-steps) -> the chain slot,
+// which sum to x*hi(w) + h*lo(w) -- the 3xTF32 budget (lo*lo dropped, 11 bits per part).  The chain is drained with 2^-sw
+// (bias[np + 1]).  A stage is 17 KB + 3 x NP x 128 B instead of twice that, so the ring is twice as deep.
+// round_out (the output's storage format): 0 fp32, 1 fp32 rounded to TF32 (for a following split = 0 layer), 2 split16 (for a
+// following split = 3 layer; ldc == np).
+//
+// Warp roles as in conv3d_tcgen05.cu: 0 TMA producer, 1 MMA issuer, 2-5 epilogue, 6-9 converters (split modes 1 and 2 only);
 // persistent CTAs, two TMEM slots.
 #include "common.cuh"
 #include "tma_utils.cuh"
@@ -58,8 +69,8 @@ struct Params {
     int cp, np;
     int nchunks, last_ksteps;
     long long P;                                   // B * (h+2) * (w+2) padded pixels
-    int relu, round_tf32, tmem_cols, num_tiles, stages;
-    int split;                                     // 1: 3xTF32 (hi/lo split of both operands)
+    int relu, out_format, tmem_cols, num_tiles, stages;
+    int split;                                     // 0 TF32, 1 3xTF32, 2 TF32 + fp16 corrections, 3 split16 input
     int taps;                                      // 3: 3x3 conv on the zero-bordered layout; 1: plain GEMM (1x1 conv) over P rows
     int border;                                    // 1: rows are pixels of [B, h+2, w+2] and border pixels are stored as zeros
     int ldc;                                       // output row stride in floats (>= np: writes a channel slice of a wider tensor)
@@ -230,7 +241,8 @@ conv2d_nhwc_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
     unsigned char *base = reinterpret_cast<unsigned char *>(
         (reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
     const int b_tap_bytes = p.np * 128;                       // one column tap of the weights: NP rows x 128 B
-    const int nsplit = p.split ? 2 : 1;
+    const bool conv_mode = p.split == 1 || p.split == 2;      // the converters build a second A tile, two weight blocks
+    const int nsplit = conv_mode ? 2 : 1;
     const int T = p.taps;                                     // taps per dimension: 3 (conv) or 1 (GEMM)
     const int a_rows = T == 3 ? kARows : kTileM;
     const int b_off = nsplit * kABytes;                       // stage: [A hi][A lo][B hi (T taps)][B lo (T taps)]
@@ -277,9 +289,9 @@ conv2d_nhwc_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
                         const bool skip_b = (p.dbg & 8) && nfill >= kStages;
                         if (p.trace && blockIdx.x == 0 && nfill < 256) p.trace[nfill * 8 + 0] = clock64();
                         ++nfill;
-                        // split mode: the activation tile completes its own barrier, which is all the converters wait for
-                        uint64_t *abar = p.split ? &afull_bar[s] : &full_bar[s];
-                        if (p.split) {
+                        // converter modes: the activation tile completes its own barrier, which is all the converters wait for
+                        uint64_t *abar = conv_mode ? &afull_bar[s] : &full_bar[s];
+                        if (conv_mode) {
                             mbar_arrive_expect_tx(abar, (uint32_t)(a_rows * 128));
                             if (skip_b) mbar_arrive(&full_bar[s]);
                             else mbar_arrive_expect_tx(&full_bar[s], (uint32_t)(tx_bytes - a_rows * 128));
@@ -289,7 +301,7 @@ conv2d_nhwc_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
                         tma_load_2d(sa, &tmA, ck * 32, T == 3 ? p0 + (kh - 1) * pitch - 1 : p0, abar);
                         if (!skip_b) {
                         tma_load_3d(sa + b_off, &tmB, ck * 32, 0, kh * T, &full_bar[s]);
-                        if (p.split) tma_load_3d(sa + b_off + T * b_tap_bytes, &tmB, ck * 32, 0, T * T + kh * T, &full_bar[s]);
+                        if (conv_mode) tma_load_3d(sa + b_off + T * b_tap_bytes, &tmB, ck * 32, 0, T * T + kh * T, &full_bar[s]);
                         }
                         if (++s == kStages) { s = 0; ph ^= 1u; }
                     }
@@ -327,8 +339,8 @@ conv2d_nhwc_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
                             acc_b = tmem_base + slot * (uint32_t)acc_stride;
                             first_b = 0u;
                         }
-                        if (!ready) mbar_wait(&ready_bar[s], ph);
-                        mbar_wait(&full_bar[s], ph);                      // the weights of the stage
+                        if (!ready && conv_mode) mbar_wait(&ready_bar[s], ph);
+                        mbar_wait(&full_bar[s], ph);                      // the weights of the stage (split = 3: the whole stage)
                         const bool tr = p.trace && blockIdx.x == 0 && lane == 0 && nmma < 256;
                         if (tr) p.trace[nmma * 8 + 3] = clock64();
                         tc_fence_after();
@@ -338,9 +350,14 @@ conv2d_nhwc_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
                         const uint64_t db_lo = make_desc_sw128(sa + (uint32_t)(b_off + T * b_tap_bytes));
                         int sn = s + 1; uint32_t phn = ph;
                         if (sn == kStages) { sn = 0; phn ^= 1u; }
-                        ready = mbar_test_wait(&ready_bar[sn], phn);
+                        ready = conv_mode && mbar_test_wait(&ready_bar[sn], phn);
                         const int ks = ck == p.nchunks - 1 ? p.last_ksteps : 4;
-                        if (p.dbg & 2) {
+                        if (p.split == 3) {
+                            // split16 tile [lo | h] (cl = 8 ks channels): small terms over all 2 cl halves, h * hi16(w) over the
+                            // h half (ks 16-byte units in) and the hi16 half of B
+                            if (!(p.dbg & 2)) umma_taps3_f16(ks, acc_s, da, db, db_tap_step, idesc16, first_s, T);
+                            if (!(p.dbg & 4)) umma_taps3_f16(ks >> 1, acc_b, da + (uint64_t)ks, db, db_tap_step, idesc16, first_b, T);
+                        } else if (p.dbg & 2) {
                         } else if (p.split == 2) {
                             // [lo16(x) | fp16(x)] * [hi16(w) ; lo16(w)]: both correction terms, K-concatenated fp16
                             umma_taps3_f16(ks, acc_s, da_lo, db_lo, db_tap_step, idesc16, first_s, T);
@@ -348,7 +365,7 @@ conv2d_nhwc_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
                             umma_taps3(ks, acc_s, da_lo, db, db_tap_step, idesc, first_s, T); // lo(x) * hi(w)
                             umma_taps3(ks, acc_s, da, db_lo, db_tap_step, idesc, 1u, T);      // hi(x) * lo(w)
                         }
-                        if (!(p.dbg & 4))
+                        if (!(p.dbg & 4) && p.split != 3)
                         umma_taps3(ks, acc_b, da, db, db_tap_step, idesc, first_b, T);        // hi(x) * hi(w)
                         first_s = 1u; first_b = 1u;
                         umma_commit_elect(empty_base + (uint32_t)(s * 8));
@@ -386,8 +403,8 @@ conv2d_nhwc_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
             }
         }
     } else if (warp >= 6) {
-        // ===================== converters (warps 6..9, split mode): hi in place, lo beside it =====================
-        if (p.split) {
+        // ===================== converters (warps 6..9, split modes 1 and 2): hi in place, lo beside it =====================
+        if (conv_mode) {
             const int ctid = threadIdx.x - 6 * 32;
             const int n16 = a_rows * 128 / 16;                    // 16-byte words TMA delivered for A
             int s = 0; uint32_t ph = 0;
@@ -441,25 +458,28 @@ conv2d_nhwc_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
                 dst = (b * (p.dst_h + 2) + yy + 1) * (p.dst_w + 2) + xx + 1;
             }
         };
-        // bias / ReLU / optional TF32 rounding / zero border, 16 channels from c0
+        // bias / ReLU / storage format (out_format) / zero border, 16 channels from c0
         auto store16 = [&](const float (&v)[16], long long pix, bool interior, int c0) {
             const float4 *bp = reinterpret_cast<const float4 *>(p.bias + c0);
-            float4 *op = reinterpret_cast<float4 *>(p.out + pix * p.ldc + c0);
+            float o[16];
 #pragma unroll
             for (int i4 = 0; i4 < 4; ++i4) {
-                float4 o = make_float4(0.f, 0.f, 0.f, 0.f);
-                if (interior) {
-                    const float4 bv = __ldg(bp + i4);
-                    o = make_float4(v[4 * i4] + bv.x, v[4 * i4 + 1] + bv.y, v[4 * i4 + 2] + bv.z, v[4 * i4 + 3] + bv.w);
-                    if (p.relu) { o.x = fmaxf(o.x, 0.f); o.y = fmaxf(o.y, 0.f); o.z = fmaxf(o.z, 0.f); o.w = fmaxf(o.w, 0.f); }
-                    if (p.round_tf32) {
-                        o.x = __uint_as_float((__float_as_uint(o.x) + 0x1000u) & 0xFFFFE000u);
-                        o.y = __uint_as_float((__float_as_uint(o.y) + 0x1000u) & 0xFFFFE000u);
-                        o.z = __uint_as_float((__float_as_uint(o.z) + 0x1000u) & 0xFFFFE000u);
-                        o.w = __uint_as_float((__float_as_uint(o.w) + 0x1000u) & 0xFFFFE000u);
-                    }
-                }
-                op[i4] = o;
+                const float4 bv = interior ? __ldg(bp + i4) : make_float4(0.f, 0.f, 0.f, 0.f);
+                o[4 * i4] = v[4 * i4] + bv.x; o[4 * i4 + 1] = v[4 * i4 + 1] + bv.y;
+                o[4 * i4 + 2] = v[4 * i4 + 2] + bv.z; o[4 * i4 + 3] = v[4 * i4 + 3] + bv.w;
+            }
+#pragma unroll
+            for (int i = 0; i < 16; ++i) {
+                if (p.relu) o[i] = fmaxf(o[i], 0.f);
+                if (p.out_format == 1) o[i] = __uint_as_float((__float_as_uint(o[i]) + 0x1000u) & 0xFFFFE000u);
+                if (!interior) o[i] = 0.f;
+            }
+            if (p.out_format == 2) {
+                split16_store<16>(p.out + pix * p.ldc, p.np, c0, o);
+            } else {
+                float4 *op = reinterpret_cast<float4 *>(p.out + pix * p.ldc + c0);
+#pragma unroll
+                for (int i4 = 0; i4 < 4; ++i4) op[i4] = make_float4(o[4 * i4], o[4 * i4 + 1], o[4 * i4 + 2], o[4 * i4 + 3]);
             }
         };
         if (p.split) {
@@ -481,8 +501,10 @@ conv2d_nhwc_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
                 tc_fence_before();
                 __syncwarp();
             };
-            // split = 2: the correction accumulator holds 2^(11+sw) x the value (see the weight packer); bias[np] = 2^-(11+sw)
-            const float small_scale = p.split == 2 ? __ldg(p.bias + p.np) : 1.f;
+            // split = 2, 3: the correction accumulator holds 2^(11+sw) x the value (see the weight packer); bias[np] = 2^-(11+sw);
+            // split = 3: the chains hold 2^sw x the big term; bias[np + 1] = 2^-sw
+            const float small_scale = p.split >= 2 ? __ldg(p.bias + p.np) : 1.f;
+            const float big_scale = p.split == 3 ? __ldg(p.bias + p.np + 1) : 1.f;
             uint32_t it = 0, j = 0;
             for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++j) {
                 const long long pix = (long long)tile * kTileM + r;
@@ -499,7 +521,7 @@ conv2d_nhwc_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
                     const bool tr = p.trace && blockIdx.x == 0 && warp == 2 && lane == 0 && it < 256;
                     if (tr) p.trace[2048 + it * 2] = clock64();
                     tc_fence_after();
-                    drain(lane_base + slot * (uint32_t)acc_stride, 1.f);
+                    drain(lane_base + slot * (uint32_t)acc_stride, big_scale);
                     if (tr) p.trace[2048 + it * 2 + 1] = clock64();
                     if (lane == 0) mbar_arrive(&tmem_empty_bar[slot]);
                 }
@@ -808,16 +830,19 @@ extern "C" {
 // tensor and border rows are stored as zeros; dst_h > 0: the P = B*dst_h*dst_w rows of a flat grid are stored at the interior
 // pixels of a bordered [B, dst_h+2, dst_w+2, ldc] tensor).
 static int launch_nhwc(const float *x, const float *w_packed, const float *bias, float *out, long long P, int B, int h, int w,
-                       int cp, int np, int taps, int border, int relu, int round_out_tf32, int split, int ldc, int dst_h, int dst_w,
+                       int cp, int np, int taps, int border, int relu, int round_out, int split, int ldc, int dst_h, int dst_w,
                        void *stream)
 {
     DECNET_REQUIRE(x && w_packed && bias && out, "null pointer");
     DECNET_REQUIRE(P > 0, "non-positive size");
     DECNET_REQUIRE(cp % 8 == 0 && cp >= 8 && cp <= 8192, "cp=%d must be a multiple of 8", cp);
     DECNET_REQUIRE(np % 16 == 0 && np >= 16 && np <= 256, "np=%d must be a multiple of 16 in [16,256]", np);
-    DECNET_REQUIRE(split >= 0 && split <= 2, "split must be 0 (TF32), 1 (3xTF32) or 2 (TF32 + fp16 corrections)");
+    DECNET_REQUIRE(split >= 0 && split <= 3, "split must be 0 (TF32), 1 (3xTF32), 2 (TF32 + fp16 corrections) or 3 (split16 input)");
     DECNET_REQUIRE(!split || np <= 128, "split (3xTF32) mode accumulates in registers: np=%d must be <= 128", np);
+    DECNET_REQUIRE(split != 3 || cp % 16 == 0, "split16 input needs cp %% 16 == 0, got cp=%d", cp);
     DECNET_REQUIRE(ldc >= np && ldc % 4 == 0, "ldc=%d must be a multiple of 4 and >= np=%d", ldc, np);
+    DECNET_REQUIRE(round_out >= 0 && round_out <= 2, "round_out=%d must be 0 (fp32), 1 (TF32-rounded) or 2 (split16)", round_out);
+    DECNET_REQUIRE(round_out != 2 || ldc == np, "split16 output needs ldc == np");
     DECNET_REQUIRE((reinterpret_cast<uintptr_t>(x) & 15u) == 0 && (reinterpret_cast<uintptr_t>(w_packed) & 15u) == 0 &&
                    (reinterpret_cast<uintptr_t>(out) & 15u) == 0 && (reinterpret_cast<uintptr_t>(bias) & 15u) == 0,
                    "pointers must be 16-byte aligned");
@@ -830,11 +855,12 @@ static int launch_nhwc(const float *x, const float *w_packed, const float *bias,
     p.last_ksteps = (cp - (p.nchunks - 1) * 32) / 8;
     p.P = P;
     DECNET_REQUIRE(p.P + 2ll * (w + 3) < (1ll << 31), "tensor too large for 32-bit TMA coordinates");
-    p.relu = relu; p.round_tf32 = round_out_tf32; p.split = split;
+    p.relu = relu; p.out_format = round_out; p.split = split;
+    const bool conv_mode = split == 1 || split == 2;
     p.tmem_cols = np <= 16 ? 32 : np <= 32 ? 64 : np <= 64 ? 128 : np <= 128 ? 256 : 512;
     if (p.split) p.tmem_cols *= 2;                                  // two chain slots + two small-term slots
     p.num_tiles = (int)((p.P + kTileM - 1) / kTileM);
-    const size_t stage_bytes = ((size_t)kABytes + (size_t)taps * np * 128) * (p.split ? 2 : 1);
+    const size_t stage_bytes = ((size_t)kABytes + (size_t)taps * np * 128) * (conv_mode ? 2 : 1);
     p.stages = (int)((226 * 1024 - 1024) / stage_bytes);
     if (p.stages > kMaxStages) p.stages = kMaxStages;
     DECNET_REQUIRE(p.stages >= 2, "stage too large (np=%d)", np);
@@ -849,7 +875,7 @@ static int launch_nhwc(const float *x, const float *w_packed, const float *bias,
         if (rc) return rc;
     }
     {
-        const uint64_t dims[3] = {(uint64_t)cp, (uint64_t)np, (uint64_t)(taps * taps * (p.split ? 2 : 1))};
+        const uint64_t dims[3] = {(uint64_t)cp, (uint64_t)np, (uint64_t)(taps * taps * (conv_mode ? 2 : 1))};
         const uint64_t strides[2] = {(uint64_t)cp * 4, (uint64_t)np * cp * 4};
         const uint32_t box[3] = {32u, (uint32_t)np, (uint32_t)taps};
         int rc = encode_tensor_map(&tmB, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, w_packed, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B,
@@ -869,7 +895,7 @@ static int launch_nhwc(const float *x, const float *w_packed, const float *bias,
     }
     const int sms = sm_count_cached();
     // opt-in (variant 2): two tiles per CTA share each weight stage (pair kernel; exact, measured slower: see its header)
-    if (p.split && np <= 16 * kPairChunks && p.num_tiles >= 2 * sms && g_halo_variant == 2 && !round_out_tf32) {
+    if (conv_mode && np <= 16 * kPairChunks && p.num_tiles >= 2 * sms && g_halo_variant == 2 && !round_out) {
         const size_t b_slot = (size_t)2 * taps * np * 128, a_slot = (size_t)2 * kABytes;
         int na = (int)((226 * 1024 - 1024 - 2 * b_slot) / a_slot);
         if (na > kMaxASlots) na = kMaxASlots;
@@ -904,11 +930,11 @@ void decnet_conv2d_nhwc_set_variant(int variant) { g_halo_variant = variant; }
 void decnet_conv2d_nhwc_debug_trace(void *buffer) { g_halo_trace = static_cast<long long *>(buffer); }
 
 int decnet_conv2d_tc_nhwc_halo(const float *x_pad, const float *w_packed, const float *bias, float *out_pad,
-                               int B, int h, int w, int cp, int np, int relu, int round_out_tf32, int split, void *stream)
+                               int B, int h, int w, int cp, int np, int relu, int round_out, int split, void *stream)
 {
     DECNET_REQUIRE(B > 0 && h > 0 && w > 0, "non-positive size");
     return launch_nhwc(x_pad, w_packed, bias, out_pad, (long long)B * (h + 2) * (w + 2), B, h, w, cp, np, 3, 1, relu,
-                       round_out_tf32, split, np, 0, 0, stream);
+                       round_out, split, np, 0, 0, stream);
 }
 
 int decnet_conv2d_tc_nhwc_halo_ldc(const float *x_pad, const float *w_packed, const float *bias, float *out_pad,

@@ -367,7 +367,7 @@ dynup_glue_kernel(const float *__restrict__ logits, const float *__restrict__ di
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(kBlock)
 dynup_pack_nhwc_kernel(const float *__restrict__ disp, const float *__restrict__ Lf, float *__restrict__ out,
-                       int C, int h, int w, int CP, int TX, int round_tf32, int pad)
+                       int C, int h, int w, int CP, int TX, int fmt, int pad)
 {
     // pad = 1: the output is [B, h+2, w+2, CP] with a zero border (decnet_conv2d_tf32_nhwc_halo's layout); blockIdx.y
     // then runs over h+2 rows: the two border rows are zero-filled, interior rows get a zero pixel at both ends
@@ -423,10 +423,11 @@ dynup_pack_nhwc_kernel(const float *__restrict__ disp, const float *__restrict__
         for (int e = 0; e < 4; ++e) {
             const int l = lut[4 * c4 + e];
             float v = l >= 0 ? rows[l + 3 * xl] : ((l == -2 && disp) ? __ldg(db + xl) : 0.f);
-            if (round_tf32) v = __uint_as_float((__float_as_uint(v) + 0x1000u) & 0xFFFFE000u);   // == cvt.rna.tf32
+            if (fmt == 1) v = __uint_as_float((__float_as_uint(v) + 0x1000u) & 0xFFFFE000u);   // == cvt.rna.tf32
             o[e] = v;
         }
-        ob[i] = make_float4(o[0], o[1], o[2], o[3]);
+        if (fmt == 2) split16_store<4>(ob + (i - c4), CP, 4 * c4, o);
+        else ob[i] = make_float4(o[0], o[1], o[2], o[3]);
         xl += dxl; c4 += dc4;
         if (c4 >= cp4) { c4 -= cp4; ++xl; }
     }
@@ -436,16 +437,18 @@ dynup_pack_nhwc_kernel(const float *__restrict__ disp, const float *__restrict__
 // packed ahead of time, on another stream, with disp = NULL.
 __global__ void __launch_bounds__(kBlock)
 dynup_set_disp_nhwc_kernel(const float *__restrict__ disp, float *__restrict__ out, int h, int w, int CP,
-                           int round_tf32, int pad, long long n)
+                           int fmt, int pad, long long n)
 {
     const long long i = (long long)blockIdx.x * kBlock + threadIdx.x;
     if (i >= n) return;
     const int x = (int)(i % w);
     const long long t = i / w;
     const int y = (int)(t % h), b = (int)(t / h);
-    float v = __ldg(disp + i);
-    if (round_tf32) v = __uint_as_float((__float_as_uint(v) + 0x1000u) & 0xFFFFE000u);
-    out[(((size_t)b * (h + 2 * pad) + y + pad) * (w + 2 * pad) + x + pad) * CP] = v;
+    float v[1] = {__ldg(disp + i)};
+    float *px = out + (((size_t)b * (h + 2 * pad) + y + pad) * (w + 2 * pad) + x + pad) * CP;
+    if (fmt == 2) { split16_store<1>(px, CP, 0, v); return; }
+    if (fmt == 1) v[0] = __uint_as_float((__float_as_uint(v[0]) + 0x1000u) & 0xFFFFE000u);
+    *px = v[0];
 }
 
 // Block = 32 coarse pixels of one row x 9 sub-pixels (288 threads).  The 32 x NP logits are staged through
@@ -508,13 +511,13 @@ dynup_glue_nhwc_kernel(const float *__restrict__ logits, const float *__restrict
 // Layout bridges for the wide (72-channel) refinement layers of the 1/9 level, which run on the zero-bordered
 // channels-last TF32 kernel (conv2d_nhwc_tcgen05.cu):
 //   nchw_cat_to_nhwc_pad : cat of up to three NCHW sources -> [B, h+2, w+2, CP] (border and channel padding zero;
-//                          round_tf32: values rounded to TF32 for the kernel's plain-TF32 mode)
+//                          fmt 0: fp32, 1: rounded to TF32 for the kernel's plain-TF32 mode, 2: split16, see common.cuh)
 //   nhwc_pad_to_nchw     : interior of [B, h+2, w+2, NP], first C channels -> NCHW [B, C, h, w]
 // The tensors are small (52 k pixels at SceneFlow size); one thread per output element.
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(kBlock)
 nchw_cat_to_nhwc_pad_kernel(const float *__restrict__ s0, const float *__restrict__ s1, const float *__restrict__ s2,
-                            int c0, int c1, int c2, float *__restrict__ out, int h, int w, int CP, int round_tf32, long long n)
+                            int c0, int c1, int c2, float *__restrict__ out, int h, int w, int CP, int fmt, long long n)
 {
     const long long i = (long long)blockIdx.x * kBlock + threadIdx.x;      // over B*(h+2)*(w+2)*CP
     if (i >= n) return;
@@ -529,9 +532,14 @@ nchw_cat_to_nhwc_pad_kernel(const float *__restrict__ s0, const float *__restric
         if (c < c0) v = __ldg(s0 + (b * c0 + c) * plane + pix);
         else if (c < c0 + c1) v = __ldg(s1 + (b * c1 + (c - c0)) * plane + pix);
         else v = __ldg(s2 + (b * c2 + (c - c0 - c1)) * plane + pix);
-        if (round_tf32) v = __uint_as_float((__float_as_uint(v) + 0x1000u) & 0xFFFFE000u);
+        if (fmt == 1) v = __uint_as_float((__float_as_uint(v) + 0x1000u) & 0xFFFFE000u);
     }
-    out[i] = v;
+    if (fmt == 2) {
+        const float r[1] = {v};
+        split16_store<1>(out + (i - c), CP, c, r);
+    } else {
+        out[i] = v;
+    }
 }
 
 // Tiled form of the kernel above for CP % 4 == 0 (the product shapes): a block owns 32 padded pixels of one row; warps read one
@@ -540,7 +548,7 @@ nchw_cat_to_nhwc_pad_kernel(const float *__restrict__ s0, const float *__restric
 // 32 different planes per warp load (52 us for 33 MB at the 1/9 level).
 __global__ void __launch_bounds__(kBlock)
 nchw_cat_to_nhwc_pad_tiled_kernel(const float *__restrict__ s0, const float *__restrict__ s1, const float *__restrict__ s2,
-                                  int c0, int c1, int c2, float *__restrict__ out, int h, int w, int CP, int round_tf32)
+                                  int c0, int c1, int c2, float *__restrict__ out, int h, int w, int CP, int fmt)
 {
     extern __shared__ float tile[];                        // [32][CP + 1]
     const int xp0 = blockIdx.x * 32, yp = blockIdx.y, b = blockIdx.z;
@@ -557,7 +565,7 @@ nchw_cat_to_nhwc_pad_tiled_kernel(const float *__restrict__ s0, const float *__r
                              : c < c0 + c1 ? s1 + ((size_t)b * c1 + (c - c0)) * plane
                                            : s2 + ((size_t)b * c2 + (c - c0 - c1)) * plane;
             v = __ldg(src + pix);
-            if (round_tf32) v = __uint_as_float((__float_as_uint(v) + 0x1000u) & 0xFFFFE000u);
+            if (fmt == 1) v = __uint_as_float((__float_as_uint(v) + 0x1000u) & 0xFFFFE000u);
         }
         tile[lane * ts + c] = v;
     }
@@ -568,7 +576,12 @@ nchw_cat_to_nhwc_pad_tiled_kernel(const float *__restrict__ s0, const float *__r
     const int dpx = kBlock / cp4, dc4 = kBlock - dpx * cp4;
     for (int i = threadIdx.x; i < total4; i += kBlock) {
         const float *t = tile + px * ts + 4 * c4;
-        ob[i] = make_float4(t[0], t[1], t[2], t[3]);
+        if (fmt == 2) {
+            const float r[4] = {t[0], t[1], t[2], t[3]};
+            split16_store<4>(ob + (i - c4), CP, 4 * c4, r);
+        } else {
+            ob[i] = make_float4(t[0], t[1], t[2], t[3]);
+        }
         px += dpx; c4 += dc4;
         if (c4 >= cp4) { c4 -= cp4; ++px; }
     }
@@ -869,6 +882,13 @@ static inline int grid_for(long long n, int cap = 148 * 16) {
 using namespace decnet;
 using namespace decnet::glue;
 
+// the storage format of the channels-last writers: 0 fp32, 1 fp32 rounded to TF32, 2 split16 (common.cuh)
+static int check_format(int format, int CP) {
+    DECNET_REQUIRE(format >= 0 && format <= 2, "format=%d must be 0 (fp32), 1 (TF32-rounded) or 2 (split16)", format);
+    DECNET_REQUIRE(format != 2 || CP % 16 == 0, "split16 storage needs CP %% 16 == 0, got CP=%d", CP);
+    return 0;
+}
+
 extern "C" {
 
 int decnet_costvol_fwd(const float *L, const float *R, float *vol, int B, int C, int H, int W, int D, void *stream) {
@@ -967,8 +987,9 @@ int decnet_dynup_glue(const float *logits, const float *disp, float *out, int B,
 }
 
 int decnet_nchw_cat_to_nhwc_pad(const float *const *srcs, const int *src_channels, int nsrc, float *out,
-                                int B, int h, int w, int CP, int round_tf32, void *stream) {
+                                int B, int h, int w, int CP, int format, void *stream) {
     DECNET_REQUIRE(srcs && src_channels && out, "null pointer");
+    if (int rc = check_format(format, CP)) return rc;
     DECNET_REQUIRE(nsrc >= 1 && nsrc <= 3 && B > 0 && h > 0 && w > 0, "bad size");
     int c[3] = {0, 0, 0};
     const float *s[3] = {nullptr, nullptr, nullptr};
@@ -979,12 +1000,12 @@ int decnet_nchw_cat_to_nhwc_pad(const float *const *srcs, const int *src_channel
     if ((CP & 3) == 0 && tile_bytes <= 48 * 1024 && h + 2 <= 65535 && B <= 65535 &&
         (reinterpret_cast<uintptr_t>(out) & 15u) == 0) {
         nchw_cat_to_nhwc_pad_tiled_kernel<<<dim3((w + 2 + 31) / 32, h + 2, B), kBlock, tile_bytes, (cudaStream_t)stream>>>(
-            s[0], s[1], s[2], c[0], c[1], c[2], out, h, w, CP, round_tf32);
+            s[0], s[1], s[2], c[0], c[1], c[2], out, h, w, CP, format);
         return after_launch("nchw_cat_to_nhwc_pad_tiled_kernel");
     }
     const long long n = (long long)B * (h + 2) * (w + 2) * CP;
     nchw_cat_to_nhwc_pad_kernel<<<(unsigned)((n + kBlock - 1) / kBlock), kBlock, 0, (cudaStream_t)stream>>>(s[0], s[1], s[2], c[0], c[1], c[2],
-                                                                                                     out, h, w, CP, round_tf32, n);
+                                                                                                     out, h, w, CP, format, n);
     return after_launch("nchw_cat_to_nhwc_pad_kernel");
 }
 
@@ -1068,9 +1089,10 @@ int decnet_haar_level(const float *x, float *ll, float *detail, float *mask, voi
 }
 
 int decnet_dynup_pack_nhwc(const float *disp, const float *left_fea, float *out, int B, int C, int h, int w, int CP,
-                           int round_tf32, int pad, void *stream) {
+                           int format, int pad, void *stream) {
     DECNET_REQUIRE(pad == 0 || pad == 1, "pad must be 0 or 1");
-    DECNET_REQUIRE(left_fea && out, "null pointer");         // disp may be NULL: channel 0 is written as zero
+    DECNET_REQUIRE(left_fea && out, "null pointer");
+    if (int rc = check_format(format, CP)) return rc;         // disp may be NULL: channel 0 is written as zero
     DECNET_REQUIRE(B > 0 && B <= 65535 && C > 0 && h > 0 && h <= 65535 && w > 0, "bad size");
     DECNET_REQUIRE(CP >= 9 * C + 1, "CP=%d must hold 9*C+1=%d channels", CP, 9 * C + 1);
     int TX = 1200 / C;                            // <= 43 KB of shared memory: 5 blocks per SM
@@ -1083,18 +1105,19 @@ int decnet_dynup_pack_nhwc(const float *disp, const float *left_fea, float *out,
         DECNET_CUDA(cudaFuncSetAttribute(dynup_pack_nhwc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     DECNET_REQUIRE(h + 2 <= 65535, "too many rows");
     dynup_pack_nhwc_kernel<<<dim3((w + TX - 1) / TX, h + 2 * pad, B), kBlock, smem, (cudaStream_t)stream>>>(disp, left_fea, out, C, h, w, CP, TX,
-                                                                                                        round_tf32, pad);
+                                                                                                        format, pad);
     return after_launch("dynup_pack_nhwc_kernel");
 }
 
-int decnet_dynup_set_disp_nhwc(const float *disp, float *packed, int B, int h, int w, int CP, int round_tf32, int pad,
+int decnet_dynup_set_disp_nhwc(const float *disp, float *packed, int B, int h, int w, int CP, int format, int pad,
                                void *stream) {
     DECNET_REQUIRE(pad == 0 || pad == 1, "pad must be 0 or 1");
     DECNET_REQUIRE(disp && packed, "null pointer");
     DECNET_REQUIRE(B > 0 && h > 0 && w > 0 && CP > 0, "bad size");
+    if (int rc = check_format(format, CP)) return rc;
     const long long n = (long long)B * h * w;
     dynup_set_disp_nhwc_kernel<<<(unsigned)((n + kBlock - 1) / kBlock), kBlock, 0, (cudaStream_t)stream>>>(
-        disp, packed, h, w, CP, round_tf32, pad, n);
+        disp, packed, h, w, CP, format, pad, n);
     return after_launch("dynup_set_disp_nhwc_kernel");
 }
 

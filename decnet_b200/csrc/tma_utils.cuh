@@ -103,11 +103,6 @@ __device__ __forceinline__ void tma_load_5d(void *dst, const CUtensorMap *tm, in
 // the low half:
 //   lo16 = fp16(2^11 * (x - trunc_tf32(x)))   (the residual has <= 13 significant bits; fp16 keeps 11, like the TF32 lo part)
 //   hi16 = fp16(x)                            (multiplies the 2^-11-sized lo part of the weights: its 2^-11 rounding is 2^-22 overall)
-__device__ __forceinline__ uint32_t cvt_f16x2_sat(float hi_half, float lo_half) {
-    uint32_t d;
-    asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(hi_half), "f"(lo_half));
-    return d;
-}
 __device__ __forceinline__ uint32_t lo16x2(uint32_t a, uint32_t b) {
     const float fa = (__uint_as_float(a) - __uint_as_float(a & 0xFFFFE000u)) * 2048.f;
     const float fb = (__uint_as_float(b) - __uint_as_float(b & 0xFFFFE000u)) * 2048.f;

@@ -74,6 +74,19 @@ def _split(unit) -> int:
     return ops.SPLIT_KIND if unit.precision == "fp32" else 0
 
 
+def _split16(split) -> bool:
+    """Whether a channels-last halo-conv stack stores the activations it chains on as split16 (common.cuh): with the fp16
+    corrections (split kind 2) the producers write the operand the conv's MMAs read, so the conv needs no converter pass;
+    only the stack's last layer writes fp32 for the glue after it."""
+    return split == 2
+
+
+def _stack_cp(cin, split) -> int:
+    """The channel padding of a stack's first input: whole 8-channel K-steps, 16 for split16 storage."""
+    m = 16 if _split16(split) else 8
+    return (cin + m - 1) // m * m
+
+
 # --------------------------------------------------------------------------------------
 # units with the reference's parameter names (conv.weight / conv.bias / bn.*)
 # --------------------------------------------------------------------------------------
@@ -388,22 +401,22 @@ class DynamicUpsampling(_Cached, nn.Module):
 
         def build():
             units = list(self.weight_learning)
-            cin0 = units[0].conv.in_channels
-            cp = (cin0 + 7) // 8 * 8
+            cp0 = cp = _stack_cp(units[0].conv.in_channels, split)
             packed = []
             for u in units:
                 w, b = u.folded()
-                wp, bp, np_ = ops.pack_conv2d_tf32_weights(w, b, cp, split=split)
+                wp, bp, np_ = ops.pack_conv2d_tf32_weights(w, b, cp, split=split, split16_in=_split16(split))
                 packed.append((wp, bp, u.relu))
                 cp = np_
-            return ((cin0 + 7) // 8 * 8, packed)
+            return (cp0, packed)
         return self._cached(("pack", split), build)
 
     def prepack(self, left_fea):
         """The feature channels of the conv input (everything but the disparity channel).  Independent of the
         disparity: the stage loop runs it ahead, on its second stream."""
         cp0, _ = self._pack()
-        return ops.dynup_pack_nhwc(None, left_fea.contiguous(), cp0, round_tf32=not _split(self), pad=True)
+        split = _split(self)
+        return ops.dynup_pack_nhwc(None, left_fea.contiguous(), cp0, round_tf32=not split, pad=True, split16=_split16(split))
 
     def forward(self, disp_map, left_fea, packed=None):
         disp_map = disp_map.contiguous()
@@ -413,9 +426,11 @@ class DynamicUpsampling(_Cached, nn.Module):
         if packed is not None:
             x = ops.dynup_set_disp_nhwc(packed, disp_map, round_tf32=not split, pad=True)   # features packed ahead (prepack)
         else:
-            x = ops.dynup_pack_nhwc(disp_map, left_fea.contiguous(), cp0, round_tf32=not split, pad=True)
+            x = ops.dynup_pack_nhwc(disp_map, left_fea.contiguous(), cp0, round_tf32=not split, pad=True, split16=_split16(split))
         for i, (wp, bp, relu) in enumerate(packed_w):
-            x = ops.conv2d_tf32_nhwc_halo(x, wp, bp, relu, round_out=(not split) and i + 1 < len(packed_w), split=split)
+            inner = i + 1 < len(packed_w)
+            x = ops.conv2d_tf32_nhwc_halo(x, wp, bp, relu, round_out=(not split) and inner, split=split,
+                                          split16_out=_split16(split) and inner)
         return ops.dynup_glue_nhwc(x, disp_map, pad=True)
 
 
@@ -477,14 +492,14 @@ class Refinement(_Cached, nn.Module):
 
         def build():
             units = list(self.conv)
-            cp = (units[0].conv.in_channels + 7) // 8 * 8
+            cp0 = cp = _stack_cp(units[0].conv.in_channels, split)
             packed = []
             for u in units[:n_wide]:
                 w, b = u.folded()
-                wp, bp, np_ = ops.pack_conv2d_tf32_weights(w, b, cp, split=split)
+                wp, bp, np_ = ops.pack_conv2d_tf32_weights(w, b, cp, split=split, split16_in=_split16(split))
                 packed.append((wp, bp, u.relu))
                 cp = np_
-            return ((units[0].conv.in_channels + 7) // 8 * 8, packed)
+            return (cp0, packed)
         return self._cached(("wide", split, n_wide), build)
 
     def _is_wide(self):
@@ -496,9 +511,11 @@ class Refinement(_Cached, nn.Module):
         kernel -> zero-bordered channels-last kernel between two layout bridges; returns the NCHW input of layer 4."""
         split = _split(self)
         cp0, packed = self._wide_pack(4)
-        x = ops.nchw_cat_to_nhwc_pad(srcs, cp0, round_tf32=not split)
+        x = ops.nchw_cat_to_nhwc_pad(srcs, cp0, round_tf32=not split, split16=_split16(split))
         for i, (wp, bp, relu) in enumerate(packed):
-            x = ops.conv2d_tf32_nhwc_halo(x, wp, bp, relu, round_out=(not split) and i + 1 < len(packed), split=split)
+            inner = i + 1 < len(packed)
+            x = ops.conv2d_tf32_nhwc_halo(x, wp, bp, relu, round_out=(not split) and inner, split=split,
+                                          split16_out=_split16(split) and inner)
         return ops.nhwc_pad_to_nchw(x, self.conv[3].conv.out_channels)
 
     def _tail(self, x, disp_map, start, wv, want_residual=True):

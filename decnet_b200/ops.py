@@ -25,12 +25,13 @@ def _call(name, t, *args):
     _lib.check(st, name)
 
 
-def _chk(name: str, t: torch.Tensor, ref: torch.Tensor | None = None, shape=None) -> None:
+def _chk(name: str, t: torch.Tensor, ref: torch.Tensor | None = None, shape=None, split16_ok=False) -> None:
+    """split16_ok: fp16 is accepted too, as the split16 storage of a channels-last tensor (see conv2d_tf32_nhwc_halo)."""
     if not isinstance(t, torch.Tensor):
         raise TypeError(f"{name} must be a torch.Tensor")
     if not t.is_cuda:
         raise _lib.DecnetError(f"{name} must be a CUDA tensor (decnet_b200 has no CPU path)")
-    if t.dtype != torch.float32:
+    if t.dtype != torch.float32 and not (split16_ok and t.dtype == torch.float16):
         raise TypeError(f"{name} must be float32, got {t.dtype}")
     if not t.is_contiguous():
         raise ValueError(f"{name} must be contiguous")
@@ -608,16 +609,18 @@ def _fp16_split(hi, lo):
     return sw, wh, wl
 
 
-def _pack_split_weights(out, bias_np):
+def _pack_split_weights(out, bias_np, split16_in=False):
     """out fp32 [T][NP][cp] -> ([2T][NP][cp] for the split modes of the channels-last kernel, bias [NP + 4]).
     Taps 0..T-1: the TF32 hi parts.  Taps T..2T-1, SPLIT_KIND 1: the TF32 lo parts; SPLIT_KIND 2: per 32-channel chunk of cl
     channels the 4*cl bytes [fp16(hi * 2^sw) x cl | fp16(lo * 2^(11+sw)) x cl] -- the B operand of the fp16 correction MMA,
     whose A operand is [fp16(2^11 * lo(x)) | fp16(x)]; both products carry the factor 2^(11+sw), and bias[NP] = 2^-(11+sw) is
-    what the epilogue multiplies the correction accumulator with.  sw puts the largest weight just below 2^13."""
+    what the epilogue multiplies the correction accumulator with.  sw puts the largest weight just below 2^13.
+    split16_in (activations stored as split16, kernel split = 3): only those fp16 taps, [T][NP][cp]; the kernel also multiplies
+    their hi16 half with h = fp16(x), and bias[NP + 1] = 2^-sw scales that product back."""
     hi, lo = split_tf32(out)
     b = torch.zeros(bias_np.numel() + 4, dtype=torch.float32, device=out.device)
     b[:bias_np.numel()] = bias_np
-    if SPLIT_KIND == 1:
+    if SPLIT_KIND == 1 and not split16_in:
         b[bias_np.numel()] = 1.0
         return torch.cat((hi, lo), 0).contiguous(), b
     T, np_, cp = out.shape
@@ -628,12 +631,18 @@ def _pack_split_weights(out, bias_np):
         b2[:, :, 2 * c0:2 * c0 + cl] = wh[:, :, c0:c0 + cl]
         b2[:, :, 2 * c0 + cl:2 * c0 + 2 * cl] = wl[:, :, c0:c0 + cl]
     b[bias_np.numel()] = torch.ldexp(torch.ones((), device=out.device), -(sw + 11))
+    if split16_in:
+        b[bias_np.numel() + 1] = torch.ldexp(torch.ones((), device=out.device), -sw)
+        return b2.view(torch.float32).contiguous(), b
     return torch.cat((hi, b2.view(torch.float32)), 0).contiguous(), b
 
 
-def pack_conv2d_tf32_weights(w, bias, cp, split=False):
+def pack_conv2d_tf32_weights(w, bias, cp, split=False, split16_in=False):
     """[Cout,Cin,3,3] (+ bias [Cout]) -> ([9][NP][cp] fp32, bias [NP]); NP = Cout rounded up to 16.
-    split: [18][NP][cp] -- taps 0-8 the TF32 hi parts, 9-17 the correction operand (_pack_split_weights), bias [NP + 4]."""
+    split: [18][NP][cp] -- taps 0-8 the TF32 hi parts, 9-17 the correction operand (_pack_split_weights), bias [NP + 4].
+    split16_in (with split): [9][NP][cp], the fp16 taps alone, for a layer whose input is stored as split16."""
+    if split16_in and not split:
+        raise ValueError("split16_in needs split=True")
     cout, cin = w.shape[:2]
     np_ = (cout + 15) // 16 * 16
     out = torch.zeros((9, np_, cp), dtype=torch.float32, device=w.device)
@@ -641,7 +650,7 @@ def pack_conv2d_tf32_weights(w, bias, cp, split=False):
     b = torch.zeros(np_, dtype=torch.float32, device=w.device)
     b[:cout] = bias.float()
     if split:
-        out, b = _pack_split_weights(out, b)
+        out, b = _pack_split_weights(out, b, split16_in)
         return out, b, np_
     return rna_tf32(out).contiguous(), b.contiguous(), np_
 
@@ -794,26 +803,47 @@ def conv2d_tf32_rows_nchw_cat(srcs, w_compact, bias8, cout, dilation=1, relu=Fal
     return out
 
 
-def conv2d_tf32_nhwc_halo(x_pad, w_packed, bias, relu, round_out=False, split=False):
+def _nhwc_format(round_tf32, split16):
+    """The storage-format argument of the channels-last writers: 0 fp32, 1 fp32 rounded to TF32, 2 split16."""
+    return 2 if split16 else (1 if round_tf32 else 0)
+
+
+def _nhwc_empty(B, h, w, cp, split16, device):
+    """[B,h,w,cp] fp32, or its split16 form: the same bytes as fp16 [B,h,w,2*cp] (the dtype tells the formats apart)."""
+    if split16:
+        return torch.empty((B, h, w, 2 * cp), dtype=torch.float16, device=device)
+    return torch.empty((B, h, w, cp), dtype=torch.float32, device=device)
+
+
+def conv2d_tf32_nhwc_halo(x_pad, w_packed, bias, relu, round_out=False, split=False, split16_out=False):
     """x fp32 [B,h+2,w+2,cp] channels-last with a zero border -> fp32 [B,h+2,w+2,NP] (border zeros).
-    split: 3xTF32 -- x unrounded fp32, w_packed [18][NP][cp] from pack_conv2d_tf32_weights(split=True)."""
-    _chk("x_pad", x_pad)
+    split: 3xTF32 -- x unrounded fp32, w_packed [18][NP][cp] from pack_conv2d_tf32_weights(split=True).
+    x fp16 [B,h+2,w+2,2*cp] is split16 storage (common.cuh: split16_store; needs split, w_packed [9][NP][cp] from
+    split16_in=True, cp % 16 == 0).  split16_out: the output stored as split16 too, fp16 [B,h+2,w+2,2*NP]."""
+    _chk("x_pad", x_pad, split16_ok=True)
     B, hp, wp, cp = x_pad.shape
     np_ = w_packed.shape[1]
-    if w_packed.shape[0] != (18 if split else 9) or w_packed.shape[2] != cp:
-        raise ValueError(f"w_packed {tuple(w_packed.shape)} does not match cp={cp}, split={split}")
-    out = torch.empty((B, hp, wp, np_), dtype=torch.float32, device=x_pad.device)
+    split16_in = x_pad.dtype == torch.float16
+    if split16_in:
+        cp //= 2
+        if not split:
+            raise ValueError("split16 input needs split=True")
+    if w_packed.shape[0] != (18 if split and not split16_in else 9) or w_packed.shape[2] != cp:
+        raise ValueError(f"w_packed {tuple(w_packed.shape)} does not match cp={cp}, split={split}, split16 input={split16_in}")
+    out = _nhwc_empty(B, hp, wp, np_, split16_out, x_pad.device)
     _call("decnet_conv2d_tc_nhwc_halo", x_pad, x_pad.data_ptr(), w_packed.data_ptr(), bias.data_ptr(), out.data_ptr(),
-          B, hp - 2, wp - 2, cp, np_, 1 if relu else 0, 1 if round_out else 0, _split_arg(split))
+          B, hp - 2, wp - 2, cp, np_, 1 if relu else 0, _nhwc_format(round_out, split16_out),
+          3 if split16_in else _split_arg(split))
     return out
 
 
-def nchw_cat_to_nhwc_pad(srcs, cp, round_tf32=True):
+def nchw_cat_to_nhwc_pad(srcs, cp, round_tf32=True, split16=False):
     """cat(srcs, 1) (NCHW, single-channel maps as [B,H,W]) -> zero-bordered channels-last [B,H+2,W+2,cp]
-    (round_tf32: values rounded to TF32 for the halo kernel's plain-TF32 mode; its 3xTF32 mode takes them unrounded)."""
+    (round_tf32: values rounded to TF32 for the halo kernel's plain-TF32 mode; its 3xTF32 mode takes them unrounded;
+    split16: stored as split16, fp16 [B,H+2,W+2,2*cp], for its split16-input mode)."""
     x0, B, H, W, ptrs, cs, n = _cat_srcs(srcs)
-    out = torch.empty((B, H + 2, W + 2, int(cp)), dtype=torch.float32, device=x0.device)
-    _call("decnet_nchw_cat_to_nhwc_pad", x0, ptrs, cs, n, out.data_ptr(), B, H, W, int(cp), 1 if round_tf32 else 0)
+    out = _nhwc_empty(B, H + 2, W + 2, int(cp), split16, x0.device)
+    _call("decnet_nchw_cat_to_nhwc_pad", x0, ptrs, cs, n, out.data_ptr(), B, H, W, int(cp), _nhwc_format(round_tf32, split16))
     return out
 
 
@@ -825,9 +855,10 @@ def nhwc_pad_to_nchw(x_pad, channels):
     return out
 
 
-def dynup_pack_nhwc(disp, left_fea, cp, round_tf32=True, pad=False):
+def dynup_pack_nhwc(disp, left_fea, cp, round_tf32=True, pad=False, split16=False):
     """pad=True: [B,h+2,w+2,cp] with a zero border (the layout conv2d_tf32_nhwc_halo chains on).
-    disp=None: only the feature channels (channel 0 zero) -- dynup_set_disp_nhwc() completes it later."""
+    disp=None: only the feature channels (channel 0 zero) -- dynup_set_disp_nhwc() completes it later.
+    split16: stored as split16, fp16 [B,h(+2),w(+2),2*cp]."""
     _chk("left_fea", left_fea)
     B, Cc, H3, W3 = left_fea.shape
     if H3 % 3 or W3 % 3:
@@ -838,22 +869,24 @@ def dynup_pack_nhwc(disp, left_fea, cp, round_tf32=True, pad=False):
         if tuple(disp.shape) != (B, h, w):
             raise ValueError(f"left_fea {tuple(left_fea.shape)} is not 3x the disparity map {tuple(disp.shape)}")
     k = 2 if pad else 0
-    out = torch.empty((B, h + k, w + k, int(cp)), dtype=torch.float32, device=left_fea.device)
+    out = _nhwc_empty(B, h + k, w + k, int(cp), split16, left_fea.device)
     _call("decnet_dynup_pack_nhwc", left_fea, disp.data_ptr() if disp is not None else None, left_fea.data_ptr(),
-          out.data_ptr(), B, Cc, h, w, int(cp), 1 if round_tf32 else 0, 1 if pad else 0)
+          out.data_ptr(), B, Cc, h, w, int(cp), _nhwc_format(round_tf32, split16), 1 if pad else 0)
     return out
 
 
 def dynup_set_disp_nhwc(packed, disp, round_tf32=True, pad=False):
-    """Writes channel 0 (the disparity) of a tensor packed with disp=None, in place; returns it."""
+    """Writes channel 0 (the disparity) of a tensor packed with disp=None, in place, in the tensor's format (fp16: split16,
+    round_tf32 ignored); returns it."""
     _chk("disp", disp)
     B, h, w = disp.shape
-    _chk("packed", packed, disp)
+    _chk("packed", packed, disp, split16_ok=True)
     k = 2 if pad else 0
     if tuple(packed.shape[:3]) != (B, h + k, w + k):
         raise ValueError(f"packed {tuple(packed.shape)} does not match disp {tuple(disp.shape)} (pad={pad})")
-    _call("decnet_dynup_set_disp_nhwc", disp, disp.data_ptr(), packed.data_ptr(), B, h, w, packed.shape[-1],
-          1 if round_tf32 else 0, 1 if pad else 0)
+    split16 = packed.dtype == torch.float16
+    _call("decnet_dynup_set_disp_nhwc", disp, disp.data_ptr(), packed.data_ptr(), B, h, w,
+          packed.shape[-1] // (2 if split16 else 1), _nhwc_format(round_tf32, split16), 1 if pad else 0)
     return packed
 
 

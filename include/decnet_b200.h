@@ -281,9 +281,16 @@ int decnet_conv2d_tf32_nhwc_halo(const float *x_pad, const float *w_packed, cons
  * [fp16(hi(w) * 2^sw) x cl | fp16(lo(w) * 2^(11+sw)) x cl]; the kernel builds [fp16(2^11 * lo(x)) x cl | fp16(x) x cl]; taps
  * 0-8 are the plain TF32 hi parts; bias has np + 4 floats and bias[np] = 2^-(11+sw), the factor of the correction accumulator
  * (decnet_b200/ops.py: _pack_split_weights).  np <= 96 for the 3x3 form in the split modes (two stages must fit in shared memory).
- * The same holds for the _ldc form and for decnet_gemm_tc_nhwc (taps 0 / 1 instead of 0-8 / 9-17). */
+ * The same holds for the _ldc form and for decnet_gemm_tc_nhwc (taps 0 / 1 instead of 0-8 / 9-17).
+ * split = 3 (split16 input; the Python side's default inside the DynamicUpsampling and wide Refinement stacks): x_pad holds
+ * "split16" storage, the same 4 bytes per channel, per 32-channel chunk of cl channels the halves
+ * [fp16(2^11 * (x - h)) x cl | h x cl] with h = fp16(x), both rounded to nearest and saturating; cp % 16 == 0.  w_packed is
+ * [9][np][cp], split = 2's taps 9-17 alone; bias[np] = 2^-(11+sw) and bias[np + 1] = 2^-sw.  Results are fp32-class (the
+ * 3xTF32 error budget) for |activations| < 65504; beyond that the stored halves saturate and the results stay finite.
+ * round_out is the output's storage format: 0 fp32, 1 fp32 rounded to TF32, 2 split16 (out_pad then holds np channels of
+ * split16, as the next split = 3 layer reads them). */
 int decnet_conv2d_tc_nhwc_halo(const float *x_pad, const float *w_packed, const float *bias, float *out_pad,
-                               int B, int h, int w, int cp, int np, int relu, int round_out_tf32, int split, void *stream);
+                               int B, int h, int w, int cp, int np, int relu, int round_out, int split, void *stream);
 
 /* Tuning switch (per calling thread): 0 / 1 = one 128-pixel tile per CTA (default); 2 = split-mode launches with at least two
  * tiles per SM and np <= 96 run the pair kernel (two tiles per CTA share every weight stage: 1.7x fewer bytes from L2 per MMA;
@@ -326,10 +333,10 @@ int decnet_conv3x3s3_nchw(const float *x, const float *w_packed, const float *bi
 
 /* Layout bridges around decnet_conv2d_tf32_nhwc_halo for layers whose neighbours are NCHW (the 72-channel refinement
  * layers of the 1/9 level): concatenation of up to three NCHW fp32 sources -> zero-bordered channels-last
- * [B,h+2,w+2,CP] (channel padding zero; round_tf32 != 0 rounds the values to TF32 for the kernel's plain-TF32 mode),
- * and back: interior / first C channels -> NCHW [B,C,h,w]. */
+ * [B,h+2,w+2,CP] (channel padding zero; format: 0 fp32, 1 rounded to TF32 for the kernel's plain-TF32 mode, 2 split16
+ * for its split = 3 mode, CP % 16 == 0), and back: interior / first C channels -> NCHW [B,C,h,w]. */
 int decnet_nchw_cat_to_nhwc_pad(const float *const *srcs, const int *src_channels, int nsrc, float *out,
-                                int B, int h, int w, int CP, int round_tf32, void *stream);
+                                int B, int h, int w, int CP, int format, void *stream);
 int decnet_nhwc_pad_to_nchw(const float *in_pad, float *out, int B, int C, int NP, int h, int w, void *stream);
 
 /* Profiling hook: when set to a device buffer of 4*SMs int64, every conv3d launch on this thread
@@ -371,15 +378,16 @@ int decnet_dynup_glue(const float *logits, const float *disp, float *out,
 
 /* Channels-last variants around decnet_conv2d_tf32_nhwc: pack writes [B,h,w,CP] (CP >= 9C+1, padding
  * channels zero), glue reads logits [B,h,w,NP] (NP >= 81, channel = sub*9+k).  pad = 1: both tensors are
- * [B,h+2,w+2,.] with a one-pixel zero border (decnet_conv2d_tf32_nhwc_halo's layout; the pack writes the border). */
+ * [B,h+2,w+2,.] with a one-pixel zero border (decnet_conv2d_tf32_nhwc_halo's layout; the pack writes the border).
+ * format as for decnet_nchw_cat_to_nhwc_pad (2: split16, CP % 16 == 0). */
 int decnet_dynup_pack_nhwc(const float *disp, const float *left_fea, float *out,
-                           int B, int C, int h, int w, int CP, int round_tf32, int pad, void *stream);
+                           int B, int C, int h, int w, int CP, int format, int pad, void *stream);
 int decnet_dynup_glue_nhwc(const float *logits, const float *disp, float *out,
                            int B, int h, int w, int NP, int pad, void *stream);
 /* The feature channels do not depend on the disparity: decnet_dynup_pack_nhwc with disp = NULL writes channel 0 as
  * zero (it can run ahead of the disparity, on another stream) and this fills channel 0 of the interior pixels. */
 int decnet_dynup_set_disp_nhwc(const float *disp, float *packed,
-                               int B, int h, int w, int CP, int round_tf32, int pad, void *stream);
+                               int B, int h, int w, int CP, int format, int pad, void *stream);
 
 /* Skip-stage up-sampling (row a15; modules/SparseDenseNetRefinementMask.py:143-144): pred fp32 [B,h,w] (contiguous) ->
  * out fp32 [B,H,W] = F.interpolate(pred*3, (H, W), mode="bicubic", align_corners=False), bit for bit what ATen's CUDA

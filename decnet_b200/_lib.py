@@ -75,7 +75,9 @@ SIGNATURES = {
     "decnet_detail_level_scratch_floats": (C.c_longlong, [_i] * 3),
     "decnet_detail_level": (_i, [_ptr] * 4 + [C.c_float] + [_i] * 3 + [C.c_void_p]),
     "decnet_image_prepare_u8": (_i, [_ptr] * 5 + [_i] * 5 + [C.c_void_p]),
+    "decnet_image_prepare_u8_shift": (_i, [_ptr] * 5 + [_i] * 6 + [C.c_void_p]),
     "decnet_disp_to_u16": (_i, [_ptr] * 2 + [_i] * 5 + [C.c_void_p]),
+    "decnet_disp_add": (_i, [_ptr, C.c_float, C.c_longlong, C.c_void_p]),
     "decnet_epe_3px": (_i, [_ptr] * 2 + [C.c_float, _ptr, C.c_longlong, C.c_void_p]),
     "decnet_mirror_swap_u8": (_i, [_ptr] * 4 + [_i] * 3 + [C.c_void_p]),
     "decnet_lr_check": (_i, [_ptr] + [_i] * 5 + [C.c_float] + [_ptr] * 3 + [C.c_void_p]),

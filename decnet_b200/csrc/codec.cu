@@ -2,6 +2,9 @@
 //   image_prepare_u8 : uint8 RGB HWC image -> top/left zero pad to the network size (demo.py:75-81 `padding`), /255
 //                      (the input of detailDetection, demo.py:158-162) and ToTensor + Normalize(mean, std)
 //                      (demo.py:82-88 `transform`), NCHW fp32 -- one pass, a quarter of the upload bytes of fp32 images.
+//                      Its _shift form reads the image shifted by a column offset: the right view of a search range
+//                      [min_disp, max_disp) that does not start at 0.
+//   disp_add         : the minimum disparity added back to the prediction of that shifted search (fp32, rounded to nearest).
 //   disp_to_u16      : the KITTI-style 16-bit disparity image demo.py:191-197 writes: clamp(pred * 256, 0, 65535)
 //                      truncated to uint16, cropped to the last ori_h rows / ori_w columns (the PNG deflate stays on the host).
 //   epe_3px          : modules/loss.py:427-437 `test_loss_func`: EPE and 3-px / 5 % error over 0 < gt < max_disp.
@@ -23,18 +26,24 @@ namespace codec {
 
 constexpr int kBlock = 256;
 
+// kShift: the image is read shifted right by col_shift columns (image column x - col_shift, black outside [0, w)), the
+// right view of StereoMatcher's minimum disparity; |col_shift| <= w.  Without it col_shift is unused and the code is the
+// unshifted kernel's.
+template <bool kShift>
 __global__ void __launch_bounds__(kBlock)
 image_prepare_u8_kernel(const unsigned char *__restrict__ img, float *__restrict__ out01, float *__restrict__ norm,
-                        float m0, float m1, float m2, float s0, float s1, float s2, int h, int w, int H, int W, long long n)
+                        float m0, float m1, float m2, float s0, float s1, float s2, int h, int w, int H, int W, long long n,
+                        int col_shift)
 {
     const long long i = (long long)blockIdx.x * kBlock + threadIdx.x;      // over B*H*W padded pixels
     if (i >= n) return;
     const int x = (int)(i % W), y = (int)((i / W) % H);
     const long long b = i / ((long long)W * H);
     const int ry = H - h, rx = W - w;                                      // residual rows / columns come FIRST
+    const int sx = kShift ? x - rx - col_shift : x - rx;                   // source column in the image
     float v[3] = {0.f, 0.f, 0.f};
-    if (y >= ry && x >= rx) {
-        const unsigned char *p = img + ((b * h + (y - ry)) * (long long)w + (x - rx)) * 3;
+    if (y >= ry && x >= rx && (!kShift || (sx >= 0 && sx < w))) {
+        const unsigned char *p = img + ((b * h + (y - ry)) * (long long)w + sx) * 3;
         v[0] = __fdiv_rn((float)p[0], 255.f); v[1] = __fdiv_rn((float)p[1], 255.f); v[2] = __fdiv_rn((float)p[2], 255.f);
     }
     const long long plane = (long long)H * W, o = b * 3 * plane + (long long)y * W + x;
@@ -63,6 +72,23 @@ disp_to_u16_kernel(const float *__restrict__ pred, unsigned short *__restrict__ 
     const int x = (int)(i % ow), y = (int)((i / ow) % oh);
     const long long b = i / ((long long)ow * oh);
     out[i] = disp_u16(pred[(b * H + (H - oh + y)) * (long long)W + (W - ow + x)]);
+}
+
+// pred[i] = pred[i] + offset in fp32, rounded to nearest (StereoMatcher's minimum disparity).  Threads 0..nvec-1 each take
+// one float4 of the 16-byte aligned body p[head, head + 4*nvec); the rest take one float of the unaligned head and the tail.
+__global__ void __launch_bounds__(kBlock)
+disp_add_kernel(float *__restrict__ p, float offset, long long head, long long nvec, long long n)
+{
+    const long long i = (long long)blockIdx.x * kBlock + threadIdx.x;
+    if (i < nvec) {
+        float4 *q = reinterpret_cast<float4 *>(p + head) + i;
+        float4 v = *q;
+        v.x = __fadd_rn(v.x, offset); v.y = __fadd_rn(v.y, offset); v.z = __fadd_rn(v.z, offset); v.w = __fadd_rn(v.w, offset);
+        *q = v;
+        return;
+    }
+    const long long j = i - nvec, k = j < head ? j : j + 4 * nvec;        // scalar j: head element, then tail element
+    if (k < n) p[k] = __fadd_rn(p[k], offset);
 }
 
 // Reverse order of 4 RGB pixels held in 3 little-endian words: pixel k is bytes 3k..3k+2 of (a, b, c).
@@ -762,8 +788,22 @@ int decnet_image_prepare_u8(const unsigned char *img_hwc, float *out01, float *o
     DECNET_REQUIRE(img_hwc && (out01 || out_norm) && mean3_host && std3_host, "null pointer");
     DECNET_REQUIRE(B > 0 && h > 0 && w > 0 && H >= h && W >= w, "padded size %dx%d must cover the image %dx%d", H, W, h, w);
     const long long n = (long long)B * H * W;
-    image_prepare_u8_kernel<<<(unsigned)((n + kBlock - 1) / kBlock), kBlock, 0, static_cast<cudaStream_t>(stream)>>>(
-        img_hwc, out01, out_norm, mean3_host[0], mean3_host[1], mean3_host[2], std3_host[0], std3_host[1], std3_host[2], h, w, H, W, n);
+    image_prepare_u8_kernel<false><<<(unsigned)((n + kBlock - 1) / kBlock), kBlock, 0, static_cast<cudaStream_t>(stream)>>>(
+        img_hwc, out01, out_norm, mean3_host[0], mean3_host[1], mean3_host[2], std3_host[0], std3_host[1], std3_host[2], h, w, H, W, n,
+        0);
+    return after_launch("image_prepare_u8_kernel");
+}
+
+int decnet_image_prepare_u8_shift(const unsigned char *img_hwc, float *out01, float *out_norm, const float *mean3_host,
+                                  const float *std3_host, int B, int h, int w, int H, int W, int col_shift, void *stream)
+{
+    DECNET_REQUIRE(img_hwc && (out01 || out_norm) && mean3_host && std3_host, "null pointer");
+    DECNET_REQUIRE(B > 0 && h > 0 && w > 0 && H >= h && W >= w, "padded size %dx%d must cover the image %dx%d", H, W, h, w);
+    const long long n = (long long)B * H * W;
+    col_shift = std::max(-w, std::min(w, col_shift));                      // beyond +-w every column is black alike
+    image_prepare_u8_kernel<true><<<(unsigned)((n + kBlock - 1) / kBlock), kBlock, 0, static_cast<cudaStream_t>(stream)>>>(
+        img_hwc, out01, out_norm, mean3_host[0], mean3_host[1], mean3_host[2], std3_host[0], std3_host[1], std3_host[2], h, w, H, W, n,
+        col_shift);
     return after_launch("image_prepare_u8_kernel");
 }
 
@@ -774,6 +814,17 @@ int decnet_disp_to_u16(const float *pred, unsigned short *out, int B, int H, int
     const long long n = (long long)B * ori_h * ori_w;
     disp_to_u16_kernel<<<(unsigned)((n + kBlock - 1) / kBlock), kBlock, 0, static_cast<cudaStream_t>(stream)>>>(pred, out, H, W, ori_h, ori_w, n);
     return after_launch("disp_to_u16_kernel");
+}
+
+int decnet_disp_add(float *pred, float offset, long long n, void *stream)
+{
+    DECNET_REQUIRE(pred && (reinterpret_cast<uintptr_t>(pred) & 3) == 0, "pred must be a non-null, 4-byte aligned float pointer");
+    DECNET_REQUIRE(n > 0, "empty map (n = %lld)", n);
+    const long long head = std::min(n, (long long)(((16 - (reinterpret_cast<uintptr_t>(pred) & 15)) & 15) / 4));
+    const long long nvec = (n - head) / 4, threads = nvec + (n - 4 * nvec);
+    disp_add_kernel<<<(unsigned)((threads + kBlock - 1) / kBlock), kBlock, 0, static_cast<cudaStream_t>(stream)>>>(
+        pred, offset, head, nvec, n);
+    return after_launch("disp_add_kernel");
 }
 
 int decnet_mirror_swap_u8(const unsigned char *left, const unsigned char *right, unsigned char *out_left,

@@ -243,18 +243,20 @@ class FeatExtNetChannelPlus(_Cached, nn.Module):
         return out
 
 
-def extract_pair(fe, left, right, prepare=None):
+def extract_pair(fe, left, right, prepare=None, prepare_right=None):
     """Features of both views, the right view on a forked second stream (the two extractions are independent;
     demo.py:166-167 runs them back to back inside the model).  `prepare` is applied to each input first
-    (e.g. the uint8 -> padded / normalised image kernel).  Returns (left_feats, right_feats), joined on the
-    current stream; capturable in a CUDA graph (two branches)."""
+    (e.g. the uint8 -> padded / normalised image kernel), `prepare_right`, when given, to the right one instead (e.g. the
+    shifted prepare of a search range not starting at 0), on the forked stream too.  Returns (left_feats, right_feats),
+    joined on the current stream; capturable in a CUDA graph (two branches)."""
     main = torch.cuda.current_stream(left.device)
     side = getattr(fe, "_side", None)
     if side is None or side.device != left.device:
         side = fe._side = torch.cuda.Stream(left.device)
+    prepare_right = prepare_right or prepare
     side.wait_stream(main)                               # fork
     with torch.cuda.stream(side):
-        fr = fe(prepare(right) if prepare is not None else right)
+        fr = fe(prepare_right(right) if prepare_right is not None else right)
     fl = fe(prepare(left) if prepare is not None else left)
     # join; the right view's tensors live in the side stream's pool and are reused only behind the next fork
     main.wait_stream(side)

@@ -264,18 +264,26 @@ def detail_head(x_l, x_r, w3, bias, logit_thold):
 IMAGENET_MEAN, IMAGENET_STD = (0.485, 0.456, 0.406), (0.229, 0.224, 0.225)       # demo.py:85-86
 
 
-def image_prepare_u8(img_u8, multiple=27, want01=True, want_norm=True, mean=IMAGENET_MEAN, std=IMAGENET_STD):
+def image_prepare_u8(img_u8, multiple=27, want01=True, want_norm=True, mean=IMAGENET_MEAN, std=IMAGENET_STD, col_shift=0):
     """uint8 RGB [B,h,w,3] (CUDA) -> (img01, img_norm) fp32 [B,3,H,W], top/left zero-padded to multiples of
-    `multiple` like demo.py:75-81; img01 = v/255, img_norm = (v/255 - mean)/std (demo.py:82-88)."""
+    `multiple` like demo.py:75-81; img01 = v/255, img_norm = (v/255 - mean)/std (demo.py:82-88).  col_shift (an int)
+    first shifts the image right by that many columns, black where the source column lies outside the image
+    (oracle/disp_range.py's shift_cols_u8): the right view of a search range starting at min_disp = col_shift."""
     if not (isinstance(img_u8, torch.Tensor) and img_u8.is_cuda and img_u8.dtype == torch.uint8 and img_u8.is_contiguous()
             and img_u8.dim() == 4 and img_u8.shape[3] == 3):
         raise ValueError("img_u8 must be a contiguous CUDA uint8 tensor [B,h,w,3]")
+    if isinstance(col_shift, (bool, np.bool_)) or not isinstance(col_shift, numbers.Integral):
+        raise ValueError(f"col_shift must be an integer number of columns, got {col_shift!r}")
     B, h, w, _ = img_u8.shape
     H, W = -(-h // multiple) * multiple, -(-w // multiple) * multiple
     o01 = torch.empty((B, 3, H, W), dtype=torch.float32, device=img_u8.device) if want01 else None
     onm = torch.empty((B, 3, H, W), dtype=torch.float32, device=img_u8.device) if want_norm else None
-    _call("decnet_image_prepare_u8", img_u8, img_u8.data_ptr(), o01.data_ptr() if want01 else None,
-          onm.data_ptr() if want_norm else None, (ctypes.c_float * 3)(*mean), (ctypes.c_float * 3)(*std), B, h, w, H, W)
+    args = (img_u8.data_ptr(), o01.data_ptr() if want01 else None, onm.data_ptr() if want_norm else None,
+            (ctypes.c_float * 3)(*mean), (ctypes.c_float * 3)(*std), B, h, w, H, W)
+    if col_shift == 0:
+        _call("decnet_image_prepare_u8", img_u8, *args)
+    else:                                                                  # beyond +-w every column is black alike
+        _call("decnet_image_prepare_u8_shift", img_u8, *args, max(-w, min(w, int(col_shift))))
     return o01, onm
 
 
@@ -286,6 +294,18 @@ def disp_to_u16(pred, ori_h, ori_w):
     out = torch.empty((B, int(ori_h), int(ori_w)), dtype=torch.uint16, device=pred.device)
     _call("decnet_disp_to_u16", pred, pred.data_ptr(), out.data_ptr(), B, H, W, int(ori_h), int(ori_w))
     return out
+
+
+def disp_add(pred, offset):
+    """pred += offset in place, in fp32 rounded to nearest (pred + torch.float32(offset) bit for bit); pred a contiguous
+    CUDA fp32 tensor of any shape, offset a real number (not a bool) that float32 represents exactly.  Returns pred."""
+    _chk("pred", pred)
+    if (isinstance(offset, (bool, np.bool_)) or not isinstance(offset, numbers.Real)
+            or float(np.float32(offset)) != float(offset)):
+        raise ValueError(f"offset must be a number that float32 represents exactly, got {offset!r}")
+    if pred.numel():
+        _call("decnet_disp_add", pred, pred.data_ptr(), float(offset), pred.numel())
+    return pred
 
 
 def mirror_swap_u8(left, right, out_left, out_right):

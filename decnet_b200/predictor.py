@@ -8,6 +8,7 @@
     dense = StereoMatcher(lr_check=1.0, fill="background")(left, right)         # ... and its holes filled
     dense = StereoMatcher(lr_check=1.0, fill="guided")(left, right)             # ... filled along the left image
     dense = StereoMatcher(lr_check=1.0, speckle_size=100, fill="background")(left, right)   # ... speckles removed first
+    disp = m(left, right, min_disp=243, max_disp=768)   # search [243, 783) only; min_disp may be negative
 
 Every call of one shape (B, h, w, max_disp) replays one CUDA graph of the whole step: uint8 -> pad / normalise ->
 feature extractor (both views, the right one on a forked stream) -> [image-space detail masks] -> decomposed matching.
@@ -38,6 +39,16 @@ the check by coincidence and form small islands, which either fill would spread 
 pixels becomes invalid: 0 without a fill, filled with one, False in `valid`.  It runs outside the graph with the check, so
 it never re-captures either.
 
+The search range is [min_disp, max_disp) (OpenCV's minDisparity, Middlebury's vmin / vmax; min_disp = 0 by default): only its
+width is rounded up to a multiple of 27, D = round_max_disp(max_disp - min_disp), and the range searched is
+[min_disp, min_disp + D).  The step runs the unchanged model at width D on (L, shift(R, min_disp)), shift(R, k)[:, x] =
+R[:, x - k] with black columns where the source lies outside the image (oracle/disp_range.py), and adds min_disp to the
+prediction in fp32: ops.image_prepare_u8(..., col_shift=min_disp) prepares every right view of the graph's batch, the
+reverse direction's shift(mirror(L), k) included, and ops.disp_add runs at the end of the graph.  With min_disp = 0 neither
+runs and the graph is today's.  The check, the fills and the speckle filter then see true disparities, negative ones
+included; output="u16" clamps a negative disparity to 0 (KITTI's "no value").  The start is baked into the graph like
+max_disp, so it is part of cache_key.
+
 The capture and the double-buffered loop of `stream()` restate bench.py's `capture` / `pipelined_e2e` on purpose:
 bench.py is the fixed measuring stick of the project and does not import the package's public API.
 """
@@ -66,9 +77,29 @@ def round_max_disp(max_disp):
     return -(-int(max_disp) // MULTIPLE) * MULTIPLE
 
 
-def cache_key(B, h, w, max_disp, masks, precision, lr=False):
-    """What one captured graph is specific to (a graph with the left-right check's reverse direction has a trailing "lr")."""
+DISP_LIMIT = 2 ** 24           # |min_disp|, |max_disp| at most this: the offset added to the prediction stays exact in fp32
+
+
+def disparity_range(min_disp, max_disp):
+    """The search range [min_disp, max_disp) as (min_disp, D): the model runs at the width D = max_disp - min_disp rounded up
+    to a multiple of 27, so the range searched is [min_disp, min_disp + D).  Host-only; ValueError when either end is not an
+    integer (or is a bool) or lies outside [-2**24, 2**24], or when max_disp <= min_disp."""
+    for name, v in (("min_disp", min_disp), ("max_disp", max_disp)):
+        if isinstance(v, (bool, np.bool_)) or not isinstance(v, (int, np.integer)):
+            raise ValueError(f"{name} must be an integer number of pixels, got {v!r}")
+        if not -DISP_LIMIT <= v <= DISP_LIMIT:
+            raise ValueError(f"{name} must lie in [-2**24, 2**24] (where the offset stays exact in fp32), got {v!r}")
+    if max_disp <= min_disp:
+        raise ValueError(f"max_disp must be larger than min_disp, got the range [{min_disp}, {max_disp})")
+    return int(min_disp), round_max_disp(int(max_disp) - int(min_disp))
+
+
+def cache_key(B, h, w, max_disp, masks, precision, lr=False, min_disp=0):
+    """What one captured graph is specific to: max_disp is the model's width D; a nonzero min_disp (the right views' shift)
+    adds ("min_disp", min_disp); a graph with the left-right check's reverse direction has a trailing "lr"."""
     key = (int(B), int(h), int(w), int(max_disp), masks, precision)
+    if min_disp:
+        key += (("min_disp", int(min_disp)),)
     return key + ("lr",) if lr else key
 
 
@@ -138,13 +169,17 @@ class _Set:
         self.host_r = torch.empty_like(self.host_l).pin_memory()
         self.graph = self.pred = self.sig = None
         self.uploaded = self.computed = None
+        self.min_disp = 0                          # the right views' column shift, baked into the graph at its capture
 
 
 class StereoMatcher:
     """Stereo matcher from uint8 RGB image pairs to disparity (see the module docstring).
 
     state_dict    reference-layout checkpoint, or None for the seeded random init (params, seed 17)
-    max_disp      rounded up to a multiple of 27; a call may override it
+    max_disp      the exclusive end of the search range; the width max_disp - min_disp is rounded up to a multiple of 27,
+                  and m.max_disp is min_disp + that width; a call may override it
+    min_disp      the start of the search range, an integer that may be negative (converging rigs, Middlebury's vmin);
+                  a call may override it
     masks         "learned": DecompMatching's detectors (use_detail=True, `thold`); "image": demo.py's route,
                   ops.detail_detection of the padded [0,1] images with `detail_thold`, finest level last
     skip_stage_id 3 skips the finest level (bicubic x3 of the 1/3 disparity; Middlebury, demo.sh:5)
@@ -162,7 +197,7 @@ class StereoMatcher:
 
     def __init__(self, state_dict=None, max_disp=192, masks="learned", thold=0.9, detail_thold=0.3, skip_stage_id=4,
                  precision="fp32", device="cuda", max_graphs=4, lr_check=None, fill="none", speckle_size=0,
-                 speckle_range=1.0):
+                 speckle_range=1.0, min_disp=0):
         if masks not in MASKS:
             raise ValueError(f"masks must be one of {MASKS}, got {masks!r}")
         if precision not in PRECISIONS:
@@ -177,10 +212,11 @@ class StereoMatcher:
         dev = torch.device(device)
         if dev.type != "cuda":
             raise ValueError(f"device must be a CUDA device (decnet_b200 has no CPU path), got {device!r}")
-        self.max_disp = round_max_disp(max_disp)
+        self.min_disp, D = disparity_range(min_disp, max_disp)
+        self.max_disp = self.min_disp + D
         self.masks, self.precision, self.detail_thold, self.max_graphs = masks, precision, float(detail_thold), max_graphs
         fe = FeatExtNetChannelPlus(8, precision=precision)
-        model = DecompMatching(max_disp=self.max_disp, skip_stage_id=skip_stage_id, use_detail=masks == "learned",
+        model = DecompMatching(max_disp=D, skip_stage_id=skip_stage_id, use_detail=masks == "learned",
                                thold=thold, precision=precision)
         self.fe, self.model = fe, model
         self.load_state_dict(state_dict)
@@ -214,26 +250,30 @@ class StereoMatcher:
                     st.graph.reset()
         self._graphs.clear()
 
-    def _forward(self, l, r):
-        """The whole step on the device, for the static inputs l, r -> padded prediction [B,H,W]."""
+    def _forward(self, l, r, min_disp=0):
+        """The whole step on the device, for the static inputs l, r -> padded prediction [B,H,W].  A nonzero min_disp
+        shifts the right views by min_disp columns as they are prepared and adds min_disp to the prediction."""
         if self.masks == "learned":
-            fl, fr = extract_pair(self.fe, l, r, prepare=lambda u8: ops.image_prepare_u8(u8, want01=False)[1])
-            return self.model(fl, fr)[0]
-        l01, lnorm = ops.image_prepare_u8(l)
-        r01, rnorm = ops.image_prepare_u8(r)
-        fl, fr = extract_pair(self.fe, lnorm, rnorm)
-        lm = ops.detail_detection(l01, 3, self.detail_thold)[::-1]       # finest level last (demo.py:161-162)
-        rm = ops.detail_detection(r01, 3, self.detail_thold)[::-1]
-        return self.model(fl, fr, lm, rm)[0]
+            prepare = lambda u8, shift=0: ops.image_prepare_u8(u8, want01=False, col_shift=shift)[1]
+            fl, fr = extract_pair(self.fe, l, r, prepare=prepare, prepare_right=lambda u8: prepare(u8, min_disp))
+            pred = self.model(fl, fr)[0]
+        else:
+            l01, lnorm = ops.image_prepare_u8(l)
+            r01, rnorm = ops.image_prepare_u8(r, col_shift=min_disp)
+            fl, fr = extract_pair(self.fe, lnorm, rnorm)
+            lm = ops.detail_detection(l01, 3, self.detail_thold)[::-1]   # finest level last (demo.py:161-162)
+            rm = ops.detail_detection(r01, 3, self.detail_thold)[::-1]
+            pred = self.model(fl, fr, lm, rm)[0]
+        return ops.disp_add(pred, min_disp) if min_disp else pred
 
     def _step(self, st):
         """What the graph of a set runs: [the reverse direction's inputs, then] the step at the set's batch."""
         if st.lr:
             B = st.l.shape[0]
             ops.mirror_swap_u8(st.l, st.r, st.xl[B:], st.xr[B:])
-        return self._forward(st.xl, st.xr)
+        return self._forward(st.xl, st.xr, st.min_disp)
 
-    def _capture(self, st, max_disp):
+    def _capture(self, st, max_disp, min_disp=0):
         """One eager run on a side stream (it rebuilds any stale weight cache), then the capture (bench.py's capture)."""
         if st.graph is not None:
             st.graph.reset()
@@ -241,6 +281,7 @@ class StereoMatcher:
             self._cap_stream = torch.cuda.Stream(self.dev)
         side, main = self._cap_stream, torch.cuda.current_stream(self.dev)
         graph = torch.cuda.CUDAGraph()
+        st.min_disp = min_disp
         saved, self.model.max_disp = self.model.max_disp, max_disp
         try:
             side.wait_stream(main)
@@ -271,10 +312,10 @@ class StereoMatcher:
             sets.append(_Set(B, h, w, self.dev, lr=key[-1] == "lr"))
         return sets
 
-    def _replay(self, st, max_disp):
+    def _replay(self, st, max_disp, min_disp=0):
         """Replay, re-capturing first when the set is new or any weight changed since its capture."""
         if st.graph is None or st.sig != self._sig():
-            self._capture(st, max_disp)
+            self._capture(st, max_disp, min_disp)
         st.graph.replay()
 
     # ------------------------------------------------------------------------------------------------------------ calls
@@ -292,8 +333,9 @@ class StereoMatcher:
         H, W = st.pred.shape[-2:]
         return st.pred[:, H - h:, W - w:].clone()                        # demo.py's crop: the last h rows, w columns
 
-    def _max_disp(self, max_disp):
-        return self.max_disp if max_disp is None else round_max_disp(max_disp)
+    def _range(self, min_disp=None, max_disp=None):
+        """The call's search range as (min_disp, width D), either end None for the matcher's, validated on the host."""
+        return disparity_range(self.min_disp if min_disp is None else min_disp, self.max_disp if max_disp is None else max_disp)
 
     def _lr(self, lr_check, return_valid, fill=None):
         """The call's left-right check tolerance (None: off) and fill rule, validated before any device work."""
@@ -317,25 +359,26 @@ class StereoMatcher:
         return size, rng
 
     def __call__(self, left, right, output="float", max_disp=None, lr_check=None, return_valid=False, fill=None,
-                 speckle_size=None, speckle_range=None):
+                 speckle_size=None, speckle_range=None, min_disp=None):
         """Disparity of one pair ([h,w,3]), a batch ([B,h,w,3]) or lists of single pairs (any sizes; one batch per
         distinct size, results in input order).  output "float" (pixels) or "u16" (x256, demo.py:191-197); the result
         has the kind of the input (numpy, CPU tensor or CUDA tensor).  lr_check (None: the matcher's) is the left-right
         check's tolerance in pixels; pixels that fail it are 0, or filled from their neighbours with fill="background" or
         along the left image with fill="guided" (None: the matcher's fill).  return_valid: each result is (disparity, bool valid), valid False on filled pixels.
-        speckle_size / speckle_range (None: the matcher's) remove speckles between the check and the fill."""
+        speckle_size / speckle_range (None: the matcher's) remove speckles between the check and the fill.  min_disp /
+        max_disp (None: the matcher's) give the search range [min_disp, max_disp) as for the constructor."""
         if output not in OUTPUTS:
             raise ValueError(f"output must be one of {OUTPUTS}, got {output!r}")
-        D = self._max_disp(max_disp)
         tol, fill = self._lr(lr_check, return_valid, fill)
         speckle = self._speckle(tol, speckle_size, speckle_range)
+        span = self._range(min_disp, max_disp)
         if isinstance(left, (list, tuple)):
-            return self._call_list(left, right, output, D, tol, return_valid, fill, speckle)
+            return self._call_list(left, right, output, span, tol, return_valid, fill, speckle)
         kind, batched, B, h, w = check_pair(left, right)
-        out = self._run(left, right, kind, B, h, w, output, D, tol, return_valid, fill, speckle)
+        out = self._run(left, right, kind, B, h, w, output, span, tol, return_valid, fill, speckle)
         return out if batched else _index(out, 0)
 
-    def _call_list(self, lefts, rights, output, D, tol, return_valid, fill, speckle):
+    def _call_list(self, lefts, rights, output, span, tol, return_valid, fill, speckle):
         if not isinstance(rights, (list, tuple)) or len(rights) != len(lefts):
             raise ValueError("left and right lists must have the same length")
         groups = OrderedDict()
@@ -347,7 +390,7 @@ class StereoMatcher:
         results = [None] * len(lefts)
         for (kind, h, w), idx in groups.items():
             stack = np.stack if kind == "numpy" else torch.stack
-            out = self._run(stack([lefts[i] for i in idx]), stack([rights[i] for i in idx]), kind, len(idx), h, w, output, D,
+            out = self._run(stack([lefts[i] for i in idx]), stack([rights[i] for i in idx]), kind, len(idx), h, w, output, span,
                             tol, return_valid, fill, speckle)
             for j, i in enumerate(idx):
                 results[i] = _index(out, j)
@@ -367,13 +410,14 @@ class StereoMatcher:
         st.r.copy_(st.host_r, non_blocking=True)
 
     @torch.no_grad()
-    def _run(self, left, right, kind, B, h, w, output, D, tol=None, return_valid=False, fill="none", speckle=(0, 1.0)):
+    def _run(self, left, right, kind, B, h, w, output, span, tol=None, return_valid=False, fill="none", speckle=(0, 1.0)):
         if kind == "cuda" and left.device != self.dev:
             raise ValueError(f"inputs are on {left.device}, the matcher on {self.dev}")
+        k, D = span
         with torch.cuda.device(self.dev):
-            st = self._sets(cache_key(B, h, w, D, self.masks, self.precision, tol is not None), 1)[0]
+            st = self._sets(cache_key(B, h, w, D, self.masks, self.precision, tol is not None, k), 1)[0]
             self._upload(st, left, right, kind)
-            self._replay(st, D)
+            self._replay(st, D, k)
             out = self._result(st, h, w, output, tol, return_valid, fill, speckle)
             if kind == "cuda":
                 return out
@@ -381,21 +425,22 @@ class StereoMatcher:
             return _map(lambda t: t.numpy(), out) if kind == "numpy" else out
 
     def stream(self, pairs, output="float", max_disp=None, lr_check=None, return_valid=False, fill=None, speckle_size=None,
-               speckle_range=None):
+               speckle_range=None, min_disp=None):
         """Yield the result of each (left, right) of `pairs` in order, software-pipelined over two buffer sets per shape:
         while the graph of item i runs, the copy stream uploads item i+1 into the other set (bench.py's pipelined_e2e).
         Host results are read back through pinned memory and yielded as fresh arrays.  A change of shape drains the
-        pipeline and continues with the new shape's sets.  lr_check / return_valid / fill / speckle_size / speckle_range as
-        for a call."""
+        pipeline and continues with the new shape's sets.  lr_check / return_valid / fill / speckle_size / speckle_range /
+        min_disp / max_disp as for a call."""
         if output not in OUTPUTS:
             raise ValueError(f"output must be one of {OUTPUTS}, got {output!r}")
-        D = self._max_disp(max_disp)
         tol, fill = self._lr(lr_check, return_valid, fill)
         speckle = self._speckle(tol, speckle_size, speckle_range)
-        return self._stream(pairs, output, D, tol, return_valid, fill, speckle)   # arguments checked now, not at the first item
+        span = self._range(min_disp, max_disp)
+        return self._stream(pairs, output, span, tol, return_valid, fill, speckle)   # arguments checked now, not at the first item
 
     @torch.no_grad()
-    def _stream(self, pairs, output, D, tol, return_valid, fill, speckle):
+    def _stream(self, pairs, output, span, tol, return_valid, fill, speckle):
+        min_disp, D = span
         with torch.cuda.device(self.dev):
             if self._copy_stream is None:
                 self._copy_stream = torch.cuda.Stream(self.dev)
@@ -405,7 +450,7 @@ class StereoMatcher:
                 kind, batched, B, h, w = check_pair(left, right)
                 if kind == "cuda" and left.device != self.dev:
                     raise ValueError(f"inputs are on {left.device}, the matcher on {self.dev}")
-                k = cache_key(B, h, w, D, self.masks, self.precision, tol is not None)
+                k = cache_key(B, h, w, D, self.masks, self.precision, tol is not None, min_disp)
                 if k != key:
                     while pending:
                         yield self._finish(pending.popleft())
@@ -430,7 +475,7 @@ class StereoMatcher:
                     st.uploaded = torch.cuda.Event()
                     st.uploaded.record(copy)
                 main.wait_event(st.uploaded)
-                self._replay(st, D)
+                self._replay(st, D, min_disp)
                 res = self._result(st, h, w, output, tol, return_valid, fill, speckle)
                 if kind != "cuda":
                     res = _map(_to_pinned, res)

@@ -418,13 +418,22 @@ int decnet_detail_level(const float *data, float *down, float *mask, float *scra
  *   decnet_image_prepare_u8: uint8 RGB [B,h,w,3] -> top/left zero pad to HxW (demo.py:75-81), out01 = v/255 fp32
  *     [B,3,H,W] (input of detailDetection, demo.py:158-162) and out_norm = (v/255 - mean)/std (demo.py:82-88); either
  *     output may be NULL; mean3 / std3 are HOST pointers.
+ *   decnet_image_prepare_u8_shift: decnet_image_prepare_u8 of the image shifted right by col_shift columns: image column
+ *     x takes the input's column x - col_shift, and 0 (black) where that lies outside [0, w); any col_shift, negative
+ *     included.  Bit for bit the unshifted entry run on the shifted image.  StereoMatcher prepares the right views of a
+ *     search range [min_disp, max_disp) with col_shift = min_disp.
  *   decnet_disp_to_u16: clamp(pred*256, 0, 65535) truncated to uint16 and cropped to the last ori_h rows / ori_w
  *     columns (demo.py:191-197; the PNG container is written on the host).
+ *   decnet_disp_add: pred[i] = pred[i] + offset in fp32 rounded to nearest (__fadd_rn), in place over n > 0 floats; pred
+ *     4-byte aligned, 16-byte vector accesses on its aligned body.  Adds min_disp back to the shifted search's prediction.
  *   decnet_epe_3px: sums3 (device, 3 doubles) = {sum |pred-gt|, #(|err|<3 or <5% gt), #valid} over 0 < gt < max_disp
  *     (modules/loss.py:427-437: epe = sums[0]/sums[2], loss_3 = 100 - 100*sums[1]/sums[2]). */
 int decnet_image_prepare_u8(const unsigned char *img_hwc, float *out01, float *out_norm, const float *mean3_host,
                             const float *std3_host, int B, int h, int w, int H, int W, void *stream);
+int decnet_image_prepare_u8_shift(const unsigned char *img_hwc, float *out01, float *out_norm, const float *mean3_host,
+                                  const float *std3_host, int B, int h, int w, int H, int W, int col_shift, void *stream);
 int decnet_disp_to_u16(const float *pred, unsigned short *out, int B, int H, int W, int ori_h, int ori_w, void *stream);
+int decnet_disp_add(float *pred, float offset, long long n, void *stream);
 int decnet_epe_3px(const float *pred, const float *gt, float max_disp, double *sums3, long long n, void *stream);
 
 /* Left-right consistency check of StereoMatcher (no counterpart in the reference; oracle/lr_check.py is the spec).

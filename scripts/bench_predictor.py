@@ -39,12 +39,21 @@
                      the HBM share is taken on lr_fill's algorithmic bytes (the check's 8 bytes read per pixel and the
                      outputs), so it also shows what the labeller's planes cost
   sceneflow_stream_lr_speckle  sceneflow_stream_lr_fill with speckle_size=100, runs alternating with the _lr_fill ones
+  middlebury_single_range  middlebury_single's pair searched over [0, 783) and over [243, 783) (min_disp=243, max_disp=768:
+                     width 540 instead of 783), alternating call by call: p50 / p90, the replay's device time, their ratios
+  sceneflow_stream_min_disp  sceneflow_stream with [27, 243) against [0, 216) (the same width: the cost of the shifted
+                     prepare and of disp_add_kernel), runs alternating, best of three
+  image_prepare_u8_shift, disp_add  the two kernels of the search range at B = 8 SceneFlow pairs, us per launch and the share
+                     of the HBM bound, rotating over buffer sets larger than L2; the shifted prepare alternates with
+                     image_prepare_u8 on the same buffers (bytes: the uint8 input and the fp32 normalised output);
+                     disp_add moves 8 bytes per pixel of the [8, 540, 972] padded prediction
 
-    python scripts/bench_predictor.py --out DIR
+    python scripts/bench_predictor.py --out DIR [--legs disp_range]
 """
 from __future__ import annotations
 
 import argparse
+import ctypes
 import json
 import subprocess
 import sys
@@ -247,6 +256,112 @@ def lr_speckle_legs(torch, res):
             torch.cuda.empty_cache()
 
 
+def disp_range_legs(torch, res, calls, stream_steps):
+    """9. the search range [min_disp, max_disp): what a range not starting at 0 saves on Middlebury, what the shift and the
+    offset cost a SceneFlow stream of the same width, and the two kernels beside image_prepare_u8."""
+    import numpy as np
+    from decnet_b200 import StereoMatcher, ops
+    from decnet_b200.predictor import cache_key
+    from decnet_b200.synthetic import calibrate_mask_density
+    dev = torch.device("cuda", 0)
+
+    # one Middlebury pair: [0, 783) against [243, 783) (width 540), alternating call by call
+    g = np.random.default_rng(1)
+    lm, rm = (g.integers(0, 256, (2000, 2900, 3), dtype=np.uint8) for _ in range(2))
+    m = StereoMatcher(max_disp=768, masks="image", skip_stage_id=3)
+    legs = {"full": {"min_disp": 0}, "range": {"min_disp": 243}}
+    for kw in legs.values():
+        for _ in range(3):
+            m(lm, rm, output="u16", **kw)
+    ts = {k: [] for k in legs}
+    for _ in range(calls):
+        for k, kw in legs.items():
+            t0 = time.perf_counter()
+            m(lm, rm, output="u16", **kw)
+            ts[k].append((time.perf_counter() - t0) * 1e3)
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    dev_ms = {k: [] for k in legs}
+    for _ in range(2):
+        for k, kw in legs.items():
+            lo, D = m._range(kw["min_disp"])
+            (st,) = m._graphs[cache_key(1, 2000, 2900, D, m.masks, m.precision, False, lo)]
+            torch.cuda.synchronize()
+            e0.record()
+            for _ in range(10):
+                st.graph.replay()
+            e1.record()
+            torch.cuda.synchronize()
+            dev_ms[k].append(e0.elapsed_time(e1) / 10)
+    r = {k: {"range": f"[{kw['min_disp']}, {m.max_disp})", "width": m._range(kw["min_disp"])[1], "p50_ms": pct(ts[k], 0.5),
+             "p90_ms": pct(ts[k], 0.9), "replay_device_ms": min(dev_ms[k]), "replay_device_ms_runs": dev_ms[k]}
+         for k, kw in legs.items()}
+    r["range_over_full"] = {"p50": r["range"]["p50_ms"] / r["full"]["p50_ms"],
+                            "replay_device": r["range"]["replay_device_ms"] / r["full"]["replay_device_ms"]}
+    res["middlebury_single_range"] = dict(r, calls=calls, shape="2000x2900 -> 2025x2916", masks="image", skip_stage_id=3,
+                                          what="m(l, r, output=\"u16\") host to host, the two ranges alternating call by call")
+    del m
+    torch.cuda.empty_cache()
+
+    # B = 8 SceneFlow pairs through stream(): [27, 243) against [0, 216), the same width, runs alternating
+    B, n = 8, stream_steps
+    m = StereoMatcher(max_disp=192)
+    gd = torch.Generator(device=dev).manual_seed(99)
+    l8 = torch.randint(0, 256, (B, 540, 960, 3), device=dev, generator=gd, dtype=torch.uint8)
+    r8 = torch.randint(0, 256, (B, 540, 960, 3), device=dev, generator=gd, dtype=torch.uint8)
+    prep = lambda u8: ops.image_prepare_u8(u8, want01=False)[1]
+    calibrate_mask_density(m.model, m.fe(prep(l8)), m.fe(prep(r8)), 0.10)
+    pair = (l8.cpu(), r8.cpu())
+    legs = {"plain": {}, "min_disp": {"min_disp": 27, "max_disp": 243}}
+    for kw in legs.values():
+        for _ in m.stream([pair] * 4, output="u16", **kw):
+            pass
+    els = {k: [] for k in legs}
+    for _ in range(3):
+        for k, kw in legs.items():
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            for _ in m.stream([pair] * n, output="u16", **kw):
+                pass
+            els[k].append(time.perf_counter() - t0)
+    rate = {k: B * n / min(v) for k, v in els.items()}
+    res["sceneflow_stream_min_disp"] = {
+        "batch": B, "steps": n, "pairs_per_s": rate["min_disp"], "plain_pairs_per_s": rate["plain"],
+        "min_disp_over_plain_rate": rate["min_disp"] / rate["plain"],
+        "pairs_per_s_runs": {k: [B * n / e for e in v] for k, v in els.items()},
+        "what": "stream() with [27, 243) against [0, 216) (both width 216), uint16 out, runs alternating; best of three"}
+    del m
+    torch.cuda.empty_cache()
+
+    # the kernels at B = 8 SceneFlow pairs, rotating over buffer sets larger than L2 together
+    B, h, w, H, W = 8, 540, 960, 540, 972
+    nsets = 8
+    imgs = [torch.randint(0, 256, (B, h, w, 3), device=dev, dtype=torch.uint8) for _ in range(nsets)]
+    outs = [torch.empty(B, 3, H, W, device=dev) for _ in range(nsets)]
+    mean, std = (ctypes.c_float * 3)(*ops.IMAGENET_MEAN), (ctypes.c_float * 3)(*ops.IMAGENET_STD)
+    plain = lambda i: ops._call("decnet_image_prepare_u8", imgs[i], imgs[i].data_ptr(), None, outs[i].data_ptr(), mean, std,
+                                B, h, w, H, W)
+    shift = lambda i: ops._call("decnet_image_prepare_u8_shift", imgs[i], imgs[i].data_ptr(), None, outs[i].data_ptr(), mean,
+                                std, B, h, w, H, W, 27)
+    runs = {"plain": [], "shift": []}
+    for _ in range(2):                                                   # alternating, best of each
+        runs["plain"].append(kernel_us(torch, plain, nsets))
+        runs["shift"].append(kernel_us(torch, shift, nsets))
+    nbytes = B * h * w * 3 + B * 3 * H * W * 4
+    t_plain, t_shift = min(runs["plain"]), min(runs["shift"])
+    res["image_prepare_u8_shift"] = dict(hbm_share(nbytes, t_shift), us=t_shift, image_prepare_u8_us=t_plain,
+                                         shift_over_plain=t_shift / t_plain,
+                                         image_prepare_u8_frac_of_hbm_bound=hbm_share(nbytes, t_plain)["frac_of_hbm_bound"],
+                                         us_runs=runs, shape=f"{B}x{h}x{w}x3 -> {B}x3x{H}x{W}, normalised output only",
+                                         col_shift=27, buffer_sets=nsets)
+    del imgs, outs
+    nsets = 20
+    preds = [torch.randn(B, H, W, device=dev) for _ in range(nsets)]
+    t = kernel_us(torch, lambda i: ops._call("decnet_disp_add", preds[i], preds[i].data_ptr(), 27.0, preds[i].numel()), nsets)
+    res["disp_add"] = dict(hbm_share(8 * B * H * W, t), us=t, shape=f"{B}x{H}x{W} in place", buffer_sets=nsets)
+    del preds
+    torch.cuda.empty_cache()
+
+
 def run_bench_py():
     cmd = [sys.executable, str(ROOT / "bench.py"), "--gpus", "1", "--steps", "20", "--warmup", "5", "--no-cpu-baseline",
            "--no-extras"]
@@ -264,6 +379,8 @@ def main():
     ap.add_argument("--out", required=True)
     ap.add_argument("--calls", type=int, default=200)
     ap.add_argument("--stream-steps", type=int, default=60)
+    ap.add_argument("--legs", choices=("all", "disp_range"), default="all",
+                    help="disp_range: only the search-range legs (and the card's name and power limit)")
     args = ap.parse_args()
     out = Path(args.out)
     out.mkdir(parents=True, exist_ok=True)
@@ -275,6 +392,11 @@ def main():
     from decnet_b200._lib import lib
     dev = torch.device("cuda", 0)
     res = {"gpu": gpu_info(torch)}
+    if args.legs == "disp_range":
+        disp_range_legs(torch, res, 30, args.stream_steps)
+        (out / "bench_predictor.json").write_text(json.dumps(res, indent=1))
+        print(json.dumps(res))
+        return
     res["bench_py"] = run_bench_py()
 
     # 1. one SceneFlow pair
@@ -480,6 +602,7 @@ def main():
         torch.cuda.empty_cache()
 
     lr_speckle_legs(torch, res)
+    disp_range_legs(torch, res, 30, args.stream_steps)
     (out / "bench_predictor.json").write_text(json.dumps(res, indent=1))
     print(json.dumps(res))
 
